@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the path-tracing hot path on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c3|c3k|c2|c1|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c3|c3k|c2|c1|c5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload (default) = BASELINE.json config 3, the one the metric is quoted on: "Dragon" at 1920x1080, 64 spp, 8 bounces,
@@ -61,7 +61,13 @@ def parse_args():
     p.add_argument("--cpu-sample", default="", help="WxHxSPP of the bounded CPU sample (default per workload)")
     p.add_argument("--lean", action="store_true", help="skip the optional legs (kernel-alone timing, RGBA8 end-to-end, dead-ray frame): for minutes-long frames (c5)")
     p.add_argument("--verify", action="store_true", help="N>1: rank 0 also renders the frame alone and asserts the gathered frame is bit-identical")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default="",
+                   help="after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0): image.npy, the tone-mapped "
+                        "RGBA frame, or prim.npy and t.npy for c2; over 60 MiB in all, the same seeded sample of pixels from each")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
 
 
 def load_workload(name, args):
@@ -242,6 +248,23 @@ def ncu_counters(workload):
     return None
 
 
+DUMP_LIMIT_BYTES = 60 << 20          # 62.9 MB of data: the files stay under 64 MB with their headers
+
+
+def dump_outputs(path, arrays):
+    """Writes each (h, w, ...) array as path/<name>.npy: float32, integer arrays as float64 (exact). Over DUMP_LIMIT_BYTES in all,
+    every array keeps the same pixels, a fixed seeded sample in row-major order, as (n_pixels, channels)."""
+    os.makedirs(path, exist_ok=True)
+    out = {k: np.asarray(a, np.float64 if np.issubdtype(a.dtype, np.integer) else np.float32) for k, a in arrays.items()}
+    n_px = {a.shape[0] * a.shape[1] for a in out.values()}.pop()
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n_px, DUMP_LIMIT_BYTES // (total // n_px), replace=False))
+        out = {k: a.reshape(n_px, -1)[keep] for k, a in out.items()}
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def emit_line(stdout_fd, line):
     """The one JSON line goes to the process's ORIGINAL stdout; everything else any library prints (NCCL's version banner, warnings)
     was sent to stderr by main()."""
@@ -335,11 +358,13 @@ def main():
     for i in range(args.steps):
         flush.fill_(i & 0xff)                 # L2 flush between timed iterations (outside the event pair)
         ev[i][0].record()
-        step()
+        frame = step()
         ev[i][1].record()
     barrier()
     sampler.stop_flag = True
     sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {k: v.cpu().numpy() for k, v in (dict(prim=prim, t=tbuf) if primary_only else dict(image=frame)).items()})
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=device)
     if world > 1:

@@ -55,7 +55,7 @@ def write_hdr_and_decode(path, env_rgb):
     return dec
 
 
-@pytest.mark.skipif(not os.path.exists(BIN), reason="drop-in main.cpp binary not built (needs /root/reference at build time)")
+@pytest.mark.skipif(not os.path.exists(BIN), reason="drop-in main.cpp binary not built: it needs the reference project's sources (REF_DIR), which are not part of this repository")
 def test_reference_main_cpp_drives_the_b200_path(rt, tmp_path):
     from PIL import Image as PILImage
     from sycl_ray_tracing_b200 import scenes

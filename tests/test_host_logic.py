@@ -6,7 +6,7 @@ import re
 import numpy as np
 import pytest
 
-from conftest import ROOT, has_cuda, load_golden, scene_arrays
+from conftest import ROOT, load_golden, scene_arrays
 
 
 def bits(a):
@@ -30,16 +30,30 @@ def test_header_cites_reference_interfaces():
         assert cite in header
 
 
-@pytest.mark.skipif(has_cuda(), reason="checks the no-GPU failure mode")
-def test_compute_fails_loudly_without_a_gpu(rt, golden_scenes):
-    a = scene_arrays(golden_scenes, "cornell")
-    with pytest.raises(rt.B200RTError, match="no CUDA device"):
-        rt.Scene(a["tri9"], a["mat_idx"], a["mats10"], a["emissive"])
-    # the stages either side of the path have no CPU fallback either
-    with pytest.raises(rt.B200RTError, match="no CUDA device"):
-        rt.BVH(a["tri9"], on_device=True)
-    with pytest.raises(rt.B200RTError, match="no CUDA device"):
-        rt.quantise_rgba8(np.zeros((4, 4, 4), np.float32))
+NO_GPU_CHECK = """
+import numpy as np
+import pytest
+import sycl_ray_tracing_b200 as rt
+g = np.load("tests/golden/scenes.npz")
+a = {k: g["cornell_" + k] for k in ("tri9", "mat_idx", "mats10", "emissive")}
+with pytest.raises(rt.B200RTError, match="no CUDA device"):
+    rt.Scene(a["tri9"], a["mat_idx"], a["mats10"], a["emissive"])
+# the stages either side of the path have no CPU fallback either
+with pytest.raises(rt.B200RTError, match="no CUDA device"):
+    rt.BVH(a["tri9"], on_device=True)
+with pytest.raises(rt.B200RTError, match="no CUDA device"):
+    rt.quantise_rgba8(np.zeros((4, 4, 4), np.float32))
+"""
+
+
+def test_compute_fails_loudly_without_a_gpu():
+    """In a process that sees no CUDA device (CUDA_VISIBLE_DEVICES empty), so that GPU machines check it too."""
+    import subprocess
+    import sys
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="", PYTHONPATH=os.pathsep.join(p for p in (ROOT, os.environ.get("PYTHONPATH")) if p))
+    r = subprocess.run([sys.executable] + (["-s"] if sys.flags.no_user_site else []) + ["-c", NO_GPU_CHECK], env=env, cwd=ROOT,
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
 
 
 @pytest.mark.parametrize("key", ["cornell", "mis", "area"])
