@@ -283,6 +283,15 @@ void b200rt_host_free(void* p);
 int b200rt_trace_primary(b200rt_scene* scene, const float* camera17, int width, int height, int sample, int spp_for_seed,
                          int* prim_out, float* t_out, const b200rt_render_options* opts_or_null, b200rt_stats* stats_or_null);
 
+/* Per-pixel feature buffers for a denoiser (OIDN's "albedo" / "normal" auxiliary images; the reference feeds OIDN the beauty
+ * alone, utils.cpp:144-196): k x k stratified camera rays per pixel over its footprint, mean diffuse colour of the closest hit's
+ * material and mean geometric normal (not renormalised; misses contribute 0). k = 1: exactly b200rt_trace_primary's un-jittered ray.
+ * 3 floats per pixel each, row 0 = bottom; either output may be NULL (not both). opts: flags select the layout (as trace_primary);
+ * rank/world must be 0/1. Multi-device scene: computed on its first device. stats: rays = samples = w*h*k*k. */
+int b200rt_render_aovs(b200rt_scene* scene, const float* camera17, int width, int height, int samples_per_axis,
+                       float* albedo_rgb_out_or_null, float* normal_xyz_out_or_null,
+                       const b200rt_render_options* opts_or_null, b200rt_stats* stats_or_null);
+
 /* Replaces BVH::intersect / FlattenedBVH::intersect for a batch (source/bvh.cpp:62-65, flattened_bvh.cpp:10-58):
  * rays6 = {origin xyz, direction xyz}; extra8_or_null receives {point xyz, normal xyz, u, v} per ray. Host pointers.
  * any_hit != 0 returns 1/0 in prim_out (any triangle or sphere hit with t > 0) instead of the closest index. */
@@ -308,6 +317,10 @@ int b200rt_untile_accumulate_device(b200rt_scene* scene, const void* dev_gathere
 int b200rt_trace_primary_device(b200rt_scene* scene, const float* camera17, int width, int height, int sample, int spp_for_seed,
                                 void* dev_prim, void* dev_t, const b200rt_render_options* opts_or_null, void* cuda_stream,
                                 b200rt_stats* stats_or_null);
+/* device-pointer variant of b200rt_render_aovs (w*h*3 floats each, either may be NULL, not both) */
+int b200rt_render_aovs_device(b200rt_scene* scene, const float* camera17, int width, int height, int samples_per_axis,
+                              void* dev_albedo_rgb_or_null, void* dev_normal_xyz_or_null,
+                              const b200rt_render_options* opts_or_null, void* cuda_stream, b200rt_stats* stats_or_null);
 
 /* device-pointer variant of b200rt_trace_rays (dev_extra8 may be NULL) */
 int b200rt_trace_rays_device(b200rt_scene* scene, const void* dev_rays6, int n_rays, int any_hit, void* dev_prim, void* dev_t,
@@ -327,6 +340,10 @@ int b200rt_quantise_rgba8_device(const void* dev_image_rgba, int width, int heig
  * place — a functional stand-in, not a parity claim (DESIGN.md). channels: 3 (OIDN's float3 buffers) or 4 (Image). iterations <= 0
  * and sigma <= 0 select the defaults (5, 0.45). in == out is allowed. Host pointers; runs on the current device. */
 int b200rt_denoise(const float* image, int channels, int width, int height, float blend_factor, int iterations, float sigma, float* out);
+/* b200rt_denoise with OIDN's auxiliary images as edge-stopping guides (w*h*3 floats each, either may be NULL; b200rt_render_aovs
+ * computes them): a tap must also agree in normal direction and albedo to contribute. Both NULL: identical to b200rt_denoise, bit for bit. */
+int b200rt_denoise_guided(const float* image, int channels, const float* albedo_rgb_or_null, const float* normal_xyz_or_null,
+                          int width, int height, float blend_factor, int iterations, float sigma, float* out);
 
 const char* b200rt_last_error(void);
 const char* b200rt_version(void);

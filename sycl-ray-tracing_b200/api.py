@@ -253,13 +253,26 @@ def env_alias_table(skysphere):
     return prob, alias, total.value
 
 
-def OIDN_denoise(image, blend_factor: float = 1.0, iterations: int = 0, sigma: float = 0.0) -> np.ndarray:
+def OIDN_denoise(image, blend_factor: float = 1.0, iterations: int = 0, sigma: float = 0.0, albedo=None, normal=None) -> np.ndarray:
     """The denoise stage of main.cpp:118-120 (Utils::OIDN_denoise, utils.cpp:144-196) on the GPU: an edge-avoiding a-trous filter
-    standing in for OIDN (whose binaries the reference does not ship), then blend * denoised + (1 - blend) * noisy. (h, w, 3|4)."""
+    standing in for OIDN (whose binaries the reference does not ship), then blend * denoised + (1 - blend) * noisy. (h, w, 3|4).
+    albedo / normal: OIDN's auxiliary images, (h, w, 3) each (Scene.render_aovs), used as edge-stopping guides when given."""
     img = _f32(image.pixels if isinstance(image, Image) else image)
     h, w, ch = img.shape
+    guides = []
+    for name, g in (("albedo", albedo), ("normal", normal)):
+        if g is not None:
+            g = _f32(g)
+            if g.shape != (h, w, 3):
+                raise ValueError(f"{name} guide has shape {g.shape}, the image needs {(h, w, 3)}")
+        guides.append(g)
     out = np.empty_like(img)
-    B.check(B.load_library().b200rt_denoise(B.fptr(img), ch, w, h, blend_factor, iterations, sigma, B.fptr(out)))
+    L = B.load_library()
+    if albedo is None and normal is None:
+        B.check(L.b200rt_denoise(B.fptr(img), ch, w, h, blend_factor, iterations, sigma, B.fptr(out)))
+    else:
+        B.check(L.b200rt_denoise_guided(B.fptr(img), ch, B.fptr(guides[0]), B.fptr(guides[1]), w, h, blend_factor, iterations, sigma,
+                                        B.fptr(out)))
     return out
 
 
@@ -511,6 +524,17 @@ class Scene:
                                                       B.iptr(prim), B.fptr(t), C.byref(o), C.byref(st)))
         return st.as_dict()
 
+    def render_aovs(self, camera: Camera, w: int, h: int, samples_per_axis: int = 2, flags: int = 0):
+        """Feature buffers for a denoiser (b200rt_render_aovs): samples_per_axis^2 stratified camera rays per pixel; returns
+        ((h, w, 3) mean albedo, (h, w, 3) mean geometric normal (not renormalised, 0 on misses), stats)."""
+        albedo = np.empty((h, w, 3), np.float32)
+        normal = np.empty((h, w, 3), np.float32)
+        st = B.Stats()
+        o = self._opts(0, flags, 0, 1)
+        B.check(B.load_library().b200rt_render_aovs(self._h, B.fptr(camera.as_array17()), w, h, samples_per_axis, B.fptr(albedo),
+                                                    B.fptr(normal), C.byref(o), C.byref(st)))
+        return albedo, normal, st.as_dict()
+
     def trace_rays(self, rays6, any_hit: bool = False, flags: int = 0):
         rays6 = _f32(rays6).reshape(-1, 6)
         n = len(rays6)
@@ -560,6 +584,17 @@ class Scene:
         B.check(B.load_library().b200rt_trace_primary_device(self._h, B.fptr(camera.as_array17()), w, h, sample, spp_for_seed,
                                                              C.c_void_p(dev_prim_ptr), C.c_void_p(dev_t_ptr), C.byref(o),
                                                              C.c_void_p(stream_ptr), C.byref(st) if want_stats else None))
+        return st.as_dict() if want_stats else None
+
+    def render_aovs_device(self, camera: Camera, w, h, dev_albedo_ptr: int, dev_normal_ptr: int, samples_per_axis: int = 2,
+                           stream_ptr: int = 0, flags: int = 0, rank: int = 0, world: int = 1, want_stats: bool = False):
+        """render_aovs into device buffers of w*h*3 floats (either pointer may be 0, not both)."""
+        st = B.Stats()
+        o = self._opts(0, flags, rank, world)
+        B.check(B.load_library().b200rt_render_aovs_device(self._h, B.fptr(camera.as_array17()), w, h, samples_per_axis,
+                                                           C.c_void_p(dev_albedo_ptr) if dev_albedo_ptr else None,
+                                                           C.c_void_p(dev_normal_ptr) if dev_normal_ptr else None, C.byref(o),
+                                                           C.c_void_p(stream_ptr), C.byref(st) if want_stats else None))
         return st.as_dict() if want_stats else None
 
 

@@ -74,6 +74,7 @@ EXPORTS = [
     "b200rt_accum_create", "b200rt_accum_add", "b200rt_accum_samples", "b200rt_accum_resolve", "b200rt_accum_destroy",
     "b200rt_denoise", "b200rt_obj_load", "b200rt_obj_get", "b200rt_obj_destroy", "b200rt_hdr_load", "b200rt_hdr_get", "b200rt_hdr_destroy", "b200rt_env_cdf_search", "b200rt_render_rgba8", "b200rt_render_region", "b200rt_rng_stream", "b200rt_host_alloc", "b200rt_host_free", "b200rt_untile_accumulate_device",
     "b200rt_untile_device", "b200rt_trace_primary_device", "b200rt_trace_rays_device", "b200rt_quantise_rgba8", "b200rt_quantise_rgba8_device", "b200rt_last_error", "b200rt_version",
+    "b200rt_render_aovs", "b200rt_render_aovs_device", "b200rt_denoise_guided",
 ]
 
 _lib = None
@@ -114,6 +115,7 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
     L.b200rt_accum_destroy.argtypes = [VP]
     L.b200rt_accum_destroy.restype = None
     L.b200rt_denoise.argtypes = [FP, I, I, I, C.c_float, I, C.c_float, FP]
+    L.b200rt_denoise_guided.argtypes = [FP, I, FP, FP, I, I, C.c_float, I, C.c_float, FP]
     L.b200rt_obj_load.argtypes = [C.c_char_p, C.POINTER(VP)]
     L.b200rt_obj_get.argtypes = [VP, C.POINTER(FP), IP, C.POINTER(IP), C.POINTER(FP), IP, C.POINTER(IP), IP]
     L.b200rt_obj_destroy.argtypes = [VP]
@@ -146,6 +148,8 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
     L.b200rt_render_tiles_device.argtypes = [VP, FP, I, I, I, I, VP, C.POINTER(RenderOptions), VP, C.POINTER(Stats)]
     L.b200rt_untile_device.argtypes = [VP, VP, I, I, I, I, VP, VP]
     L.b200rt_trace_primary_device.argtypes = [VP, FP, I, I, I, I, VP, VP, C.POINTER(RenderOptions), VP, C.POINTER(Stats)]
+    L.b200rt_render_aovs.argtypes = [VP, FP, I, I, I, FP, FP, C.POINTER(RenderOptions), C.POINTER(Stats)]
+    L.b200rt_render_aovs_device.argtypes = [VP, FP, I, I, I, VP, VP, C.POINTER(RenderOptions), VP, C.POINTER(Stats)]
     L.b200rt_trace_rays_device.argtypes = [VP, VP, I, I, VP, VP, VP, C.POINTER(RenderOptions), VP, C.POINTER(Stats)]
     _lib = L
     return L

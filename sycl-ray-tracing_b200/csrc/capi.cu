@@ -1551,7 +1551,8 @@ int b200rt_quantise_rgba8(const float* image_rgba, int w, int h, int flip_y, uns
     return B200RT_OK;
 }
 
-int b200rt_denoise(const float* image, int channels, int w, int h, float blend, int iterations, float sigma, float* out)
+int b200rt_denoise_guided(const float* image, int channels, const float* albedo, const float* normal, int w, int h, float blend,
+                          int iterations, float sigma, float* out)
 {
     if (!image || !out || w <= 0 || h <= 0 || (channels != 3 && channels != 4)) return fail(B200RT_ERR_ARG, "bad denoise arguments");
     int n_dev = 0;
@@ -1559,20 +1560,86 @@ int b200rt_denoise(const float* image, int channels, int w, int h, float blend, 
     if (iterations <= 0) iterations = 5;
     if (iterations > 8) iterations = 8;
     if (!(sigma > 0.0f)) sigma = 0.45f;
-    const size_t bytes = (size_t)w * h * channels * sizeof(float);
-    float *d_in = nullptr, *d_tmp = nullptr, *d_out = nullptr;
+    const size_t bytes = (size_t)w * h * channels * sizeof(float), guide_bytes = (size_t)w * h * 3 * sizeof(float);
+    float *d_in = nullptr, *d_tmp = nullptr, *d_out = nullptr, *d_albedo = nullptr, *d_normal = nullptr;
     cudaError_t e = cudaSuccess;
     do
     {
         if ((e = cudaMalloc(&d_in, bytes)) != cudaSuccess) break;
         if ((e = cudaMalloc(&d_tmp, bytes)) != cudaSuccess) break;
         if ((e = cudaMalloc(&d_out, bytes)) != cudaSuccess) break;
+        if (albedo && (e = cudaMalloc(&d_albedo, guide_bytes)) != cudaSuccess) break;
+        if (normal && (e = cudaMalloc(&d_normal, guide_bytes)) != cudaSuccess) break;
         if ((e = cudaMemcpy(d_in, image, bytes, cudaMemcpyHostToDevice)) != cudaSuccess) break;
-        if ((e = launch_denoise(d_in, channels, w, h, iterations, sigma, blend, d_tmp, d_out, 0)) != cudaSuccess) break;
+        if (albedo && (e = cudaMemcpy(d_albedo, albedo, guide_bytes, cudaMemcpyHostToDevice)) != cudaSuccess) break;
+        if (normal && (e = cudaMemcpy(d_normal, normal, guide_bytes, cudaMemcpyHostToDevice)) != cudaSuccess) break;
+        if ((e = launch_denoise(d_in, channels, d_albedo, d_normal, w, h, iterations, sigma, blend, d_tmp, d_out, 0)) != cudaSuccess) break;
         if ((e = cudaMemcpy(out, d_out, bytes, cudaMemcpyDeviceToHost)) != cudaSuccess) break;
     } while (0);
-    cudaFree(d_in); cudaFree(d_tmp); cudaFree(d_out);
+    cudaFree(d_in); cudaFree(d_tmp); cudaFree(d_out); cudaFree(d_albedo); cudaFree(d_normal);
     if (e != cudaSuccess) return fail(B200RT_ERR_CUDA, "denoise: %s", cudaGetErrorString(e));
+    return B200RT_OK;
+}
+
+int b200rt_denoise(const float* image, int channels, int w, int h, float blend, int iterations, float sigma, float* out)
+{
+    return b200rt_denoise_guided(image, channels, nullptr, nullptr, w, h, blend, iterations, sigma, out);
+}
+
+int b200rt_render_aovs_device(b200rt_scene* s, const float* camera17, int w, int h, int samples_per_axis, void* dev_albedo, void* dev_normal,
+                              const b200rt_render_options* opts, void* cuda_stream, b200rt_stats* stats)
+{
+    RenderParams P;
+    int rc = make_params(s, camera17, w, h, 1, 1, opts, P);
+    if (rc) return rc;
+    if (samples_per_axis < 1 || samples_per_axis > 16) return fail(B200RT_ERR_ARG, "samples_per_axis %d outside 1..16", samples_per_axis);
+    if (!dev_albedo && !dev_normal) return fail(B200RT_ERR_ARG, "at least one of the albedo / normal outputs must be given");
+    if (P.world != 1) return fail(B200RT_ERR_ARG, "feature buffers are computed for whole frames (rank/world must stay 0/1)");
+    ON_DEVICE(s->device);
+    if ((rc = ensure_scratch(s, 0, 0, 0))) return rc;
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    if (stats) CU(cudaEventRecord(s->ev0, st));
+    CU(launch_aov(s->dev, P, samples_per_axis, (float*)dev_albedo, (float*)dev_normal, st));
+    if (stats)
+    {
+        CU(cudaEventRecord(s->ev1, st));
+        CU(cudaEventSynchronize(s->ev1));
+        float ms = 0.0f;
+        CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+        std::memset(stats, 0, sizeof(*stats));
+        stats->kernel_ms = ms; stats->total_ms = ms; stats->gpu_launches = 1;
+        stats->rays = stats->samples = (unsigned long long)w * h * samples_per_axis * samples_per_axis;
+    }
+    return B200RT_OK;
+}
+
+int b200rt_render_aovs(b200rt_scene* s, const float* camera17, int w, int h, int samples_per_axis, float* albedo_out, float* normal_out,
+                       const b200rt_render_options* opts, b200rt_stats* stats)
+{
+    if (!s) return fail(B200RT_ERR_ARG, "NULL scene");
+    if (!albedo_out && !normal_out) return fail(B200RT_ERR_ARG, "at least one of the albedo / normal outputs must be given");
+    if (w <= 0 || h <= 0) return fail(B200RT_ERR_ARG, "bad frame size");
+    auto t0 = std::chrono::high_resolution_clock::now();
+    ON_DEVICE(s->device);
+    const size_t bytes = (size_t)w * h * 3 * sizeof(float);
+    float *d_albedo = nullptr, *d_normal = nullptr;
+    int rc = B200RT_OK;
+    do
+    {
+        cudaError_t e = cudaSuccess;
+        if (albedo_out && (e = cudaMalloc(&d_albedo, bytes)) != cudaSuccess) { rc = fail(B200RT_ERR_CUDA, "render_aovs: %s", cudaGetErrorString(e)); break; }
+        if (normal_out && (e = cudaMalloc(&d_normal, bytes)) != cudaSuccess) { rc = fail(B200RT_ERR_CUDA, "render_aovs: %s", cudaGetErrorString(e)); break; }
+        if ((rc = b200rt_render_aovs_device(s, camera17, w, h, samples_per_axis, d_albedo, d_normal, opts, nullptr, stats))) break;
+        if (albedo_out && (rc = copy_to_host(s, albedo_out, d_albedo, bytes, 0))) break;
+        if (normal_out && (rc = copy_to_host(s, normal_out, d_normal, bytes, 0))) break;
+    } while (0);
+    cudaFree(d_albedo); cudaFree(d_normal);
+    if (rc) return rc;
+    if (stats)
+    {
+        stats->d2h_bytes = (albedo_out ? bytes : 0) + (normal_out ? bytes : 0); stats->h2d_bytes = 17 * sizeof(float);
+        stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::high_resolution_clock::now() - t0).count();
+    }
     return B200RT_OK;
 }
 

@@ -216,6 +216,42 @@ __global__ void __launch_bounds__(256) k_primary(SceneDev S, RenderParams P, int
     t_out[idx] = found ? h.t : -1.0f;
 }
 
+// ---- feature buffers for a denoiser (OIDN's "albedo" / "normal"): k x k stratified camera rays per pixel ------------------------
+// The grid covers [x - 0.5, x + 0.5) like the beauty's jitter (x + 0.5 + r - 1, :88-89), so the guides are anti-aliased like the
+// beauty; k = 1 is exactly k_primary's un-jittered ray. Per ray: the diffuse colour of the closest hit's material (the BRDF's base
+// colour) and its geometric normal (hit_geometry: never flipped); a miss adds 0. Outputs are the means over the k^2 rays, the
+// normal not renormalised (a partly covered pixel has length < 1). No RNG: deterministic.
+template <int TL>
+__global__ void __launch_bounds__(256) k_aov(SceneDev S, RenderParams P, int k, float* __restrict__ albedo_out, float* __restrict__ normal_out)
+{
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (warp >= P.n_rank_tiles * 8) return;
+    const PixelSlot ps = unit_pixel(P, warp, lane);
+    if (!ps.inside) return;
+    col a = CO(0.0f, 0.0f, 0.0f);
+    v3 n = V(0.0f, 0.0f, 0.0f);
+    for (int j = 0; j < k; j++)
+        for (int i = 0; i < k; i++)
+        {
+            const float fx = (float)ps.x + (((float)i + 0.5f) / (float)k - 0.5f);
+            const float fy = (float)ps.y + (((float)j + 0.5f) / (float)k - 0.5f);
+            v3 o, d;
+            camera_ray(P.cam, fx, fy, o, d);
+            Hit h;
+            if (!trace_ray<TL>(S, o, d, 0.0f, TRACE_CLOSEST, h)) continue;
+            const MaterialDev m = S.mats[__ldg(S.mat_idx + h.prim)];
+            a = a + CO(m.dr, m.dg, m.db);
+            v3 p, hn;
+            hit_geometry(S, h, o, d, p, hn);
+            n = n + hn;
+        }
+    const float rays = (float)(k * k);
+    const size_t idx = 3 * ((size_t)ps.y * P.cam.w + ps.x);
+    if (albedo_out) { albedo_out[idx] = a.r / rays; albedo_out[idx + 1] = a.g / rays; albedo_out[idx + 2] = a.b / rays; }
+    if (normal_out) { normal_out[idx] = n.x / rays; normal_out[idx + 1] = n.y / rays; normal_out[idx + 2] = n.z / rays; }
+}
+
 // ---- ray batches (BVH::intersect / FlattenedBVH::intersect replacement for tests and tools) ------------------------------
 template <int TL>
 __global__ void __launch_bounds__(256) k_trace_rays(SceneDev S, const float* __restrict__ rays6, int n, int any_hit,
@@ -412,6 +448,18 @@ cudaError_t launch_primary(const SceneDev& S, const RenderParams& P, int sample,
     if (tl == TL_WIDE) k_primary<TL_WIDE><<<grid, 256, 0, stream>>>(S, P, sample, prim_out, t_out);
     else if (tl == TL_DIAG) k_primary<TL_DIAG><<<grid, 256, 0, stream>>>(S, P, sample, prim_out, t_out);
     else k_primary<TL_AXIS><<<grid, 256, 0, stream>>>(S, P, sample, prim_out, t_out);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_aov(const SceneDev& S, const RenderParams& P, int k, float* albedo_out, float* normal_out, cudaStream_t stream)
+{
+    const int n_warps = P.n_rank_tiles * 8;
+    if (n_warps <= 0) return cudaSuccess;
+    const int grid = (n_warps * 32 + 255) / 256;
+    const int tl = traversal_layout(S, P.flags, true);
+    if (tl == TL_WIDE) k_aov<TL_WIDE><<<grid, 256, 0, stream>>>(S, P, k, albedo_out, normal_out);
+    else if (tl == TL_DIAG) k_aov<TL_DIAG><<<grid, 256, 0, stream>>>(S, P, k, albedo_out, normal_out);
+    else k_aov<TL_AXIS><<<grid, 256, 0, stream>>>(S, P, k, albedo_out, normal_out);
     return cudaGetLastError();
 }
 

@@ -28,6 +28,8 @@ int tile_skew();
 cudaError_t launch_megakernel(const SceneDev& S, const RenderParams& P, const float4* fb_in_rowmajor, float4* out_tiles,
                               unsigned int* work_counter, unsigned long long* ray_counter, cudaStream_t stream);
 cudaError_t launch_primary(const SceneDev& S, const RenderParams& P, int sample, int* prim_out, float* t_out, cudaStream_t stream);
+// feature buffers (k x k stratified camera rays per pixel): mean albedo and geometric normal, 3 floats per pixel each, either may be null
+cudaError_t launch_aov(const SceneDev& S, const RenderParams& P, int k, float* albedo_out, float* normal_out, cudaStream_t stream);
 cudaError_t launch_trace_rays(const SceneDev& S, const float* rays6, int n, int any_hit, int flags, int* prim_out, float* t_out,
                               float* extra8, cudaStream_t stream);
 cudaError_t launch_untile(const float4* tiles, int tiles_per_rank_padded, int world, int only_rank, int w, int h, float4* image,
@@ -40,9 +42,9 @@ cudaError_t launch_env_cdf_search(const SceneDev& S, const float* values, int n,
 cudaError_t launch_rng_stream(int x, int y, int spp, int n, uint32_t* state_out, float* floats_out, cudaStream_t stream);
 cudaError_t launch_quantise_rgba8(const float4* image, int w, int h, int flip_y, void* out_rgba8, cudaStream_t stream);
 
-// output stage: edge-avoiding a-trous denoiser (denoise.cu)
-cudaError_t launch_denoise(const float* d_in, int channels, int w, int h, int iterations, float sigma, float blend, float* d_tmp, float* d_out,
-                           cudaStream_t stream);
+// output stage: edge-avoiding a-trous denoiser (denoise.cu); d_albedo / d_normal: optional w*h*3 guides (both null: colour only)
+cudaError_t launch_denoise(const float* d_in, int channels, const float* d_albedo, const float* d_normal, int w, int h, int iterations,
+                           float sigma, float blend, float* d_tmp, float* d_out, cudaStream_t stream);
 
 // K5 env tables (env_tables.cu)
 cudaError_t launch_env_expand_rgb(const float* rgb, size_t n, float4* rgba, cudaStream_t stream);
