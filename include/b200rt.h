@@ -184,15 +184,9 @@ void b200rt_hdr_destroy(b200rt_hdr* hdr);
                                             group stream while the tile groups overlap as in a normal frame, and the events are read after the frame.
                                             stats: trace_ms / shade_ms = summed launch durations (they overlap: the sum may exceed the frame),
                                             trace_union_ms = time during which at least one trace kernel was running */
-#define B200RT_FLAG_WF_PASSES_ONLY 1024  /* wavefront ablation: trace / shade passes to the last pixel, no barrier-free continuation */
-#define B200RT_FLAG_WF_ASYNC 2048        /* wavefront study: the continuation is wf_async (csrc/async.cu: shader warps own chunks of 32 slots, every ray of
-                                            the group is traced by whichever tracer lane is free, through a device-wide ticket ring) instead of the
-                                            default wf_tail (csrc/persist.cu: every warp finishes a few slots of its own). Also: B200RT_WF_ASYNC=1.
-                                            Bit-identical frames; measured slower on every configuration (DESIGN.md 4.3), hence not the default */
-#define B200RT_FLAG_WF_DETACH 4096        /* wavefront study: after B200RT_WF_DETACH_AT passes (default 36) the B200RT_WF_DETACH_SLOTS pixels of a device that lag
-                                            furthest behind leave the passes for a barrier-free kernel on a stream of its own (csrc/persist.cu
-                                            launch_wavefront_detach). Bit-identical; the detached pixels run 1.5-2.3x faster per step, the passes that share
-                                            the machine with them slower: no net gain (DESIGN.md 4.3), hence not the default. Also: B200RT_WF_DETACH=1 */
+#define B200RT_FLAG_WF_PASSES_ONLY 1024  /* wavefront ablation: trace / shade passes to the last pixel; the default hands the last few pixels of
+                                            each tile group to one barrier-free tail launch (csrc/persist.cu wf_tail) instead */
+/* flag bits 2048 and 4096 are retired: the library ignores them, and they must not be reused */
 #define B200RT_FLAG_LINEAR_TILES 256     /* b200rt_render_tiles_device: the tile buffer receives each pixel's mean radiance (`final_color / spp`,
                                             render_kernel.cpp:167) instead of the tone-mapped value; b200rt_untile_accumulate_device then does
                                             `framebuffer += final; tone map` (:169-180) on the gathering device, so the incoming framebuffer is

@@ -27,8 +27,6 @@ FLAG_TIME_KERNELS = 128
 FLAG_LINEAR_TILES = 256
 FLAG_TIME_INLINE = 512
 FLAG_WF_PASSES_ONLY = 1024
-FLAG_WF_ASYNC = 2048
-FLAG_WF_DETACH = 4096
 TILE_DIM = 16
 TILE_PIXELS = 256
 

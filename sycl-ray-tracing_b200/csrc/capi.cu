@@ -152,7 +152,7 @@ int make_params(const b200rt_scene* s, const float* camera17, int w, int h, int 
     P.n_rank_tiles = b200rt_tiles_for_rank(w, h, d.rank, d.world);
     P.flags = d.flags;
     P.rx0 = P.ry0 = P.rw = P.rh = 0;
-    P.sample_begin = 0; P.sample_end = spp; P.stamp0 = 0; P.acc_rng = nullptr; P.acc_sum = nullptr;
+    P.sample_begin = 0; P.sample_end = spp; P.acc_rng = nullptr; P.acc_sum = nullptr;
     return B200RT_OK;
 }
 
@@ -282,12 +282,23 @@ int copy_to_host(b200rt_scene* s, void* dst_host, const void* src_dev, size_t by
 }
 
 template <typename T>
-cudaError_t wf_alloc(b200rt_scene* s, T** p, size_t n)
+cudaError_t wf_alloc(std::vector<void*>& allocs, T** p, size_t n)
 {
     void* d = nullptr;
     cudaError_t e = cudaMalloc(&d, n * sizeof(T));
-    if (e == cudaSuccess) { s->wf_allocs.push_back(d); *p = (T*)d; }
+    if (e == cudaSuccess) { allocs.push_back(d); *p = (T*)d; }
     return e;
+}
+
+// the arrays of a WfBuffers of n slots; every allocation is recorded in `allocs`, whose owner frees them
+int alloc_wf_buffers(std::vector<void*>& allocs, WfBuffers& w, size_t n)
+{
+    CU(wf_alloc(allocs, &w.rng, n)); CU(wf_alloc(allocs, &w.sample, n)); CU(wf_alloc(allocs, &w.bounce, n)); CU(wf_alloc(allocs, &w.flags, n));
+    CU(wf_alloc(allocs, &w.final_c, n)); CU(wf_alloc(allocs, &w.sample_c, n)); CU(wf_alloc(allocs, &w.thr, n)); CU(wf_alloc(allocs, &w.thr_next, n));
+    CU(wf_alloc(allocs, &w.ray_o, 5 * n)); CU(wf_alloc(allocs, &w.ray_d, 5 * n)); CU(wf_alloc(allocs, &w.side_w, 4 * n));
+    CU(wf_alloc(allocs, &w.res, 5 * n));
+    CU(wf_alloc(allocs, &w.queue, 5 * n)); CU(wf_alloc(allocs, &w.counters, (size_t)8)); CU(wf_alloc(allocs, &w.rays_total, (size_t)1));
+    return B200RT_OK;
 }
 
 // tile groups (independent iteration chains on their own streams). 3 for a full 1080p frame; a rank that holds a fraction of it
@@ -310,11 +321,8 @@ int ensure_wavefront(b200rt_scene* s, const RenderParams& P)
         for (int g = 0; g < kMaxWfGroups; g++)
         {
             CU(cudaStreamCreateWithFlags(&s->wf[g].stream, cudaStreamNonBlocking));
-            CU(cudaStreamCreateWithFlags(&s->wf[g].detach_stream, cudaStreamNonBlocking));
             CU(cudaEventCreateWithFlags(&s->wf[g].poll_event, cudaEventDisableTiming));
             CU(cudaEventCreateWithFlags(&s->wf[g].join_event, cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&s->wf[g].detach_ready, cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&s->wf[g].detach_join, cudaEventDisableTiming));
             s->wf[g].host_active = s->h_active + g;
         }
     }
@@ -336,41 +344,11 @@ int ensure_wavefront(b200rt_scene* s, const RenderParams& P)
         s->wf_allocs.clear();
         for (int g = 0; g < G; g++)
         {
-            WfBuffers& w = s->wf[g].buf;
-            const size_t n = (size_t)most;
             s->wf_cap[g] = most;
-            CU(wf_alloc(s, &w.rng, n)); CU(wf_alloc(s, &w.sample, n)); CU(wf_alloc(s, &w.bounce, n)); CU(wf_alloc(s, &w.flags, n));
-            CU(wf_alloc(s, &w.final_c, n)); CU(wf_alloc(s, &w.sample_c, n)); CU(wf_alloc(s, &w.thr, n)); CU(wf_alloc(s, &w.thr_next, n));
-            CU(wf_alloc(s, &w.ray_o, 5 * n)); CU(wf_alloc(s, &w.ray_d, 5 * n)); CU(wf_alloc(s, &w.side_w, 4 * n));
-            CU(wf_alloc(s, &w.res, 5 * n));
-            CU(wf_alloc(s, &w.queue, 5 * n)); CU(wf_alloc(s, &w.counters, 8)); CU(wf_alloc(s, &w.rays_total, 1));
-            s->wf[g].dmem = WfDetachMem{};          // the study paths' memory is allocated below, when a frame asks for them
-            s->wf[g].amem = WfAsyncMem{};
+            const int rc = alloc_wf_buffers(s->wf_allocs, s->wf[g].buf, (size_t)most);
+            if (rc) return rc;
         }
         s->wf_groups = G;
-    }
-    // study paths (DESIGN.md 4.3), only when a frame asks for them: the early hand-over of a group's lagging pixels (persist.cu: control
-    // words, the list, the tail kernel's private queues) and the ray ring + per-chunk counts of the cross-warp continuation (async.cu);
-    // sized for the groups' capacity, freed with the rest
-    const auto env_on = [](const char* name) { const char* e = getenv(name); return e && atoi(e) != 0; };
-    const bool want_detach = s->dev.has_wide && ((P.flags & B200RT_FLAG_WF_DETACH) || env_on("B200RT_WF_DETACH"));
-    const bool want_async = s->dev.has_wide && ((P.flags & B200RT_FLAG_WF_ASYNC) || env_on("B200RT_WF_ASYNC"));
-    for (int g = 0; g < G; g++)
-    {
-        WfDetachMem& dm = s->wf[g].dmem;
-        if (want_detach && !dm.list)
-        {
-            dm.list_words = 65536; dm.ctas = wavefront_tail_max_ctas();
-            CU(wf_alloc(s, &dm.ctl, (size_t)wavefront_detach_ctl_words())); CU(wf_alloc(s, &dm.list, (size_t)dm.list_words));
-            CU(wf_alloc(s, &dm.queue, (size_t)wavefront_detach_queue_words(dm.ctas)));
-        }
-        WfAsyncMem& a = s->wf[g].amem;
-        if (want_async && !a.ray_ring && wavefront_async_fits(s->wf_cap[g]))
-        {
-            a.ray_log2 = wavefront_async_ray_log2(s->wf_cap[g]); a.chunk_words = wavefront_async_chunk_words(s->wf_cap[g]);
-            CU(wf_alloc(s, &a.ray_ring, (size_t)1 << a.ray_log2)); CU(wf_alloc(s, &a.ctrl, 64));
-            CU(wf_alloc(s, &a.chunk_cnt, (size_t)a.chunk_words)); CU(wf_alloc(s, &a.chunk_live, (size_t)a.chunk_words));
-        }
     }
     for (int g = 0; g < G; g++)
     {
@@ -379,15 +357,6 @@ int ensure_wavefront(b200rt_scene* s, const RenderParams& P)
         s->wf[g].buf.tile_offset = g;
     }
     return B200RT_OK;
-}
-
-template <typename T>
-cudaError_t pw_alloc(b200rt_scene* s, T** p, size_t n)
-{
-    void* d = nullptr;
-    cudaError_t e = cudaMalloc(&d, n * sizeof(T));
-    if (e == cudaSuccess) { s->pw_allocs.push_back(d); *p = (T*)d; }
-    return e;
 }
 
 int ensure_persistent(b200rt_scene* s)
@@ -399,12 +368,8 @@ int ensure_persistent(b200rt_scene* s)
     for (void* p : s->pw_allocs) cudaFree(p);
     s->pw_allocs.clear(); s->pw_cap = 0;
     WfBuffers& w = s->pw;
-    const size_t m = (size_t)n;
-    CU(pw_alloc(s, &w.rng, m)); CU(pw_alloc(s, &w.sample, m)); CU(pw_alloc(s, &w.bounce, m)); CU(pw_alloc(s, &w.flags, m));
-    CU(pw_alloc(s, &w.final_c, m)); CU(pw_alloc(s, &w.sample_c, m)); CU(pw_alloc(s, &w.thr, m)); CU(pw_alloc(s, &w.thr_next, m));
-    CU(pw_alloc(s, &w.ray_o, 5 * m)); CU(pw_alloc(s, &w.ray_d, 5 * m)); CU(pw_alloc(s, &w.side_w, 4 * m));
-    CU(pw_alloc(s, &w.res, 5 * m));
-    CU(pw_alloc(s, &w.queue, 5 * m)); CU(pw_alloc(s, &w.counters, (size_t)8)); CU(pw_alloc(s, &w.rays_total, (size_t)1));
+    const int rc = alloc_wf_buffers(s->pw_allocs, w, (size_t)n);
+    if (rc) return rc;
     w.n_slots = n; w.tile_stride = 1; w.tile_offset = 0;
     s->pw_cap = n;
     return B200RT_OK;
@@ -991,11 +956,8 @@ void b200rt_scene_destroy(b200rt_scene* s)
         for (int g = 0; g < kMaxWfGroups; g++)
         {
             if (s->wf[g].stream) cudaStreamDestroy(s->wf[g].stream);
-            if (s->wf[g].detach_stream) cudaStreamDestroy(s->wf[g].detach_stream);
             if (s->wf[g].poll_event) cudaEventDestroy(s->wf[g].poll_event);
             if (s->wf[g].join_event) cudaEventDestroy(s->wf[g].join_event);
-            if (s->wf[g].detach_ready) cudaEventDestroy(s->wf[g].detach_ready);
-            if (s->wf[g].detach_join) cudaEventDestroy(s->wf[g].detach_join);
         }
         cudaEventDestroy(s->fork_event);
         cudaFreeHost(s->h_active);

@@ -97,7 +97,6 @@ struct RenderParams
     // (31 + x*y*spp, render_kernel.cpp:77). acc_rng / acc_sum (indexed like the tile buffer) carry each pixel's generator state
     // and radiance sum from one launch to the next; null = an ordinary one-shot frame (sample_begin = 0, sample_end = spp).
     int sample_begin, sample_end;
-    int stamp0;                // wavefront: first value of the per-slot shading-step counter of this frame (results carry it as a stamp)
     uint32_t* acc_rng;
     float4* acc_sum;
 };
@@ -111,7 +110,7 @@ struct WfBuffers
     float4* final_c; float4* sample_c; float4* thr; float4* thr_next;
     float4* ray_o; float4* ray_d;             // [5 * n_slots]: k * n_slots + slot; k = 0..3 side rays, 4 = path ray; .w = tmax / ray kind
     float4* side_w;                           // [4 * n_slots]: MIS-weighted contribution if unoccluded (.w = direction pdf for k = 1)
-    float4* res;                              // [5 * n_slots]: {t, primitive (closest hit) | occlusion flag, triangle slot, stamp} of each ray
+    float4* res;                              // [5 * n_slots]: {t, primitive (closest hit) | occlusion flag, triangle slot, -} of each ray
     unsigned int* queue;                      // [5 * n_slots]: (slot << 3) | k
     unsigned int* counters;                   // [2] = pixels still rendering, [3], [4] = ping-pong queue lengths
     unsigned long long* rays_total;
@@ -119,29 +118,12 @@ struct WfBuffers
 
 constexpr int kMaxWfGroups = 8;
 
-// device memory of the barrier-free continuation (async.cu): the ray ring, its counters (64 words), and per chunk of 32 slots the
-// count of outstanding rays and of unfinished slots; null until the group was allocated with it
-struct WfAsyncMem
-{
-    unsigned int* ray_ring; unsigned int* ctrl; unsigned int* chunk_cnt; unsigned int* chunk_live;
-    int ray_log2, chunk_words;
-};
-
-// device memory of the early hand-over of a group's lagging pixels to a barrier-free kernel (persist.cu: launch_wavefront_detach)
-struct WfDetachMem
-{
-    unsigned int* ctl; unsigned int* list; unsigned int* queue;
-    int list_words, ctas;
-};
-
 // one interleaved tile group of the wavefront integrator: its state, stream and polling resources
 struct WfGroup
 {
     WfBuffers buf;
-    WfAsyncMem amem;
-    WfDetachMem dmem;
-    cudaStream_t stream, detach_stream;
-    cudaEvent_t poll_event, join_event, detach_ready, detach_join;
+    cudaStream_t stream;
+    cudaEvent_t poll_event, join_event;
     unsigned int* host_active;      // pinned
 };
 

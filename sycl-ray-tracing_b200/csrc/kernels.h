@@ -84,19 +84,6 @@ cudaError_t wavefront_sum_rays(const WfGroup* groups, int n_groups, unsigned lon
 cudaError_t launch_wavefront_tail(const SceneDev& S, const RenderParams& P, const WfBuffers& B, int max_ctas, const float4* fb_in_rowmajor,
                                   float4* out_tiles, cudaStream_t stream);
 int wavefront_tail_max_ctas();
-// the lagging pixels of a group leave the passes early (persist.cu)
-int wavefront_detach_ctl_words();
-int wavefront_detach_queue_words(int ctas);
-cudaError_t launch_wavefront_detach(const SceneDev& S, const RenderParams& P, const WfBuffers& B, const WfDetachMem& D, unsigned int budget, int ctas,
-                                    const float4* fb_in_rowmajor, float4* out_tiles, cudaStream_t stream, cudaStream_t detach_stream, cudaEvent_t ready);
-
-// barrier-free continuation that pools rays and shading work across warps through device-wide ticket rings (async.cu)
-int wavefront_async_ray_log2(int n_slots);
-int wavefront_async_chunk_words(int n_slots);
-bool wavefront_async_fits(int n_slots);
-int wavefront_async_max_ctas();
-cudaError_t launch_wavefront_async(const SceneDev& S, const RenderParams& P, const WfBuffers& B, const WfAsyncMem& M, int ctas,
-                                   const float4* fb_in_rowmajor, float4* out_tiles, cudaStream_t stream);
 
 // persistent integrator (persist.cu): one launch per frame, every warp its own wavefront machine
 int persistent_grid();

@@ -131,13 +131,13 @@ pt_persist(SceneDev S, RenderParams P, WfBuffers B, unsigned int* next_pixel, in
 __global__ void __launch_bounds__(256) wf_compact_active(WfBuffers B, unsigned int* list, unsigned int* n_active)
 {
     const int slot = blockIdx.x * blockDim.x + threadIdx.x;
-    const bool alive = slot < B.n_slots && !(B.flags[slot] & (WF_DONE | WF_DETACHED));
+    const bool alive = slot < B.n_slots && !(B.flags[slot] & WF_DONE);
     wf_enqueue(list, n_active, alive, (unsigned int)slot);
 }
 
 __global__ void __launch_bounds__(32 * kCoopMaxWarps, PERSIST_MIN_BLOCKS)
 wf_tail(SceneDev S, RenderParams P, WfBuffers B, const unsigned int* list, const unsigned int* n_active_ptr, unsigned int* claim_counter,
-        unsigned int* queue_mem, const float4* __restrict__ fb_in_rowmajor, float4* __restrict__ out_tiles, int detached)
+        unsigned int* queue_mem, const float4* __restrict__ fb_in_rowmajor, float4* __restrict__ out_tiles)
 {
     __shared__ CoopWarp s_warps[kCoopMaxWarps];
     __shared__ uint2 s_stack[kSharedStackDepth * 32 * kCoopMaxWarps];
@@ -168,8 +168,7 @@ wf_tail(SceneDev S, RenderParams P, WfBuffers B, const unsigned int* list, const
         int st = mine ? B.flags[slot] : WF_DONE;
         int x = 0, y = 0;
         if (mine) wf_slot_pixel(P, slot, x, y);
-        // detached slots (wf_detach_mark) were taken out between a trace and a shade pass: their results wait to be shaded
-        bool first_iteration = detached == 0;
+        bool first_iteration = true;
         for (;;)
         {
             ShadeOut R;
@@ -226,7 +225,7 @@ wf_tail(SceneDev S, RenderParams P, WfBuffers B, const unsigned int* list, const
     if (lane == 0)
     {
         if (rays) atomicAdd(B.rays_total, rays);
-        if (finished_pixels && !detached) atomicSub(&B.counters[2], finished_pixels);     // (detached slots left the count when they were marked)
+        if (finished_pixels) atomicSub(&B.counters[2], finished_pixels);
     }
 }
 
@@ -242,86 +241,7 @@ cudaError_t launch_wavefront_tail(const SceneDev& S, const RenderParams& P, cons
     // private queues: 160 words per warp behind the list -> at most (4 * n_slots) / 160 warps
     const int max_warps = std::max(1, (int)(((size_t)4 * B.n_slots) / 160));
     int ctas = std::min(max_ctas, std::max(1, max_warps / kCoopMaxWarps));
-    wf_tail<<<ctas, 32 * kCoopMaxWarps, 0, stream>>>(S, P, B, B.queue, B.counters + 6, B.counters + 7, B.queue + B.n_slots, fb_in_rowmajor, out_tiles, 0);
-    return cudaGetLastError();
-}
-
-// ---- the lagging pixels leave the passes early --------------------------------------------------------------------------------------------
-// A tile group's chain of passes is as long as its slowest pixel's: spp * (bounces + 1) = 576 on C3 for the few pixels whose every
-// path runs to the last bounce, ~190 us per pass when a rank holds 1/8 of a frame — however few pixels are still alive. After
-// `detach_at` passes a pixel's sample index tells how long its chain is going to be (a pixel that has finished s samples in p passes
-// needs p / s passes per sample). The `budget` pixels that lag furthest behind are taken out of the passes, between a trace and a
-// shade pass, and one wf_tail launch on a stream of its own runs them to the end barrier-free (~1.6x faster per step when every ray
-// has a lane), while the passes go on for the others and end when THEIR slowest pixel ends. Same device functions, same per-pixel
-// RNG streams: the frame stays bit-identical.
-// Status: a study path (B200RT_FLAG_WF_DETACH), tested, NOT the default: the detached pixels do run faster (81 us per step for 256 of
-// them per group on one rank of 8), but the passes are bound by the bulk of the object's pixels, not by the few deepest, and slow down
-// when the detached kernels take a share of every SM — no net gain (DESIGN.md 4.3, profiles/r2g_detach_lagging_pixels_64spp.txt).
-constexpr int kLagBins = 1024;
-
-__global__ void __launch_bounds__(256) wf_lag_histogram(WfBuffers B, int sample_begin, unsigned int* hist)
-{
-    __shared__ unsigned int sh[kLagBins];
-    for (int i = threadIdx.x; i < kLagBins; i += blockDim.x) sh[i] = 0u;
-    __syncthreads();
-    const int slot = blockIdx.x * blockDim.x + threadIdx.x;
-    if (slot < B.n_slots && !(B.flags[slot] & (WF_DONE | WF_DETACHED)))
-        atomicAdd(&sh[min(max(B.sample[slot] - sample_begin, 0), kLagBins - 1)], 1u);
-    __syncthreads();
-    for (int i = threadIdx.x; i < kLagBins; i += blockDim.x) if (sh[i]) atomicAdd(&hist[i], sh[i]);
-}
-
-// ctl[0] = the largest sample count s such that at most `budget` unfinished pixels have finished <= s samples (-1: none), ctl[1] = how many
-__global__ void wf_lag_threshold(const unsigned int* hist, unsigned int budget, int* ctl)
-{
-    unsigned int cum = 0u;
-    int thr = -1;
-    for (int b = 0; b < kLagBins - 1; b++)
-    {
-        if (cum + hist[b] > budget) break;
-        cum += hist[b];
-        thr = b;
-    }
-    ctl[0] = thr; ctl[1] = (int)cum;
-}
-
-__global__ void __launch_bounds__(256) wf_detach_mark(WfBuffers B, int sample_begin, const int* ctl, unsigned int* list, unsigned int* n_listed)
-{
-    const int slot = blockIdx.x * blockDim.x + threadIdx.x;
-    bool sel = false;
-    if (slot < B.n_slots)
-    {
-        const int st = B.flags[slot];
-        sel = !(st & (WF_DONE | WF_DETACHED)) && B.sample[slot] - sample_begin <= ctl[0];
-        if (sel) B.flags[slot] = st | WF_DETACHED;
-    }
-    const unsigned int m = __ballot_sync(0xffffffffu, sel);
-    if ((threadIdx.x & 31) == 0 && m) atomicSub(&B.counters[2], (unsigned int)__popc(m));      // the passes' count of unfinished pixels
-    wf_enqueue(list, n_listed, sel, (unsigned int)slot);
-}
-
-int wavefront_detach_ctl_words() { return kLagBins + 8; }
-int wavefront_detach_queue_words(int ctas) { return ctas * kCoopMaxWarps * 160; }
-
-// D: ctl = kLagBins + 8 words, list = at least `budget` words, queue = wavefront_detach_queue_words(ctas). Enqueues on `stream` (the
-// group's pass stream, between a trace and a shade launch) the selection, and on `detach_stream` — behind `ready` — the kernel.
-cudaError_t launch_wavefront_detach(const SceneDev& S, const RenderParams& P, const WfBuffers& B, const WfDetachMem& D, unsigned int budget, int ctas,
-                                    const float4* fb_in_rowmajor, float4* out_tiles, cudaStream_t stream, cudaStream_t detach_stream, cudaEvent_t ready)
-{
-    if (B.n_slots <= 0 || budget == 0u) return cudaSuccess;
-    cudaError_t e;
-    if ((e = cudaMemsetAsync(D.ctl, 0, (size_t)wavefront_detach_ctl_words() * sizeof(unsigned int), stream)) != cudaSuccess) return e;
-    unsigned int* hist = D.ctl;
-    int* thr = (int*)(D.ctl + kLagBins);                 // [0] threshold, [1] count
-    unsigned int* n_listed = D.ctl + kLagBins + 2;
-    unsigned int* claim = D.ctl + kLagBins + 3;
-    const int grid = (B.n_slots + 255) / 256;
-    wf_lag_histogram<<<grid, 256, 0, stream>>>(B, P.sample_begin, hist);
-    wf_lag_threshold<<<1, 1, 0, stream>>>(hist, budget, thr);
-    wf_detach_mark<<<grid, 256, 0, stream>>>(B, P.sample_begin, thr, D.list, n_listed);
-    if ((e = cudaEventRecord(ready, stream)) != cudaSuccess) return e;
-    if ((e = cudaStreamWaitEvent(detach_stream, ready, 0)) != cudaSuccess) return e;
-    wf_tail<<<std::max(1, ctas), 32 * kCoopMaxWarps, 0, detach_stream>>>(S, P, B, D.list, n_listed, claim, D.queue, fb_in_rowmajor, out_tiles, 1);
+    wf_tail<<<ctas, 32 * kCoopMaxWarps, 0, stream>>>(S, P, B, B.queue, B.counters + 6, B.counters + 7, B.queue + B.n_slots, fb_in_rowmajor, out_tiles);
     return cudaGetLastError();
 }
 

@@ -15,7 +15,6 @@
 // No RNG draw depends on a trace result (SURVEY a5), which is what allows a whole surface interaction — all four side
 // rays and the continuation ray — to be generated in one shade pass and traced in one trace pass.
 #include <algorithm>
-#include <atomic>
 #include <cstdio>
 #include <cstdlib>
 #include <utility>
@@ -73,7 +72,7 @@ __global__ void __launch_bounds__(WF_SHADE_BLOCK, WF_SHADE_MIN_BLOCKS) wf_shade(
     ShadeOut R;
     R.q_path = R.q0 = R.q1 = R.q2 = R.q3 = R.pixel_done = false; R.flags = 0;
     const int flags_in = slot < n ? B.flags[slot] : WF_DONE;
-    if (!(flags_in & (WF_DONE | WF_DETACHED)))
+    if (!(flags_in & WF_DONE))
     {
         int x, y;
         wf_slot_pixel(P, slot, x, y);
@@ -299,46 +298,26 @@ cudaError_t run_wavefront(const SceneDev& S, const RenderParams& P, const WfGrou
     if ((e = cudaEventRecord(fork_event, stream)) != cudaSuccess) return e;
     cudaError_t err = cudaSuccess;
 #define WF_TRY(expr) do { if (err == cudaSuccess) { const cudaError_t e__ = (expr); if (e__ != cudaSuccess) err = e__; } } while (0)
-    struct GroupRun { RenderParams P; int parity; bool finished, forked, barrier_free, detach, detached; int slot_grid; long long it, poll_it; bool poll_pending; unsigned int tail_below; };
+    struct GroupRun { RenderParams P; int parity; bool finished, forked; int slot_grid; long long it, poll_it; bool poll_pending; unsigned int tail_below; };
     // barrier-free tail (persist.cu): when a group has at most B200RT_WF_TAIL_PCT % of its pixels (and at most B200RT_WF_TAIL_CAP) left,
     // or is smaller than B200RT_WF_TAIL_MIN pixels to begin with. 8-ary layout, default trace kernel only; not in the per-kernel timing modes.
     // Measured on C3 at 64 spp (profiles/r2_tail.jsonl): whole frame 433.3 ms without, 428.9 with a 30 k cap (445 with 100 k: the tail
     // kernel's throughput is below the pass kernels', it only pays once passes are latency-bound); one rank of 8: 108.1 -> 101.7 ms at 20 %.
-    // (the knobs are read per frame: tools/async_bench.py sweeps them inside one process)
+    // (the knobs are read per frame: tools/tail_bench.py sweeps them inside one process)
     auto env_ll = [](const char* name, long long dflt) { const char* e = getenv(name); return e ? atoll(e) : dflt; };
     const int tail_pct = (int)std::min(100ll, std::max(0ll, env_ll("B200RT_WF_TAIL_PCT", 20)));
     const long long tail_cap = env_ll("B200RT_WF_TAIL_CAP", 30000);
     const int tail_min = (int)env_ll("B200RT_WF_TAIL_MIN", 16384);
-    // Which barrier-free kernel finishes a group: wf_tail (persist.cu), or — B200RT_FLAG_WF_ASYNC / B200RT_WF_ASYNC=1 — wf_async
-    // (async.cu: shading by chunk-owning warps, tracing pooled across the whole grid through a device-wide ticket ring), which takes
-    // over below B200RT_WF_ASYNC_PCT % of the group's pixels (and B200RT_WF_ASYNC_CAP), or from the first pass on for groups of at
-    // most B200RT_WF_ASYNC_MIN pixels. Bit-identical; measured slower than passes + wf_tail everywhere (DESIGN.md 4.3): a study path.
-    const bool async_env = env_ll("B200RT_WF_ASYNC", 0) != 0 || (P.flags & B200RT_FLAG_WF_ASYNC) != 0;
-    const int async_pct = (int)std::min(100ll, std::max(0ll, env_ll("B200RT_WF_ASYNC_PCT", 20)));
-    const long long async_cap = env_ll("B200RT_WF_ASYNC_CAP", 60000);
-    const int async_min = (int)env_ll("B200RT_WF_ASYNC_MIN", 70000);
     const bool passes_only = (P.flags & B200RT_FLAG_WF_PASSES_ONLY) != 0;
     const bool tail_ok = coop && tail_pct > 0 && !timing && !passes_only;
     const int tail_ctas = tail_ok ? std::max(1, wavefront_tail_max_ctas() / n_groups) : 0;
-    const bool async_ok = coop && async_env && !timing && !passes_only;
-    // Early hand-over of the pixels that lag furthest behind (persist.cu: launch_wavefront_detach; B200RT_FLAG_WF_DETACH or
-    // B200RT_WF_DETACH=1 — a study path, off by default): after B200RT_WF_DETACH_AT passes (default 36) the B200RT_WF_DETACH_SLOTS
-    // (default 12 288 per device, shared by the groups) slowest pixels of a group go to a barrier-free kernel of
-    // B200RT_WF_DETACH_CTAS CTAs per SM (default 2, shared by the groups) on a stream of its own.
-    const long long detach_at = env_ll("B200RT_WF_DETACH_AT", 36);
-    const unsigned int detach_budget = (unsigned int)std::max(0ll, env_ll("B200RT_WF_DETACH_SLOTS", 12288) / n_groups);
-    const int detach_ctas = (int)std::max(1ll, env_ll("B200RT_WF_DETACH_CTAS", 2) * n_sm / n_groups);
-    const bool detach_ok = tail_ok && !async_ok && detach_at > 0 && detach_budget > 0u && ((P.flags & B200RT_FLAG_WF_DETACH) || env_ll("B200RT_WF_DETACH", 0) != 0);
-    const int async_ctas = async_ok ? std::max(1, wavefront_async_max_ctas() / n_groups) : 0;
-    // one of the two for group g: launches the barrier-free kernel that finishes the group behind whatever is queued on its stream
-    auto group_async = [&](int g) { return async_ok && groups[g].amem.ray_ring != nullptr && wavefront_async_fits(groups[g].buf.n_slots); };
+    // launches the tail that finishes group g behind whatever is queued on its stream
     auto finish_group = [&](int g, const RenderParams& GP) -> cudaError_t
     {
         const WfGroup& G = groups[g];
         WfTimeline::Launch tlt = { g, 0, 0, 0 };
         if (tln) { tlt.e0 = tln->used; cudaEventRecord(tln->take(), G.stream); }
-        const cudaError_t fe = group_async(g) ? launch_wavefront_async(S, GP, G.buf, G.amem, async_ctas, fb_in_rowmajor, out_tiles, G.stream)
-                                              : launch_wavefront_tail(S, GP, G.buf, tail_ctas, fb_in_rowmajor, out_tiles, G.stream);
+        const cudaError_t fe = launch_wavefront_tail(S, GP, G.buf, tail_ctas, fb_in_rowmajor, out_tiles, G.stream);
         if (tln) { tlt.e1 = tln->used; cudaEventRecord(tln->take(), G.stream); tln->tails.push_back(tlt); }
         launches += 2;
         return fe;
@@ -352,11 +331,7 @@ cudaError_t run_wavefront(const SceneDev& S, const RenderParams& P, const WfGrou
         R.P.rank = P.rank + g * P.world;
         R.P.world = P.world * n_groups;
         R.P.n_rank_tiles = G.buf.n_slots / kTilePixels;
-        // results carry the slot's shading-step count as a stamp (async.cu): every frame starts the count somewhere else, so that
-        // what an earlier frame left in the result records cannot pass for this frame's
-        static std::atomic<unsigned int> frame_nonce{0u};        // (multi-device scenes render from one host thread per device)
-        R.P.stamp0 = (int)((frame_nonce.fetch_add(1000003u, std::memory_order_relaxed) + 1000003u) & kWfSeqMask);
-        R.parity = 0; R.it = 0; R.poll_it = 0; R.poll_pending = false; R.forked = false; R.barrier_free = false; R.detach = false; R.detached = false;
+        R.parity = 0; R.it = 0; R.poll_it = 0; R.poll_pending = false; R.forked = false;
         R.slot_grid = (G.buf.n_slots + 255) / 256;
         R.finished = R.slot_grid <= 0;
         if (err != cudaSuccess) { R.finished = true; continue; }
@@ -369,14 +344,8 @@ cudaError_t run_wavefront(const SceneDev& S, const RenderParams& P, const WfGrou
         if (R.finished) continue;
         wf_init<<<R.slot_grid, 256, 0, G.stream>>>(S, R.P, G.buf, fb_in_rowmajor, out_tiles);
         launches++;
-        const bool as = group_async(g);
-        R.barrier_free = as || tail_ok;
-        // worth it when the chain is long and the group much larger than what is taken out of it
-        R.detach = detach_ok && !as && G.dmem.list != nullptr && (long long)G.buf.n_slots > 4ll * detach_budget && detach_budget <= (unsigned int)G.dmem.list_words &&
-                   (long long)(P.sample_end - P.sample_begin) * (P.max_bounces + 1) >= 4 * detach_at;
-        R.tail_below = as ? (unsigned int)std::min<long long>(async_cap, (long long)G.buf.n_slots * async_pct / 100)
-                          : (unsigned int)std::min<long long>(tail_cap, (long long)G.buf.n_slots * tail_pct / 100);
-        if (R.barrier_free && G.buf.n_slots <= (as ? async_min : tail_min))
+        R.tail_below = (unsigned int)std::min<long long>(tail_cap, (long long)G.buf.n_slots * tail_pct / 100);
+        if (tail_ok && G.buf.n_slots <= tail_min)
         {
             // a group this small is latency-bound from its first pass on: barrier-free from the start
             WF_TRY(finish_group(g, R.P));
@@ -402,7 +371,7 @@ cudaError_t run_wavefront(const SceneDev& S, const RenderParams& P, const WfGrou
             {
                 R.poll_pending = false;
                 if (*G.host_active == 0) { R.finished = true; remaining--; continue; }
-                if (R.barrier_free && *G.host_active <= R.tail_below)
+                if (tail_ok && *G.host_active <= R.tail_below)
                 {
                     // few pixels left: no more passes; one barrier-free launch finishes them, behind the passes already queued
                     WF_TRY(finish_group(g, R.P));
@@ -431,17 +400,6 @@ cudaError_t run_wavefront(const SceneDev& S, const RenderParams& P, const WfGrou
             if (timing) cudaEventRecord(tev[1], G.stream);
             if (tln) { tll.e1 = tln->used; cudaEventRecord(tln->take(), G.stream); }
             R.parity ^= 1;
-            if (R.detach && !R.detached && R.it + 1 == detach_at)
-            {
-                // between this trace pass and its shade pass: the lagging pixels' results wait for the barrier-free kernel
-                WfTimeline::Launch tlt = { g, 0, 0, 0 };
-                if (tln) { tlt.e0 = tln->used; cudaEventRecord(tln->take(), G.stream); }
-                WF_TRY(launch_wavefront_detach(S, R.P, G.buf, G.dmem, detach_budget, std::min(detach_ctas, G.dmem.ctas), fb_in_rowmajor, out_tiles, G.stream,
-                                               G.detach_stream, G.detach_ready));
-                if (tln) { tlt.e1 = tln->used; cudaEventRecord(tln->take(), G.detach_stream); tln->tails.push_back(tlt); }
-                R.detached = true;
-                launches += 4;
-            }
             wf_shade<<<(G.buf.n_slots + WF_SHADE_BLOCK - 1) / WF_SHADE_BLOCK, WF_SHADE_BLOCK, 0, G.stream>>>(S, R.P, G.buf, fb_in_rowmajor, out_tiles, R.parity);
             if (tln) { tll.e2 = tln->used; cudaEventRecord(tln->take(), G.stream); tln->launches.push_back(tll); }
             launches += 2;
@@ -474,12 +432,6 @@ cudaError_t run_wavefront(const SceneDev& S, const RenderParams& P, const WfGrou
         const cudaError_t e1 = cudaEventRecord(G.join_event, G.stream);
         const cudaError_t e2 = e1 == cudaSuccess ? cudaStreamWaitEvent(stream, G.join_event, 0) : e1;
         if (err == cudaSuccess && e2 != cudaSuccess) err = e2;
-        if (run[g].detached)
-        {
-            const cudaError_t e3 = cudaEventRecord(G.detach_join, G.detach_stream);
-            const cudaError_t e4 = e3 == cudaSuccess ? cudaStreamWaitEvent(stream, G.detach_join, 0) : e3;
-            if (err == cudaSuccess && e4 != cudaSuccess) err = e4;
-        }
     }
 #undef WF_TRY
     if (timing)

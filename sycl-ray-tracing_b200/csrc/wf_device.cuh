@@ -7,14 +7,10 @@
 
 namespace b200rt {
 
-enum { WF_ALIVE = 1, WF_PENDING = 2, WF_TERMINATED = 4, WF_DONE = 8,
-       WF_DETACHED = 16 };        // the slot left the passes: a barrier-free kernel runs it to the end (wavefront.cu, persist.cu)
-constexpr int kWfSeqShift = 8;    // bits 8..31 of a slot's flag word: its shading-step count (the stamp of its rays' results)
-constexpr unsigned int kWfSeqMask = 0xffffffu;
+enum { WF_ALIVE = 1, WF_PENDING = 2, WF_TERMINATED = 4, WF_DONE = 8 };
 
-// Loads of per-slot integrator state (WfBuffers) go to L2 (ld.global.cg), never through L1: in the barrier-free kernels
-// (async.cu) a slot is shaded and its rays are traced by whichever warps of the machine take them, and L1 is not coherent
-// between SMs. The pass-synchronous kernels read every word of the state once per launch, so they lose nothing by it.
+// Loads of per-slot integrator state (WfBuffers) go to L2 (ld.global.cg), not through L1: a kernel reads each state word of a
+// slot once per launch (DESIGN.md §2), so caching it in L1 would buy no reuse.
 template <typename T>
 __device__ __forceinline__ T wf_ld(const T* p) { return __ldcg(p); }
 
@@ -78,10 +74,6 @@ __device__ __forceinline__ size_t wf_out_index(const WfBuffers& B, int slot)
 // pixel index of this rank's tile-major buffer (8x4 patches inside 16x16 tiles) -> pixel; false outside the frame
 __device__ __forceinline__ bool wf_slot_pixel(const RenderParams& P, int slot, int& x, int& y)
 {
-#ifdef B200RT_EXPERIMENT_SCRAMBLE
-    // timing experiment only (the image is wrong): neighbouring slots hold unrelated pixels — what a wavefront without any ray coherence costs
-    slot = (int)(((unsigned long long)(unsigned int)slot * 2654435761ull) % (unsigned long long)(P.n_rank_tiles * kTilePixels));
-#endif
     const int unit = slot >> 5, lane = slot & 31;
     const int k = unit >> 3, sub = unit & 7;
     int tx, ty;
@@ -116,7 +108,7 @@ __device__ __forceinline__ void wf_begin_pixel(const RenderParams& P, const WfBu
     B.final_c[slot] = resume ? P.acc_sum[out_index] : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
     B.sample_c[slot] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
     B.thr[slot] = make_float4(1.0f, 1.0f, 1.0f, 0.0f);
-    B.flags[slot] = WF_ALIVE | (int)(((unsigned int)P.stamp0 & kWfSeqMask) << kWfSeqShift);
+    B.flags[slot] = WF_ALIVE;
 }
 
 // what one shading step of a slot produced: which of its ray slots (0..3 side rays, 4 path ray) hold a ray to trace now
@@ -140,9 +132,7 @@ __device__ __forceinline__ ShadeOut wf_shade_slot(const SceneDev& S, const Rende
     int sample = wf_ld(B.sample + slot), bounce = wf_ld(B.bounce + slot);
     float4 t4 = wf_ld(B.thr + slot), s4 = wf_ld(B.sample_c + slot);
     col throughput = CO(t4.x, t4.y, t4.z), sample_color = CO(s4.x, s4.y, s4.z);
-    // the upper bits of the slot's flag word count its shading steps: the stamp its rays' results must carry (async.cu)
-    const unsigned int seq = (unsigned int)flags_in >> kWfSeqShift;
-    int flags = flags_in & 15;
+    int flags = flags_in;
     bool finish = false;
     const bool trace_light_brdf = S.any_emissive_material || !(P.flags & B200RT_FLAG_SKIP_DEAD_RAYS);
 
@@ -159,7 +149,7 @@ __device__ __forceinline__ ShadeOut wf_shade_slot(const SceneDev& S, const Rende
             const int kind = __float_as_int(rd4.w);
             if (kind == SIDE_NONE) continue;
             const float4 w4 = wf_ld(B.side_w + i);
-            const float4 res = wf_ld(B.res + i);      // {t, primitive | occlusion flag, triangle slot, stamp}
+            const float4 res = wf_ld(B.res + i);      // {t, primitive | occlusion flag, triangle slot, -}
             if (kind == SIDE_CLOSEST_LIGHT)
             {
                 const float t = res.x;
@@ -282,20 +272,18 @@ __device__ __forceinline__ ShadeOut wf_shade_slot(const SceneDev& S, const Rende
     B.bounce[slot] = bounce;
     B.thr[slot] = make_float4(throughput.r, throughput.g, throughput.b, 0.0f);
     B.sample_c[slot] = make_float4(sample_color.r, sample_color.g, sample_color.b, 0.0f);
-    flags |= (flags_in & WF_DETACHED) | (int)(((seq + 1u) & kWfSeqMask) << kWfSeqShift);
     B.flags[slot] = flags;
     R.flags = flags;
     return R;
 }
 
 // result of one queue entry: one 16-byte record {t or -1, primitive (closest hit) | occlusion flag (any-hit / shadow rays),
-// triangle slot, stamp}. A single 16-byte store is single-copy atomic, so a reader that finds the stamp it expects has the whole
-// result — what lets the barrier-free kernel (async.cu) hand results over without a fence; the other kernels leave the stamp 0.
-__device__ __forceinline__ void wf_store_result(const WfBuffers& B, size_t r, int mode, bool found, const Hit& h, unsigned int stamp = 0u)
+// triangle slot, 0}, written with a single 16-byte store.
+__device__ __forceinline__ void wf_store_result(const WfBuffers& B, size_t r, int mode, bool found, const Hit& h)
 {
     float4 v;
-    if (mode == TRACE_CLOSEST) v = make_float4(found ? h.t : -1.0f, __int_as_float(h.prim), __int_as_float(h.slot), __uint_as_float(stamp));
-    else v = make_float4(0.0f, __int_as_float(found ? 1 : 0), 0.0f, __uint_as_float(stamp));
+    if (mode == TRACE_CLOSEST) v = make_float4(found ? h.t : -1.0f, __int_as_float(h.prim), __int_as_float(h.slot), 0.0f);
+    else v = make_float4(0.0f, __int_as_float(found ? 1 : 0), 0.0f, 0.0f);
     B.res[r] = v;
 }
 
@@ -418,114 +406,10 @@ __device__ __forceinline__ void coop_drain(const SceneDev& S, CoopWarp& W, const
     qtris -= lim;
 }
 
-// ---- device-wide ticket ring (async.cu) ----------------------------------------------------------------------------------------------
-// A multi-producer / multi-consumer ring in global memory. Producers reserve indices with one atomicAdd per warp on ctrl[1]
-// and store (lap tag << 25) | payload; consumers draw TICKETS — indices, possibly of entries that do not exist yet — with one
-// atomicAdd per warp on ctrl[0] and poll their own word until the entry with their ticket's lap tag shows up, then put
-// kRingEmpty back. Nobody waits on anybody in particular: a producer only waits for the consumer of the same word one lap
-// (>= 2^20 entries) earlier, a consumer only polls (once per iteration of its own work loop), so the rings cannot deadlock a
-// persistent grid whatever part of it is resident. An entry is handed to the oldest waiting ticket: FIFO, no claim races.
-constexpr unsigned int kRingEmpty = 0xffffffffu;
-constexpr int kRingPayloadBits = 25;                      // (slot << 3) | ray index k: slots < 2^22 per tile group
-struct WfRing
-{
-    unsigned int* buf;
-    unsigned int* ctrl;        // [0] tickets drawn, [1] entries reserved (one 128-byte line per ring)
-    unsigned int log2cap;
-    __device__ __forceinline__ unsigned int pos(unsigned int i) const { return i & ((1u << log2cap) - 1u); }
-    __device__ __forceinline__ unsigned int tag(unsigned int i) const { return (i >> log2cap) & 127u; }
-};
-
-// Memory ordering of the rings. Everything a ring entry (or the per-slot ray count) publishes is written with plain stores and
-// made visible by a RELEASE operation (MEMBAR.ALL.GPU + the store / atomic); it is read with loads that bypass L1 (wf_ld,
-// ld.relaxed.gpu), issued after the entry was seen. No acquire fences: on this machine fence.acq_rel / __threadfence() also
-// invalidate the SM's whole L1 (CCTL.IVALL) — the top of the BVH the tracers live on.
-__device__ __forceinline__ unsigned int ld_relaxed(const unsigned int* p)
-{
-    unsigned int v;
-    asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void st_relaxed(unsigned int* p, unsigned int v) { asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
-__device__ __forceinline__ void st_release(unsigned int* p, unsigned int v) { asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
-__device__ __forceinline__ void red_add_relaxed(unsigned int* p, unsigned int v) { asm volatile("red.relaxed.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
-
-// Every lane of the warp calls this; lane appends payload[k] for every k with q[k] — ONE reservation for the whole warp. The
-// entries are laid out kind-major (all lanes' entry 0, then all lanes' entry 1, ...), the sentinel checks of a lane's entries
-// are in flight together. release: the lane's earlier stores become visible before its first entry (its later entries follow
-// the same MEMBAR in program order).
-__device__ __forceinline__ unsigned int ring_push5(const WfRing& R, const bool q[5], const unsigned int payload[5], bool release)
-{
-    const int lane = threadIdx.x & 31;
-    const unsigned int below = (1u << lane) - 1u;
-    unsigned int m[5], total = 0u;
-#pragma unroll
-    for (int k = 0; k < 5; k++) { m[k] = __ballot_sync(0xffffffffu, q[k]); total += __popc(m[k]); }
-    if (!total) return 0u;
-    unsigned int base = 0;
-    if (lane == 0) base = atomicAdd(R.ctrl + 1, total);
-    base = __shfl_sync(0xffffffffu, base, 0);
-    unsigned int idx[5], off = base;
-#pragma unroll
-    for (int k = 0; k < 5; k++) { idx[k] = off + __popc(m[k] & below); off += __popc(m[k]); }
-    unsigned int seen[5];
-#pragma unroll
-    for (int k = 0; k < 5; k++) seen[k] = q[k] ? ld_relaxed(R.buf + R.pos(idx[k])) : kRingEmpty;
-#pragma unroll
-    for (int k = 0; k < 5; k++)
-        if (q[k])
-        {
-            unsigned int* p = R.buf + R.pos(idx[k]);
-            while (seen[k] != kRingEmpty) seen[k] = ld_relaxed(p);      // the consumer of this word one lap ago has long put the sentinel back
-            const unsigned int e = (R.tag(idx[k]) << kRingPayloadBits) | payload[k];
-            if (release) { st_release(p, e); release = false; }
-            else st_relaxed(p, e);
-        }
-    return total;
-}
-
-// every lane of the warp calls this; lanes with `want` receive a ticket
-__device__ __forceinline__ unsigned int ring_tickets(const WfRing& R, bool want)
-{
-    const unsigned int m = __ballot_sync(0xffffffffu, want);
-    if (!m) return 0u;
-    const int lane = threadIdx.x & 31;
-    const int leader = __ffs(m) - 1;
-    unsigned int base = 0;
-    if (lane == leader) base = atomicAdd(R.ctrl, (unsigned int)__popc(m));
-    base = __shfl_sync(0xffffffffu, base, leader);
-    return base + __popc(m & ((1u << lane) - 1u));
-}
-
-// has the entry of `ticket` arrived? takes it if so
-__device__ __forceinline__ bool ring_poll(const WfRing& R, unsigned int ticket, unsigned int& payload)
-{
-    unsigned int* p = R.buf + R.pos(ticket);
-    const unsigned int e = ld_relaxed(p);
-    if (e == kRingEmpty || (e >> kRingPayloadBits) != R.tag(ticket)) return false;
-    st_relaxed(p, kRingEmpty);
-    payload = e & ((1u << kRingPayloadBits) - 1u);
-    return true;
-}
-
 // Where a warp gets its rays from: blocks of a queue claimed with one atomic (the pass-synchronous kernels: every warp of
-// the grid shares one queue), a private range (the persistent integrator: a warp traces the rays its own slots produced),
-// or the device-wide ray ring of the barrier-free kernel (async.cu).
-struct CoopQueueRing
-{
-    static constexpr bool kRing = true;
-    static constexpr bool kCacheEntries = false;
-    WfRing rays;                      // rays to trace
-    unsigned int* cnt;                // per chunk of 32 slots: rays pushed and not traced yet (owner-major, see chunk_index)
-    unsigned int* chunk_live;         // per chunk: slots not finished yet (written by the chunk's shader warp only)
-    const unsigned int* live;         // pixels not finished yet (counters[2]); 0 = the frame is over
-    int n_chunks, W, K;               // W shader warps own K chunks each: chunk c belongs to warp c % W
-    __device__ __forceinline__ unsigned int chunk_index(unsigned int c) const { return (c % (unsigned int)W) * (unsigned int)K + c / (unsigned int)W; }
-    __device__ __forceinline__ bool claim(int, unsigned int&, unsigned int&) { return false; }
-};
+// the grid shares one queue) or a private range (the persistent integrator: a warp traces the rays its own slots produced).
 struct CoopQueueShared
 {
-    static constexpr bool kRing = false;
     static constexpr bool kCacheEntries = true;       // blocks of at most kWarpBlock entries: a claimed block's entries live in registers
     unsigned int* head; unsigned int n_rays, warp_block;
     __device__ __forceinline__ bool claim(int lane, unsigned int& blk_next, unsigned int& blk_end)
@@ -540,7 +424,6 @@ struct CoopQueueShared
 };
 struct CoopQueuePrivate
 {
-    static constexpr bool kRing = false;
     static constexpr bool kCacheEntries = false;
     unsigned int next, end;
     __device__ __forceinline__ bool claim(int, unsigned int& blk_next, unsigned int& blk_end)
@@ -572,68 +455,12 @@ __device__ __forceinline__ void coop_trace_queue(const SceneDev& S, const WfBuff
     unsigned int qe[kWarpBlock / 32 > 0 ? kWarpBlock / 32 : 1] = {};   // kCacheEntries: this lane's share of the block's entries
     unsigned int head = 0, dcount = 0, qtris = 0;              // warp-uniform: descriptor ring
     bool exhausted = false;                                    // warp-uniform
-    unsigned int ent = 0u, ticket = 0u;                        // ring source: the lane's queue entry; its ticket while it waits for one
-    bool has_ticket = false, starved = false;                  // starved (warp-uniform): the last poll left a lane waiting
-    unsigned int iter = 0u, idle_it = 0u, stamp = 0u;          // stamp: the shading-step count of the ray's slot, returned with the result
     W.pend[lane] = 0u;
     __syncwarp();
 
     for (;;)
     {
-        // (1) refill idle lanes: from the warp's block of the ray queue, or — ring source — every idle lane draws a ticket of the
-        //     device-wide ray ring and looks once per iteration whether its ray has arrived
-        if constexpr (Source::kRing)
-        {
-            const bool want = !active && !has_ticket;
-            const unsigned int need = __ballot_sync(FULL, want);
-            if (need && (need == FULL || __popc(need) >= kRefillThreshold || !__any_sync(FULL, has_ticket)))
-            {
-                const unsigned int tk = ring_tickets(src.rays, want);
-                if (want) { ticket = tk; has_ticket = true; }
-            }
-            // a poll is one L2 round trip the whole warp waits for: every iteration while rays arrive at once (or nothing is in
-            // flight here), every fourth while the ring is starved and other lanes of this warp are busy tracing
-            const bool waiting = !active && has_ticket;
-            const bool poll_now = !starved || (iter++ & 3u) == 0u || !__any_sync(FULL, active);
-            bool got = false;
-            if (poll_now)
-            {
-                if (waiting) got = ring_poll(src.rays, ticket, ent);
-                starved = __any_sync(FULL, waiting && !got);
-            }
-            if (got)
-            {
-                has_ticket = false;
-                const int slot = (int)(ent >> 3), k = (int)(ent & 7u);
-                r = (size_t)k * n + slot;
-                const float4 ro4 = wf_ld(B.ray_o + r), rd4 = wf_ld(B.ray_d + r);
-                stamp = (unsigned int)wf_ld(B.flags + slot) >> kWfSeqShift;
-                const int kind = __float_as_int(rd4.w);
-                mode = kind == SIDE_SHADOW ? TRACE_SHADOW : (kind == SIDE_CLOSEST_LIGHT ? TRACE_CLOSEST : TRACE_ANY);
-                const int tmode = spheres ? TRACE_CLOSEST : mode;
-                trav8_init(T, V(ro4.x, ro4.y, ro4.z), V(rd4.x, rd4.y, rd4.z), ro4.w, tmode);
-                W.ro[lane] = ro4;
-                W.rd[lane] = make_float4(rd4.x, rd4.y, rd4.z, __int_as_float(tmode));
-                W.best[lane] = kNoHit;
-                active = true;
-            }
-            __syncwarp();
-            if (!__any_sync(FULL, active))
-            {
-                // nothing in flight in this warp: over when no pixel is left, else wait for rays without hammering L2
-                // (the live-pixel counter is one word for the whole grid: looked at every 16th time)
-                if ((idle_it++ & 15u) == 0u)
-                {
-                    unsigned int left = 0;
-                    if (lane == 0) left = ld_relaxed(src.live);
-                    if (__shfl_sync(FULL, left, 0) == 0u) break;
-                }
-                __nanosleep(400);
-                continue;
-            }
-        }
-        else
-        {
+        // (1) refill idle lanes from the warp's block of the ray queue
         unsigned int idle = __ballot_sync(FULL, !active);
         if (idle && !exhausted && (idle == FULL || __popc(idle) >= kRefillThreshold))
         {
@@ -704,7 +531,6 @@ __device__ __forceinline__ void coop_trace_queue(const SceneDev& S, const WfBuff
             if (exhausted) break;
             continue;
         }
-        }
         // (2) one node step for every lane that has one
         if (active && !T.done)
         {
@@ -772,14 +598,7 @@ __device__ __forceinline__ void coop_trace_queue(const SceneDev& S, const WfBuff
                 found = finish_with_spheres(S, V(ro4.x, ro4.y, ro4.z), V(rd4.x, rd4.y, rd4.z), ro4.w, mode, h);
             }
             active = false;
-            if constexpr (Source::kRing)
-            {
-                // hand-over without a fence and without waiting for anything: the stamped 16-byte result, then one fire-and-forget
-                // decrement of the chunk's count of outstanding rays (the shader that finds the count at zero checks the stamps)
-                wf_store_result(B, r, mode, found, h, stamp);
-                red_add_relaxed(src.cnt + src.chunk_index(ent >> 8), 0xffffffffu);
-            }
-            else wf_store_result(B, r, mode, found, h);
+            wf_store_result(B, r, mode, found, h);
         }
     }
 }

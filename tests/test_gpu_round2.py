@@ -539,12 +539,12 @@ def test_denoise_stage(rt, golden_cameras):
     assert np.allclose(half[..., :3], 0.5 * den4[..., :3] + 0.5 * noisy[..., :3], atol=1e-6)
 
 
-# ---- barrier-free continuation that pools work across warps (csrc/async.cu) -----------------------------------------------------------
-def test_async_continuation_equals_passes_bit_for_bit(rt, golden_scenes, golden_cameras):
-    """wf_async (B200RT_FLAG_WF_ASYNC) finishes a tile group with chunk-owning shader warps and tracer warps fed by a device-wide ticket
-    ring: same device functions, same per-pixel RNG streams -> the frame and the ray count equal the pure pass-synchronous frame's
-    (B200RT_FLAG_WF_PASSES_ONLY), the default frame's (passes + per-warp tail) and the megakernel's, bit for bit: groups that are barrier-free from the first pass
-    (small frames), groups that switch once few pixels are left (a 1280x720 frame), interleaved ranks with a non-black incoming
+# ---- barrier-free tail of a pass-synchronous frame (csrc/persist.cu) ----------------------------------------------------------------------
+def test_tail_continuation_equals_passes_bit_for_bit(rt, golden_scenes, golden_cameras):
+    """The default wavefront frame finishes each tile group's last few pixels with one barrier-free wf_tail launch (every warp runs a
+    few slots to the end on its own): same device functions, same per-pixel RNG streams -> the frame and the ray count equal the pure
+    pass-synchronous frame's (B200RT_FLAG_WF_PASSES_ONLY) and the megakernel's, bit for bit: groups that are barrier-free from the first
+    pass (small frames), groups that switch once few pixels are left (a 1280x720 frame), interleaved ranks with a non-black incoming
     framebuffer, spheres, emissive triangles (MIS.obj), and the dead-ray elimination (slots that are alive without a ray)."""
     from sycl_ray_tracing_b200 import scenes
     for key, fixture in [("cornell", "render_cornell_env.npz"), ("mis", "render_mis_env.npz")]:
@@ -554,49 +554,46 @@ def test_async_continuation_equals_passes_bit_for_bit(rt, golden_scenes, golden_
         sc = rt.Scene(a["tri9"], a["mat_idx"], a["mats10"], a["emissive"], skysphere=g["env"])
         c = rt.Camera.from_array17(golden_cameras[key])
         mega, st_m = sc.render(c, w, h, spp, b, integrator=rt.INTEGRATOR_MEGAKERNEL)
-        asy, st_a = sc.render(c, w, h, spp, b, flags=rt.FLAG_WF_ASYNC)
         pas, st_p = sc.render(c, w, h, spp, b, flags=rt.FLAG_WF_PASSES_ONLY)
         tail, st_t = sc.render(c, w, h, spp, b)
-        for name, img, st in (("async", asy, st_a), ("passes", pas, st_p), ("warp tail", tail, st_t)):
+        for name, img, st in (("passes", pas, st_p), ("default", tail, st_t)):
             assert np.array_equal(bits(mega), bits(img)), f"{fixture} {name}: {(bits(mega) != bits(img)).any(axis=-1).sum()} pixels differ"
             assert st["rays"] == st_m["rays"], (fixture, name, st["rays"], st_m["rays"])
-        assert st_a["gpu_launches"] < st_p["gpu_launches"], "the small frame is barrier-free from its first pass"
-        assert_radiance_parity(asy, g["image"], f"async {fixture}")
+        assert st_t["gpu_launches"] < st_p["gpu_launches"], "the small frame is barrier-free from its first pass"
+        assert_radiance_parity(tail, g["image"], f"default {fixture}")
         rng = np.random.default_rng(11)
         w2, h2 = 100, 70
         fb0 = (rng.random((h2, w2, 4)) * 0.2).astype(np.float32)
         want = fb0.copy(); sc.render(c, w2, h2, 3, 4, framebuffer=want, flags=rt.FLAG_WF_PASSES_ONLY)
         got = fb0.copy()
         for rank in range(3):
-            sc.render(c, w2, h2, 3, 4, framebuffer=got, rank=rank, world=3, flags=rt.FLAG_WF_ASYNC)
+            sc.render(c, w2, h2, 3, 4, framebuffer=got, rank=rank, world=3)
         assert np.array_equal(bits(want), bits(got)), "ranks + non-black framebuffer"
     g = load_golden("render_c3small.npz")
     c3 = scenes.c3_scene(roughness=float(g["roughness"]), nu=int(g["nu"]), nv=int(g["nv"]), sky_w=int(g["sky_w"]), sky_h=int(g["sky_h"]))
     sc = scene_of(rt, c3)
     for (w, h, spp) in ((640, 360, 6), (1280, 720, 4), (1920, 1080, 2)):
         pas, st_p = sc.render(c3["camera"], w, h, spp, 8, flags=rt.FLAG_WF_PASSES_ONLY)
-        asy, st_a = sc.render(c3["camera"], w, h, spp, 8, flags=rt.FLAG_WF_ASYNC)
-        assert np.array_equal(bits(pas), bits(asy)), f"c3 {w}x{h}: {(bits(pas) != bits(asy)).any(axis=-1).sum()} pixels differ"
-        assert st_p["rays"] == st_a["rays"]
+        tail, st_t = sc.render(c3["camera"], w, h, spp, 8)
+        assert np.array_equal(bits(pas), bits(tail)), f"c3 {w}x{h}: {(bits(pas) != bits(tail)).any(axis=-1).sum()} pixels differ"
+        assert st_p["rays"] == st_t["rays"]
         skip_p, st_sp = sc.render(c3["camera"], w, h, spp, 8, flags=rt.FLAG_WF_PASSES_ONLY | rt.FLAG_SKIP_DEAD_RAYS)
-        skip_a, st_sa = sc.render(c3["camera"], w, h, spp, 8, flags=rt.FLAG_WF_ASYNC | rt.FLAG_SKIP_DEAD_RAYS)
-        assert np.array_equal(bits(pas), bits(skip_a)) and st_sp["rays"] == st_sa["rays"] < st_p["rays"]
-    # study path B200RT_FLAG_WF_DETACH: the pixels that lag furthest behind leave the passes after 36 of them for a barrier-free kernel on
-    # a stream of its own: same frame and ray count as the default, as passes only, as the megakernel; also as one rank of 2
+        skip_t, st_st = sc.render(c3["camera"], w, h, spp, 8, flags=rt.FLAG_SKIP_DEAD_RAYS)
+        assert np.array_equal(bits(pas), bits(skip_t)) and st_sp["rays"] == st_st["rays"] < st_p["rays"]
+    # a longer chain (24 spp): same frame and ray count as passes only and as the megakernel; also as one rank of 2
     for kw in (dict(), dict(rank=1, world=2)):
-        det, st_d = sc.render(c3["camera"], 960, 540, 24, 8, flags=rt.FLAG_WF_DETACH, **kw)
-        nod, st_n = sc.render(c3["camera"], 960, 540, 24, 8, **kw)
+        tail, st_t = sc.render(c3["camera"], 960, 540, 24, 8, **kw)
         pas, st_p = sc.render(c3["camera"], 960, 540, 24, 8, flags=rt.FLAG_WF_PASSES_ONLY, **kw)
-        assert np.array_equal(bits(det), bits(nod)) and np.array_equal(bits(det), bits(pas)), kw
-        assert st_d["rays"] == st_n["rays"] == st_p["rays"], (kw, st_d["rays"], st_n["rays"], st_p["rays"])
-        assert st_d["gpu_launches"] != st_n["gpu_launches"], "the detach path ran"
+        assert np.array_equal(bits(tail), bits(pas)), kw
+        assert st_t["rays"] == st_p["rays"], (kw, st_t["rays"], st_p["rays"])
     mega, st_m = sc.render(c3["camera"], 960, 540, 24, 8, integrator=rt.INTEGRATOR_MEGAKERNEL)
-    det, st_d = sc.render(c3["camera"], 960, 540, 24, 8, flags=rt.FLAG_WF_DETACH)
-    assert np.array_equal(bits(det), bits(mega)) and st_d["rays"] == st_m["rays"]
-    # one rank of 8 of the 1080p frame (the shape the continuation exists for), twice: the rings are re-armed per launch
+    tail, st_t = sc.render(c3["camera"], 960, 540, 24, 8)
+    assert np.array_equal(bits(tail), bits(mega)) and st_t["rays"] == st_m["rays"]
+    # one rank of 8 of the 1080p frame (latency-bound passes: the shape the tail exists for), twice: the second frame starts from
+    # whatever the first left in the group buffers
     want, st_w = sc.render(c3["camera"], 1920, 1080, 3, 8, rank=5, world=8, flags=rt.FLAG_WF_PASSES_ONLY)
     for _ in range(2):
-        got, st_g = sc.render(c3["camera"], 1920, 1080, 3, 8, rank=5, world=8, flags=rt.FLAG_WF_ASYNC)
+        got, st_g = sc.render(c3["camera"], 1920, 1080, 3, 8, rank=5, world=8)
         assert np.array_equal(bits(want), bits(got)) and st_w["rays"] == st_g["rays"]
     # analytic spheres finish inside the tracer lanes
     gs = load_golden("sphere_cornell.npz")
@@ -608,5 +605,5 @@ def test_async_continuation_equals_passes_bit_for_bit(rt, golden_scenes, golden_
     cs = rt.Camera.from_array17(golden_cameras["cornell"])
     ws, hs, spps, bs = int(gs["w"]), int(gs["h"]), int(gs["spp"]), int(gs["bounces"])
     m, st_m = scs.render(cs, ws, hs, spps, bs, integrator=rt.INTEGRATOR_MEGAKERNEL)
-    s_a, st_a = scs.render(cs, ws, hs, spps, bs, flags=rt.FLAG_WF_ASYNC)
-    assert np.array_equal(bits(m), bits(s_a)) and st_m["rays"] == st_a["rays"]
+    s_t, st_t = scs.render(cs, ws, hs, spps, bs)
+    assert np.array_equal(bits(m), bits(s_t)) and st_m["rays"] == st_t["rays"]
