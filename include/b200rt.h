@@ -332,7 +332,12 @@ int b200rt_quantise_rgba8_device(const void* dev_image_rgba, int width, int heig
  * image alone, then out = blend * denoised + (1 - blend) * noisy, alpha 1). The reference does not ship OIDN's binaries or weights,
  * so there is nothing to be bit-compatible with: this is an edge-avoiding a-trous wavelet filter (5 passes, colour-guided) in the same
  * place — a functional stand-in, not a parity claim (DESIGN.md). channels: 3 (OIDN's float3 buffers) or 4 (Image). iterations <= 0
- * and sigma <= 0 select the defaults (5, 0.45). in == out is allowed. Host pointers; runs on the current device. */
+ * and sigma <= 0 or NaN select the defaults (5, 0.45); iterations above 8 are clamped to 8. in == out is allowed. Host pointers;
+ * runs on the current device.
+ * Non-finite pixels: a pixel with a NaN or +-Inf in R, G or B is missing data. It contributes to no neighbour, is left out of the
+ * first pass's local-variance estimate, and is itself filtered from its finite neighbours without the colour term; its output is
+ * the denoised value alone, whatever blend_factor. A pixel with no finite pixel within reach of any pass stays non-finite (an all-NaN
+ * image stays NaN). The alpha channel is never inspected. Finite images are filtered exactly as if this rule did not exist. */
 int b200rt_denoise(const float* image, int channels, int width, int height, float blend_factor, int iterations, float sigma, float* out);
 /* b200rt_denoise with OIDN's auxiliary images as edge-stopping guides (w*h*3 floats each, either may be NULL; b200rt_render_aovs
  * computes them): a tap must also agree in normal direction and albedo to contribute. Both NULL: identical to b200rt_denoise, bit for bit. */
