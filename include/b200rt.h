@@ -246,13 +246,25 @@ int b200rt_render_region(b200rt_scene* scene, const float* camera17, int width, 
  *   b200rt_accum_create   fixes scene, camera, frame size, the TOTAL spp (it seeds the per-pixel RNG: 31 + x*y*spp, :77) and max_bounces
  *   b200rt_accum_add      renders the next n_samples samples of every pixel, continuing each pixel's RNG stream where it stopped
  *   b200rt_accum_resolve  framebuffer_out = tone_map(framebuffer_in (NULL = Color::Black()) + sum / samples so far); any time, any number of times
- * After spp_total samples — in any chunking — the resolved frame equals b200rt_render(spp_total) bit for bit.
- * opts: integrator WAVEFRONT or PERSISTENT, flags as b200rt_render; rank/world must stay 0/1. Host pointers; blocking. */
+ *   b200rt_accum_resolve_rgba8  the same frame as b200rt_accum_resolve, quantised on the device to the bytes write_image_png would write
+ *                         (as b200rt_render_rgba8: image_io.cpp:165-182, flip_y != 0 writes the bottom row last): 4 B/pixel over PCIe
+ *                         instead of 16, which is what a preview wants (33 MB instead of 133 MB per 4K resolve)
+ * After spp_total samples — in any chunking — the resolved frame equals b200rt_render(spp_total) bit for bit, and the RGBA8 resolve
+ * equals b200rt_render_rgba8(spp_total) byte for byte.
+ * On a multi-device scene (b200rt_scene_create_multi) the state is split like a frame: rank d keeps the pixels of the interleaved 16x16
+ * tiles it owns (tile_id % n_devices == d) on its own device, and a rank owns none when the frame has fewer tiles than there are
+ * devices. An add runs every rank's share of the chunk at once, one host thread per device, with no traffic between devices; a
+ * resolve gathers the ranks' tiles on the scene's first device (one peer copy per rank) and tone-maps there. Either way the
+ * results are the single-device accumulator's, bit for bit. The state is the accumulator's own: b200rt_render on the same scene
+ * between two adds does not disturb it.
+ * opts: integrator WAVEFRONT or PERSISTENT, flags as b200rt_render; rank/world must stay 0/1. A refused add changes nothing. Host
+ * pointers; blocking. Destroy an accumulator before its scene. */
 typedef struct b200rt_accum b200rt_accum;
 int b200rt_accum_create(b200rt_scene* scene, const float* camera17, int width, int height, int spp_total, int max_bounces, b200rt_accum** out);
 int b200rt_accum_add(b200rt_accum* acc, int n_samples, const b200rt_render_options* opts_or_null, b200rt_stats* stats_or_null);
 int b200rt_accum_samples(const b200rt_accum* acc);
 int b200rt_accum_resolve(b200rt_accum* acc, const float* framebuffer_rgba_in_or_null, float* framebuffer_rgba_out);
+int b200rt_accum_resolve_rgba8(b200rt_accum* acc, const float* framebuffer_rgba_in_or_null, int flip_y, unsigned char* out_rgba8);
 void b200rt_accum_destroy(b200rt_accum* acc);
 
 /* Parity hook for xorshift32_generator (include/xorshift.h:10-31) as ray_trace_pixel seeds it (render_kernel.cpp:77-82):

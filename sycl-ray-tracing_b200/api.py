@@ -600,7 +600,8 @@ class Scene:
 
 class Accumulator:
     """Progressive rendering (b200rt_accum_*): the samples of a frame streamed in chunks, each pixel's RNG stream continued across
-    chunks; after spp_total samples resolve() equals Scene.render(spp_total) bit for bit."""
+    chunks; after spp_total samples resolve() equals Scene.render(spp_total) bit for bit. On a Scene(devices=...) every device keeps
+    and renders the pixels of its own tiles, and a resolve gathers them on the first device."""
 
     def __init__(self, scene: Scene, camera: Camera, w: int, h: int, spp_total: int, max_bounces: int):
         self.scene, self.w, self.h = scene, w, h
@@ -628,6 +629,16 @@ class Accumulator:
     def resolve(self, framebuffer_in: np.ndarray | None = None) -> np.ndarray:
         out = np.empty((self.h, self.w, 4), np.float32)
         B.check(B.load_library().b200rt_accum_resolve(self._h, B.fptr(framebuffer_in), B.fptr(out)))
+        return out
+
+    def resolve_rgba8(self, framebuffer_in: np.ndarray | None = None, flip_y: bool = True) -> np.ndarray:
+        """resolve() quantised on the device as write_image_png would (b200rt_accum_resolve_rgba8): (h, w, 4) uint8, 4 B/pixel over
+        PCIe instead of 16."""
+        if framebuffer_in is not None:
+            assert framebuffer_in.dtype == np.float32 and framebuffer_in.shape == (self.h, self.w, 4) and framebuffer_in.flags["C_CONTIGUOUS"]
+        out = np.empty((self.h, self.w, 4), np.uint8)
+        B.check(B.load_library().b200rt_accum_resolve_rgba8(self._h, B.fptr(framebuffer_in), 1 if flip_y else 0,
+                                                            out.ctypes.data_as(C.POINTER(C.c_ubyte))))
         return out
 
 

@@ -69,7 +69,7 @@ EXPORTS = [
     "b200rt_scene_get_bvh_info", "b200rt_scene_device_bytes", "b200rt_default_render_options", "b200rt_render",
     "b200rt_trace_primary", "b200rt_trace_rays", "b200rt_tiles_for_rank", "b200rt_render_tiles_device",
     "b200rt_scene_create_multi", "b200rt_scene_device_count", "b200rt_scene_get_env_alias", "b200rt_scene_get_env_cdf",
-    "b200rt_accum_create", "b200rt_accum_add", "b200rt_accum_samples", "b200rt_accum_resolve", "b200rt_accum_destroy",
+    "b200rt_accum_create", "b200rt_accum_add", "b200rt_accum_samples", "b200rt_accum_resolve", "b200rt_accum_resolve_rgba8", "b200rt_accum_destroy",
     "b200rt_denoise", "b200rt_obj_load", "b200rt_obj_get", "b200rt_obj_destroy", "b200rt_hdr_load", "b200rt_hdr_get", "b200rt_hdr_destroy", "b200rt_env_cdf_search", "b200rt_render_rgba8", "b200rt_render_region", "b200rt_rng_stream", "b200rt_host_alloc", "b200rt_host_free", "b200rt_untile_accumulate_device",
     "b200rt_untile_device", "b200rt_trace_primary_device", "b200rt_trace_rays_device", "b200rt_quantise_rgba8", "b200rt_quantise_rgba8_device", "b200rt_last_error", "b200rt_version",
     "b200rt_render_aovs", "b200rt_render_aovs_device", "b200rt_denoise_guided",
@@ -110,6 +110,7 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
     L.b200rt_accum_add.argtypes = [VP, I, C.POINTER(RenderOptions), C.POINTER(Stats)]
     L.b200rt_accum_samples.argtypes = [VP]
     L.b200rt_accum_resolve.argtypes = [VP, FP, FP]
+    L.b200rt_accum_resolve_rgba8.argtypes = [VP, FP, I, C.POINTER(C.c_ubyte)]
     L.b200rt_accum_destroy.argtypes = [VP]
     L.b200rt_accum_destroy.restype = None
     L.b200rt_denoise.argtypes = [FP, I, I, I, C.c_float, I, C.c_float, FP]

@@ -1055,33 +1055,96 @@ unsigned long long pixels_of_rank(const RenderParams& P, int w, int h)
     return px;
 }
 
-// One rank of a multi-GPU frame, run by its own host thread: render this device's interleaved tiles as mean radiance
-// (B200RT_FLAG_LINEAR_TILES) and push them into rank 0's gather buffer with ONE device-to-device copy (NVLink peer copy).
-struct RankResult { int rc = B200RT_OK; std::string error; unsigned long long rays = 0; float ms = 0.0f; int launches = 0; };
-
-void render_rank(b200rt_scene* r, b200rt_scene* root, RenderParams P, int integrator, size_t tiles_padded, RankResult* out)
+int ensure_gather(b200rt_scene* s, size_t need)
 {
-    auto body = [&]() -> int {
-        ON_DEVICE(r->device);
-        int rc = ensure_scratch(r, r == root ? 0 : tiles_padded * kTilePixels, 0, 0);
-        if (rc) return rc;
-        if (!r->mg_stream) CU(cudaStreamCreateWithFlags(&r->mg_stream, cudaStreamNonBlocking));
-        cudaStream_t st = r->mg_stream;
-        float4* dst = root->d_gather + (size_t)P.rank * tiles_padded * kTilePixels;
-        float4* tiles = r == root ? dst : r->d_tiles;          // rank 0 renders straight into its slice of the gather buffer
-        CU(cudaMemsetAsync(r->d_rays, 0, sizeof(unsigned long long), st));
-        CU(cudaEventRecord(r->ev0, st));
-        if ((rc = run_integrator(r, P, integrator, nullptr, tiles, st, &out->launches))) return rc;
-        CU(cudaEventRecord(r->ev1, st));
-        if (r != root)
-            CU(cudaMemcpyPeerAsync(dst, root->device, tiles, r->device, (size_t)P.n_rank_tiles * kTilePixels * sizeof(float4), st));
-        CU(cudaStreamSynchronize(st));
-        CU(cudaEventElapsedTime(&out->ms, r->ev0, r->ev1));
-        CU(cudaMemcpy(&out->rays, r->d_rays, sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-        return B200RT_OK;
-    };
-    out->rc = body();
-    if (out->rc) out->error = g_error;
+    if (need <= s->gather_cap) return B200RT_OK;
+    if (s->d_gather) cudaFree(s->d_gather);
+    s->d_gather = nullptr; s->gather_cap = 0;
+    CU(cudaMalloc(&s->d_gather, need * sizeof(float4)));
+    s->gather_cap = need;
+    return B200RT_OK;
+}
+
+int ensure_rgba8(b200rt_scene* s, size_t image_px)
+{
+    if (image_px * 4 <= s->rgba8_cap) return B200RT_OK;
+    if (s->d_rgba8) cudaFree(s->d_rgba8);
+    s->d_rgba8 = nullptr; s->rgba8_cap = 0;
+    CU(cudaMalloc(&s->d_rgba8, image_px * 4));
+    s->rgba8_cap = image_px * 4;
+    return B200RT_OK;
+}
+
+// the stream a rank of a multi-GPU frame or accumulation runs on, created on the rank's device on first use
+int ensure_rank_stream(b200rt_scene* r)
+{
+    if (r->mg_stream) return B200RT_OK;
+    ON_DEVICE(r->device);
+    CU(cudaStreamCreateWithFlags(&r->mg_stream, cudaStreamNonBlocking));
+    return B200RT_OK;
+}
+
+struct RankResult { unsigned long long rays = 0; float ms = 0.0f; int launches = 0; };
+
+// One rank's share of a frame or of an accumulation chunk: the integrator over the tiles P names, into `tiles`, on stream `st` of
+// the rank's device. Returns when it has finished, with its kernel time and ray count in *out.
+int integrate_rank(b200rt_scene* r, const RenderParams& P, int integrator, float4* tiles, cudaStream_t st, RankResult* out)
+{
+    ON_DEVICE(r->device);
+    int rc = ensure_scratch(r, 0, 0, 0);
+    if (rc) return rc;
+    CU(cudaMemsetAsync(r->d_rays, 0, sizeof(unsigned long long), st));
+    CU(cudaEventRecord(r->ev0, st));
+    if ((rc = run_integrator(r, P, integrator, nullptr, tiles, st, &out->launches))) return rc;
+    CU(cudaEventRecord(r->ev1, st));
+    CU(cudaStreamSynchronize(st));
+    CU(cudaEventElapsedTime(&out->ms, r->ev0, r->ev1));
+    CU(cudaMemcpy(&out->rays, r->d_rays, sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+    return B200RT_OK;
+}
+
+// rank `rank`'s n_tiles tiles into its slice of rank 0's gather buffer: ONE device-to-device copy on the rank's stream (NVLink peer
+// copy; a plain copy when the rank shares rank 0's device). Returns when the copy has finished.
+int gather_rank(b200rt_scene* r, b200rt_scene* root, const float4* tiles, int rank, int n_tiles, size_t tiles_padded)
+{
+    if (n_tiles <= 0) return B200RT_OK;
+    int rc = ensure_rank_stream(r);
+    if (rc) return rc;
+    ON_DEVICE(r->device);
+    float4* dst = root->d_gather + (size_t)rank * tiles_padded * kTilePixels;
+    CU(cudaMemcpyPeerAsync(dst, root->device, tiles, r->device, (size_t)n_tiles * kTilePixels * sizeof(float4), r->mg_stream));
+    CU(cudaStreamSynchronize(r->mg_stream));
+    return B200RT_OK;
+}
+
+// Runs rank_body(d) for every rank d < n_dev: rank 0 on the calling thread, every other rank on a host thread of its own, so that
+// each device launches and waits on its own. A failure is reported as the lowest failing rank's: "device rank d: ...".
+template <typename F>
+int run_ranks(int n_dev, F rank_body)
+{
+    std::vector<int> rc((size_t)n_dev, B200RT_OK);
+    std::vector<std::string> err((size_t)n_dev);
+    auto run = [&](int d) { rc[(size_t)d] = rank_body(d); if (rc[(size_t)d]) err[(size_t)d] = g_error; };
+    std::vector<std::thread> threads;
+    for (int d = 1; d < n_dev; d++) threads.emplace_back(run, d);
+    run(0);
+    for (std::thread& t : threads) t.join();
+    for (int d = 0; d < n_dev; d++)
+        if (rc[(size_t)d]) { g_error = "device rank " + std::to_string(d) + ": " + err[(size_t)d]; return rc[(size_t)d]; }
+    return B200RT_OK;
+}
+
+// One rank of a multi-GPU frame: render this device's interleaved tiles as mean radiance (B200RT_FLAG_LINEAR_TILES) and push them
+// into rank 0's gather buffer. Rank 0 renders straight into its slice of the gather buffer.
+int render_rank(b200rt_scene* r, b200rt_scene* root, const RenderParams& P, int integrator, size_t tiles_padded, RankResult* out)
+{
+    ON_DEVICE(r->device);
+    int rc = ensure_scratch(r, r == root ? 0 : tiles_padded * kTilePixels, 0, 0);
+    if (rc) return rc;
+    if ((rc = ensure_rank_stream(r))) return rc;
+    if (r == root) return integrate_rank(r, P, integrator, root->d_gather + (size_t)P.rank * tiles_padded * kTilePixels, r->mg_stream, out);
+    if ((rc = integrate_rank(r, P, integrator, r->d_tiles, r->mg_stream, out))) return rc;
+    return gather_rank(r, root, r->d_tiles, P.rank, P.n_rank_tiles, tiles_padded);
 }
 
 // The whole frame: framebuffer in (or Color::Black()), integrator on one or several devices, un-tile, optional RGBA8 output
@@ -1101,13 +1164,7 @@ int render_frame(b200rt_scene* s, const float* camera17, int w, int h, int spp, 
     ON_DEVICE(s->device);
     const size_t image_px = (size_t)w * h;
     if ((rc = ensure_scratch(s, (size_t)std::max(P.n_rank_tiles, 1) * kTilePixels, image_px, 0))) return rc;
-    if (rgba8_out && image_px * 4 > s->rgba8_cap)
-    {
-        if (s->d_rgba8) cudaFree(s->d_rgba8);
-        s->d_rgba8 = nullptr; s->rgba8_cap = 0;
-        CU(cudaMalloc(&s->d_rgba8, image_px * 4));
-        s->rgba8_cap = image_px * 4;
-    }
+    if (rgba8_out && (rc = ensure_rgba8(s, image_px))) return rc;
     cudaStream_t st = 0;
     unsigned long long h2d = 17 * sizeof(float), d2h = 0, rays = 0;
     int launches = 0;
@@ -1132,40 +1189,21 @@ int render_frame(b200rt_scene* s, const float* camera17, int w, int h, int spp, 
         // N devices, one host thread each: interleaved tiles, scene replicated, mean radiance gathered on rank 0's device, where
         // `framebuffer += final; tone map` (render_kernel.cpp:169-180) happens against the incoming framebuffer
         const size_t tiles_padded = (size_t)b200rt_tiles_for_rank(w, h, 0, n_dev);
-        const size_t need = tiles_padded * kTilePixels * (size_t)n_dev;
-        if (need > s->gather_cap)
-        {
-            if (s->d_gather) cudaFree(s->d_gather);
-            s->d_gather = nullptr; s->gather_cap = 0;
-            CU(cudaMalloc(&s->d_gather, need * sizeof(float4)));
-            s->gather_cap = need;
-        }
+        if ((rc = ensure_gather(s, tiles_padded * kTilePixels * (size_t)n_dev))) return rc;
         if (!fb_zero) { if ((rc = copy_to_device(s, s->d_image, fb_in, image_px * sizeof(float4), st))) return rc; h2d += image_px * sizeof(float4); }
         else CU(launch_fill_f4(s->d_image, image_px, make_float4(0.0f, 0.0f, 0.0f, 1.0f), st));
         CU(cudaStreamSynchronize(st));
         std::vector<RankResult> res((size_t)n_dev);
-        std::vector<std::thread> threads;
-        for (int d = 0; d < n_dev; d++)
-        {
+        rc = run_ranks(n_dev, [&](int d) {
             RenderParams Pd = P;
             Pd.rank = d; Pd.world = n_dev;
             Pd.n_rank_tiles = b200rt_tiles_for_rank(w, h, d, n_dev);
             Pd.flags |= B200RT_FLAG_LINEAR_TILES;
-            b200rt_scene* r = d == 0 ? s : s->replicas[(size_t)d - 1];
-            if (d == 0) continue;
-            threads.emplace_back(render_rank, r, s, Pd, integrator, tiles_padded, &res[(size_t)d]);
-        }
-        {
-            RenderParams P0 = P;
-            P0.rank = 0; P0.world = n_dev;
-            P0.n_rank_tiles = b200rt_tiles_for_rank(w, h, 0, n_dev);
-            P0.flags |= B200RT_FLAG_LINEAR_TILES;
-            render_rank(s, s, P0, integrator, tiles_padded, &res[0]);
-        }
-        for (std::thread& t : threads) t.join();
+            return render_rank(d == 0 ? s : s->replicas[(size_t)d - 1], s, Pd, integrator, tiles_padded, &res[(size_t)d]);
+        });
+        if (rc) return rc;
         for (int d = 0; d < n_dev; d++)
         {
-            if (res[(size_t)d].rc) { g_error = "device rank " + std::to_string(d) + ": " + res[(size_t)d].error; return res[(size_t)d].rc; }
             rays += res[(size_t)d].rays;
             launches += res[(size_t)d].launches;
             kernel_ms = std::max(kernel_ms, res[(size_t)d].ms);
@@ -1267,14 +1305,65 @@ int b200rt_render_region(b200rt_scene* s, const float* camera17, int w, int h, i
     return B200RT_OK;
 }
 
+} // extern "C"
+
+// An accumulator keeps, for every rank d of its scene (rank 0 = the scene, rank d = replicas[d - 1]), the generator state, the linear
+// radiance sum and the mean-radiance tiles of the 16x16 tiles d owns (tile_id % n_ranks == d), tile-major, on that rank's device. A
+// single-device scene has one rank that owns the whole frame. A rank owns no tile when the frame has fewer tiles than there are ranks.
 struct b200rt_accum
 {
+    struct Rank
+    {
+        b200rt_scene* scene = nullptr;
+        int n_tiles = 0;
+        uint32_t* d_rng = nullptr; float4* d_sum = nullptr; float4* d_tiles = nullptr;
+    };
     b200rt_scene* scene = nullptr;
     float camera17[17] = {};
     int w = 0, h = 0, spp_total = 0, bounces = 0, done = 0;
-    size_t n_slots = 0;                  // tile-major pixel slots of the whole frame
-    uint32_t* d_rng = nullptr; float4* d_sum = nullptr; float4* d_tiles = nullptr;
+    std::vector<Rank> ranks;
 };
+
+namespace {
+
+// tone_map(fb_in + mean radiance so far) into fb_out, or its RGBA8 quantisation into rgba8_out (exactly one is non-NULL). On a
+// multi-device scene the ranks' tiles are first gathered into rank 0's gather buffer.
+int accum_resolve(b200rt_accum* a, const float* fb_in, float* fb_out, unsigned char* rgba8_out, int flip_y)
+{
+    if (!a || (!fb_out && !rgba8_out)) return fail(B200RT_ERR_ARG, "NULL argument");
+    if (a->done <= 0) return fail(B200RT_ERR_ARG, "nothing accumulated yet");
+    b200rt_scene* s = a->scene;
+    const int n_dev = (int)a->ranks.size();
+    ON_DEVICE(s->device);
+    const size_t image_px = (size_t)a->w * a->h;
+    int rc = ensure_scratch(s, 0, image_px, 0);
+    if (rc) return rc;
+    if (rgba8_out && (rc = ensure_rgba8(s, image_px))) return rc;
+    const float4* gathered = a->ranks[0].d_tiles;
+    int tiles_padded = a->ranks[0].n_tiles;
+    if (n_dev > 1)
+    {
+        tiles_padded = b200rt_tiles_for_rank(a->w, a->h, 0, n_dev);
+        if ((rc = ensure_gather(s, (size_t)tiles_padded * kTilePixels * n_dev))) return rc;
+        for (int d = 0; d < n_dev; d++)
+        {
+            const b200rt_accum::Rank& k = a->ranks[(size_t)d];
+            if ((rc = gather_rank(k.scene, s, k.d_tiles, d, k.n_tiles, (size_t)tiles_padded))) return rc;
+        }
+        gathered = s->d_gather;
+    }
+    cudaStream_t st = 0;
+    if (fb_in) { if ((rc = copy_to_device(s, s->d_image, fb_in, image_px * sizeof(float4), st))) return rc; }
+    else CU(launch_fill_f4(s->d_image, image_px, make_float4(0.0f, 0.0f, 0.0f, 1.0f), st));
+    CU(launch_untile_accumulate(gathered, tiles_padded, n_dev, a->w, a->h, s->d_image, st));
+    if (!rgba8_out) return copy_to_host(s, fb_out, s->d_image, image_px * sizeof(float4), st);
+    CU(launch_quantise_rgba8(s->d_image, a->w, a->h, flip_y, s->d_rgba8, st));
+    return copy_to_host(s, rgba8_out, s->d_rgba8, image_px * 4, st);
+}
+
+} // namespace
+
+extern "C" {
 
 int b200rt_accum_create(b200rt_scene* s, const float* camera17, int w, int h, int spp_total, int bounces, b200rt_accum** out)
 {
@@ -1282,17 +1371,28 @@ int b200rt_accum_create(b200rt_scene* s, const float* camera17, int w, int h, in
     *out = nullptr;
     if (!s || !camera17) return fail(B200RT_ERR_ARG, "scene and camera must not be NULL");
     if (w <= 0 || h <= 0 || spp_total <= 0 || bounces <= 0) return fail(B200RT_ERR_ARG, "bad accumulator arguments");
-    if (!s->replicas.empty()) return fail(B200RT_ERR_ARG, "accumulators run on single-device scenes");
     ON_DEVICE(s->device);
     b200rt_accum* a = new (std::nothrow) b200rt_accum;
     if (!a) return fail(B200RT_ERR_ALLOC, "out of host memory");
     a->scene = s; a->w = w; a->h = h; a->spp_total = spp_total; a->bounces = bounces;
     std::memcpy(a->camera17, camera17, sizeof(a->camera17));
-    a->n_slots = (size_t)b200rt_tiles_for_rank(w, h, 0, 1) * kTilePixels;
-    cudaError_t e = cudaMalloc(&a->d_rng, a->n_slots * sizeof(uint32_t));
-    if (e == cudaSuccess) e = cudaMalloc(&a->d_sum, a->n_slots * sizeof(float4));
-    if (e == cudaSuccess) e = cudaMalloc(&a->d_tiles, a->n_slots * sizeof(float4));
-    if (e == cudaSuccess) e = cudaMemset(a->d_tiles, 0, a->n_slots * sizeof(float4));
+    const int n_dev = 1 + (int)s->replicas.size();
+    a->ranks.resize((size_t)n_dev);
+    cudaError_t e = cudaSuccess;
+    for (int d = 0; d < n_dev && e == cudaSuccess; d++)
+    {
+        b200rt_accum::Rank& k = a->ranks[(size_t)d];
+        k.scene = d == 0 ? s : s->replicas[(size_t)d - 1];
+        k.n_tiles = b200rt_tiles_for_rank(w, h, d, n_dev);
+        if (!k.n_tiles) continue;
+        const size_t n_slots = (size_t)k.n_tiles * kTilePixels;
+        DeviceScope scope(k.scene->device);
+        e = scope.err;
+        if (e == cudaSuccess) e = cudaMalloc(&k.d_rng, n_slots * sizeof(uint32_t));
+        if (e == cudaSuccess) e = cudaMalloc(&k.d_sum, n_slots * sizeof(float4));
+        if (e == cudaSuccess) e = cudaMalloc(&k.d_tiles, n_slots * sizeof(float4));
+        if (e == cudaSuccess) e = cudaMemset(k.d_tiles, 0, n_slots * sizeof(float4));
+    }
     if (e != cudaSuccess) { b200rt_accum_destroy(a); return fail(B200RT_ERR_CUDA, "accumulator allocation: %s", cudaGetErrorString(e)); }
     *out = a;
     return B200RT_OK;
@@ -1312,27 +1412,42 @@ int b200rt_accum_add(b200rt_accum* a, int n_samples, const b200rt_render_options
     const int integrator = opts ? opts->integrator : B200RT_INTEGRATOR_WAVEFRONT;
     if (integrator != B200RT_INTEGRATOR_WAVEFRONT && integrator != B200RT_INTEGRATOR_PERSISTENT)
         return fail(B200RT_ERR_ARG, "accumulators run on the wavefront or the persistent integrator");
+    const int n_dev = (int)a->ranks.size();
+    // checked here for every rank, so that a refused add has launched on none of them
+    for (const b200rt_accum::Rank& k : a->ranks)
+        if ((P.flags & B200RT_FLAG_ENV_ALIAS) && !k.scene->d_alias) return fail(B200RT_ERR_ARG, "B200RT_FLAG_ENV_ALIAS needs b200rt_scene_build_env_alias() first");
+    auto t0 = std::chrono::high_resolution_clock::now();
     ON_DEVICE(s->device);
-    if ((rc = ensure_scratch(s, 0, 0, 0))) return rc;
     P.flags |= B200RT_FLAG_LINEAR_TILES;
     P.sample_begin = a->done; P.sample_end = a->done + n_samples;
-    P.acc_rng = a->d_rng; P.acc_sum = a->d_sum;
-    cudaStream_t st = 0;
-    CU(cudaMemsetAsync(s->d_rays, 0, sizeof(unsigned long long), st));
-    CU(cudaEventRecord(s->ev0, st));
-    int launches = 0;
-    if ((rc = run_integrator(s, P, integrator, nullptr, a->d_tiles, st, &launches))) return rc;
-    CU(cudaEventRecord(s->ev1, st));
-    CU(cudaStreamSynchronize(st));
+    std::vector<RankResult> res((size_t)n_dev);
+    // rank d continues the pixels of its own tiles from its own state; nothing crosses devices until a resolve
+    auto add_rank = [&](int d) -> int {
+        const b200rt_accum::Rank& k = a->ranks[(size_t)d];
+        if (!k.n_tiles) return B200RT_OK;
+        RenderParams Pd = P;
+        Pd.rank = d; Pd.world = n_dev; Pd.n_rank_tiles = k.n_tiles;
+        Pd.acc_rng = k.d_rng; Pd.acc_sum = k.d_sum;
+        cudaStream_t st = 0;                 // a single-device accumulator runs on the caller's thread and the legacy stream
+        if (n_dev > 1)
+        {
+            const int rc_s = ensure_rank_stream(k.scene);
+            if (rc_s) return rc_s;
+            st = k.scene->mg_stream;
+        }
+        return integrate_rank(k.scene, Pd, integrator, k.d_tiles, st, &res[(size_t)d]);
+    };
+    rc = n_dev == 1 ? add_rank(0) : run_ranks(n_dev, add_rank);
+    if (rc) return rc;
     a->done += n_samples;
     if (stats)
     {
         std::memset(stats, 0, sizeof(*stats));
         float ms = 0.0f;
-        CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
-        CU(cudaMemcpy(&stats->rays, s->d_rays, sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+        for (const RankResult& r : res) { stats->rays += r.rays; stats->gpu_launches += r.launches; ms = std::max(ms, r.ms); }
         stats->samples = (unsigned long long)a->w * a->h * (unsigned long long)n_samples;
-        stats->kernel_ms = ms; stats->total_ms = ms; stats->gpu_launches = launches;
+        stats->kernel_ms = ms;
+        stats->total_ms = n_dev == 1 ? ms : std::chrono::duration<double, std::milli>(std::chrono::high_resolution_clock::now() - t0).count();
         if ((rc = fill_kernel_times(s, stats))) return rc;
     }
     return B200RT_OK;
@@ -1340,27 +1455,23 @@ int b200rt_accum_add(b200rt_accum* a, int n_samples, const b200rt_render_options
 
 int b200rt_accum_resolve(b200rt_accum* a, const float* fb_in, float* fb_out)
 {
-    if (!a || !fb_out) return fail(B200RT_ERR_ARG, "NULL argument");
-    if (a->done <= 0) return fail(B200RT_ERR_ARG, "nothing accumulated yet");
-    b200rt_scene* s = a->scene;
-    ON_DEVICE(s->device);
-    const size_t image_px = (size_t)a->w * a->h;
-    int rc = ensure_scratch(s, 0, image_px, 0);
-    if (rc) return rc;
-    cudaStream_t st = 0;
-    if (fb_in) { if ((rc = copy_to_device(s, s->d_image, fb_in, image_px * sizeof(float4), st))) return rc; }
-    else CU(launch_fill_f4(s->d_image, image_px, make_float4(0.0f, 0.0f, 0.0f, 1.0f), st));
-    CU(launch_untile_accumulate(a->d_tiles, (int)(a->n_slots / kTilePixels), 1, a->w, a->h, s->d_image, st));
-    return copy_to_host(s, fb_out, s->d_image, image_px * sizeof(float4), st);
+    return accum_resolve(a, fb_in, fb_out, nullptr, 0);
+}
+
+int b200rt_accum_resolve_rgba8(b200rt_accum* a, const float* fb_in, int flip_y, unsigned char* out_rgba8)
+{
+    if (!out_rgba8) return fail(B200RT_ERR_ARG, "out_rgba8 must not be NULL");
+    return accum_resolve(a, fb_in, nullptr, out_rgba8, flip_y);
 }
 
 void b200rt_accum_destroy(b200rt_accum* a)
 {
     if (!a) return;
-    if (a->scene)
+    for (const b200rt_accum::Rank& k : a->ranks)
     {
-        DeviceScope scope(a->scene->device);
-        cudaFree(a->d_rng); cudaFree(a->d_sum); cudaFree(a->d_tiles);
+        if (!k.scene) continue;
+        DeviceScope scope(k.scene->device);
+        cudaFree(k.d_rng); cudaFree(k.d_sum); cudaFree(k.d_tiles);
     }
     delete a;
 }
