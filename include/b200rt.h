@@ -267,6 +267,39 @@ int b200rt_accum_resolve(b200rt_accum* acc, const float* framebuffer_rgba_in_or_
 int b200rt_accum_resolve_rgba8(b200rt_accum* acc, const float* framebuffer_rgba_in_or_null, int flip_y, unsigned char* out_rgba8);
 void b200rt_accum_destroy(b200rt_accum* acc);
 
+/* ---- geometry updates ------------------------------------------------------------------------------------------------------------
+ * New vertex positions for the scene's triangles, in place: no rebuild, no new upload of materials, lights or environment tables,
+ * and the wavefront state and every accumulator stay. tri_xyz9 holds n_tri triangles in the creation layout; triangle i replaces
+ * triangle i given at creation.
+ *   Fixed topology: n_tri must equal the scene's triangle count. Triangle order, material indices, the emissive list, spheres and the
+ *     environment stay as they are. The tree keeps its shape (which triangles share a leaf, which subtrees share a node) and every
+ *     box of both layouts, the diagonal slabs and the triangle stream are recomputed on the device from the new vertices, one tree
+ *     level per launch, deepest first.
+ *   Exact: closest hits do not depend on the tree's shape (ties go to the lowest original index), so after an update every entry point
+ *     returns bit for bit what a scene freshly created from the new vertices returns: framebuffers, RGBA8, regions, feature buffers,
+ *     primary maps, closest-hit ray batches, any-hit flags and ray counts (an any-hit t is whichever hit the traversal meets first,
+ *     which depends on the tree's shape, for a fresh scene too). Only the speed differs: a tree refitted far from the shape it was
+ *     built for has larger, more overlapping boxes. b200rt_scene_get_bvh_info then reports the refitted tree's sah_cost (sum over the binary records of child
+ *     area / root area, leaves weighted by their triangle count, in double), so a caller can watch it grow and recreate the scene.
+ *   Refusals change nothing: B200RT_ERR_ARG for a NULL pointer, a wrong n_tri, or any NaN or +-Inf coordinate (no box can bound it;
+ *     the check is the first device pass and runs before anything resident is written).
+ *   Blocking, like b200rt_scene_set_materials. Multi-device scenes: every replica is updated on its own device, from one host thread
+ *     each, and the replicas stay byte-identical.
+ *   Accumulators survive an update, and samples added afterwards see the new geometry. An accumulation that spans an update mixes
+ *     both geometries in one frame; that is the caller's choice.
+ * stats (may be NULL): kernel_ms, total_ms, gpu_launches, h2d_bytes.
+ * _device: dev_tri_xyz9 is device memory of the scene's first device; the update is ordered after the caller's prior work on
+ * cuda_stream (a cudaStream_t of that device; NULL = legacy default stream), then synchronises. Vertices produced on the GPU never
+ * cross PCIe; other replicas receive them device to device. The caller's current device is restored. */
+int b200rt_scene_update_triangles(b200rt_scene* scene, const float* tri_xyz9, int n_tri, b200rt_stats* stats_or_null);
+int b200rt_scene_update_triangles_device(b200rt_scene* scene, const void* dev_tri_xyz9, int n_tri,
+                                         void* cuda_stream, b200rt_stats* stats_or_null);
+/* Test / inspection hook: downloads replica `replica`'s resident arrays. Sizes from b200rt_scene_get_bvh_info: n_wide_nodes records
+ * of 80 bytes (csrc/bvh_build.h WideNode), n_inner_nodes binary records of 16 floats each for axis and diag (diag is written only
+ * when has_diag_slabs), n_triangles leaf records of 12 floats. Any output may be NULL. */
+int b200rt_scene_get_bvh_arrays(b200rt_scene* scene, int replica, void* wide80_out, float* axis16_out,
+                                float* diag16_out, float* tris12_out);
+
 /* Parity hook for xorshift32_generator (include/xorshift.h:10-31) as ray_trace_pixel seeds it (render_kernel.cpp:77-82):
  * *state_out = the generator state of pixel (x, y) after the 10 warm-up draws (seed 31 + x*y*spp in wrapping int arithmetic),
  * floats_out[0..n) = the next n floats. Runs on the calling thread's current device. */

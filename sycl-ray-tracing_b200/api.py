@@ -460,6 +460,38 @@ class Scene:
         self.mats = materials_to_array(materials)
         B.check(B.load_library().b200rt_scene_set_materials(self._h, B.fptr(self.mats), len(self.mats)))
 
+    def update_triangles(self, triangles) -> dict:
+        """New vertex positions for the scene's triangles (b200rt_scene_update_triangles): (n, 9) float32, n = the scene's triangle
+        count, triangle i replacing triangle i. The BVH is refitted on the device; every result afterwards equals a fresh Scene's
+        from these vertices bit for bit. Returns the stats (kernel_ms, total_ms, gpu_launches, h2d_bytes)."""
+        tri = _f32(triangles)
+        if tri.shape != self.tri.shape:
+            raise ValueError(f"triangles have shape {tri.shape}; this scene takes {self.tri.shape} (an update keeps the topology)")
+        st = B.Stats()
+        B.check(B.load_library().b200rt_scene_update_triangles(self._h, B.fptr(tri), len(tri), C.byref(st)))
+        self.tri = tri.copy() if tri is triangles else tri
+        return st.as_dict()
+
+    def update_triangles_device(self, dev_ptr: int, n: int, stream_ptr: int = 0) -> dict:
+        """update_triangles from device memory of the scene's first device (b200rt_scene_update_triangles_device), e.g.
+        tensor.data_ptr() of an (n, 9) float32 CUDA tensor, ordered after the work already queued on stream_ptr. self.tri is not
+        updated (the vertices never reach the host). Returns the stats."""
+        st = B.Stats()
+        B.check(B.load_library().b200rt_scene_update_triangles_device(self._h, C.c_void_p(dev_ptr), n, C.c_void_p(stream_ptr), C.byref(st)))
+        return st.as_dict()
+
+    def bvh_arrays(self, replica: int = 0) -> dict:
+        """The resident BVH of one replica, downloaded (b200rt_scene_get_bvh_arrays): wide (WIDE_NODE_DTYPE records), axis and diag
+        ((n_inner_nodes, 16) float32; diag is empty without diagonal slabs) and tris ((n_triangles, 12) float32)."""
+        info = self.bvh_info()
+        wide = np.zeros(info["n_wide_nodes"], WIDE_NODE_DTYPE)
+        axis = np.zeros((info["n_inner_nodes"], 16), np.float32)
+        diag = np.zeros((info["n_inner_nodes"] if info["has_diag_slabs"] else 0, 16), np.float32)
+        tris = np.zeros((info["n_triangles"], 12), np.float32)
+        B.check(B.load_library().b200rt_scene_get_bvh_arrays(self._h, replica, wide.ctypes.data_as(C.c_void_p), B.fptr(axis),
+                                                             B.fptr(diag) if len(diag) else None, B.fptr(tris)))
+        return dict(wide=wide, axis=axis, diag=diag, tris=tris)
+
     @staticmethod
     def _opts(integrator=B.INTEGRATOR_WAVEFRONT, flags=0, rank=0, world=1):
         return B.RenderOptions(integrator, flags, rank, world)

@@ -73,6 +73,7 @@ EXPORTS = [
     "b200rt_denoise", "b200rt_obj_load", "b200rt_obj_get", "b200rt_obj_destroy", "b200rt_hdr_load", "b200rt_hdr_get", "b200rt_hdr_destroy", "b200rt_env_cdf_search", "b200rt_render_rgba8", "b200rt_render_region", "b200rt_rng_stream", "b200rt_host_alloc", "b200rt_host_free", "b200rt_untile_accumulate_device",
     "b200rt_untile_device", "b200rt_trace_primary_device", "b200rt_trace_rays_device", "b200rt_quantise_rgba8", "b200rt_quantise_rgba8_device", "b200rt_last_error", "b200rt_version",
     "b200rt_render_aovs", "b200rt_render_aovs_device", "b200rt_denoise_guided",
+    "b200rt_scene_update_triangles", "b200rt_scene_update_triangles_device", "b200rt_scene_get_bvh_arrays",
 ]
 
 _lib = None
@@ -132,6 +133,9 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
     L.b200rt_scene_destroy.argtypes = [VP]
     L.b200rt_scene_destroy.restype = None
     L.b200rt_scene_set_materials.argtypes = [VP, FP, I]
+    L.b200rt_scene_update_triangles.argtypes = [VP, FP, I, C.POINTER(Stats)]
+    L.b200rt_scene_update_triangles_device.argtypes = [VP, VP, I, VP, C.POINTER(Stats)]
+    L.b200rt_scene_get_bvh_arrays.argtypes = [VP, I, VP, FP, FP, FP]
     L.b200rt_scene_build_env_alias.argtypes = [VP]
     L.b200rt_env_alias_table.argtypes = [FP, I, I, FP, C.POINTER(C.c_int), C.POINTER(C.c_double)]
     L.b200rt_quantise_rgba8.argtypes = [FP, I, I, I, C.POINTER(C.c_ubyte)]

@@ -14,8 +14,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, os.environ.get("B200RT_BUILD_LIB", "libb200rt.so"))
-SOURCES = ["capi.cu", "kernels.cu", "wavefront.cu", "persist.cu", "env_tables.cu", "denoise.cu", "bvh_build_gpu.cu", "bvh_build.cpp", "obj_ingest.cpp", "hdr_ingest.cpp"]
-HEADERS = ["bvh_build.h", "device_types.h", "kernels.h", "pt_device.cuh", "wf_device.cuh", "obj_ingest.h", os.path.join("..", "..", "include", "b200rt.h")]
+SOURCES = ["capi.cu", "kernels.cu", "wavefront.cu", "persist.cu", "env_tables.cu", "denoise.cu", "bvh_build_gpu.cu", "refit.cu", "bvh_build.cpp", "obj_ingest.cpp", "hdr_ingest.cpp"]
+HEADERS = ["bvh_build.h", "bvh_emit.cuh", "device_types.h", "kernels.h", "pt_device.cuh", "wf_device.cuh", "obj_ingest.h", os.path.join("..", "..", "include", "b200rt.h")]
 
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-lineinfo",

@@ -94,6 +94,15 @@ struct b200rt_scene
     DevArray<unsigned char> d_rgba8;      // output stage scratch (b200rt_render_rgba8)
     // pinned staging for copies from / to pageable caller memory: two chunks, ping-pong
     PinnedPtr h_stage[2]; cudaEvent_t stage_ev[2] = { nullptr, nullptr };
+    // geometry updates (b200rt_scene_update_triangles): both layouts' level lists and per-node exact boxes, made on the first update,
+    // kept and counted in `bytes`; the new vertices when they have to be staged on this device
+    bool refit_ready = false;
+    std::vector<int> wide_level, axis_level;
+    int *d_wide_idx = nullptr, *d_axis_idx = nullptr;
+    float4 *d_wide_box = nullptr, *d_axis_box = nullptr;
+    unsigned int* d_refit_misc = nullptr;     // [0] max |coord| bits, [1] non-finite flag, [2] quantisation overflow, [3] walk counter
+    double* d_sah = nullptr;
+    DevArray<float> d_vertices;
 
     ~b200rt_scene() { timeline.destroy(); }
 };
@@ -1115,6 +1124,138 @@ int run_ranks(int n_dev, F rank_body)
     return B200RT_OK;
 }
 
+// The refit state of one replica: level lists by a breadth-first walk of the resident records (which it only reads) and the per-node
+// exact-box arrays. Made once; a failure leaves the scene as it was, and the next update tries again.
+int ensure_refit(b200rt_scene* r)
+{
+    if (r->refit_ready) return B200RT_OK;
+    ON_DEVICE(r->device);
+    const size_t n_wide = (size_t)r->info.n_wide_nodes, n_axis = (size_t)r->info.n_inner_nodes;
+    int rc = B200RT_OK;
+    if (!r->d_refit_misc && (rc = device_alloc(r, &r->d_refit_misc, 4))) return rc;
+    if (!r->d_sah && (rc = device_alloc(r, &r->d_sah, refit_sah_scratch_doubles()))) return rc;
+    if (!r->d_wide_idx && (rc = device_alloc(r, &r->d_wide_idx, n_wide))) return rc;
+    if (!r->d_axis_idx && (rc = device_alloc(r, &r->d_axis_idx, n_axis))) return rc;
+    if (!r->d_wide_box && (rc = device_alloc(r, &r->d_wide_box, 2 * n_wide))) return rc;
+    if (!r->d_axis_box && (rc = device_alloc(r, &r->d_axis_box, 4 * n_axis))) return rc;
+    const cudaError_t e = refit_levels(reinterpret_cast<const WideNode*>(r->dev.wide), (int)n_wide, reinterpret_cast<const AxisNode*>(r->dev.axis),
+                                       (int)n_axis, r->d_wide_idx, r->d_axis_idx, reinterpret_cast<int*>(r->d_refit_misc + 3),
+                                       r->wide_level, r->axis_level, 0);
+    if (e == cudaErrorInvalidValue) return fail(B200RT_ERR_ARG, "the scene's BVH records do not form one tree rooted at record 0");
+    if (e != cudaSuccess) return fail(B200RT_ERR_CUDA, "BVH level lists: %s", cudaGetErrorString(e));
+    r->refit_ready = true;
+    return B200RT_OK;
+}
+
+// Refits replica r to the new vertices `v` (on r's device) on stream st: triangle stream, both layouts level by level, the SAH cost.
+// Returns when it has finished, with the kernel time and the launch count in *out.
+int refit_rank(b200rt_scene* r, const float* v, float abs_pad, cudaStream_t st, LaunchResult* out)
+{
+    ON_DEVICE(r->device);
+    int* overflow = reinterpret_cast<int*>(r->d_refit_misc + 2);
+    CU(cudaMemsetAsync(overflow, 0, sizeof(int), st));
+    RefitArgs A;
+    A.tri9 = v;
+    A.tris = const_cast<float4*>(r->dev.tris);
+    A.wide = reinterpret_cast<WideNode*>(const_cast<float4*>(r->dev.wide));
+    A.axis = reinterpret_cast<AxisNode*>(const_cast<float4*>(r->dev.axis));
+    A.diag = r->dev.has_diag ? reinterpret_cast<DiagNode*>(const_cast<float4*>(r->dev.diag)) : nullptr;
+    A.wide_idx = r->d_wide_idx; A.axis_idx = r->d_axis_idx;
+    A.wide_level = &r->wide_level; A.axis_level = &r->axis_level;
+    A.wide_box = r->d_wide_box; A.axis_box = r->d_axis_box;
+    A.n_tri = r->dev.n_tri; A.n_axis = r->info.n_inner_nodes;
+    A.abs_pad = abs_pad;
+    A.overflow = overflow;
+    A.sah = r->d_sah;
+    int flag = 0;
+    double sah = 0.0;
+    const int rc = timed_launch(r, st, false, out, [&] { CU(refit_tree(A, st, &out->launches)); return B200RT_OK; }, [&] {
+        CU(cudaMemcpyAsync(&flag, overflow, sizeof(int), cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(&sah, r->d_sah + refit_sah_scratch_doubles() - 1, sizeof(double), cudaMemcpyDeviceToHost, st));
+        return B200RT_OK;
+    });
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(st));
+    if (flag) return fail(B200RT_ERR_CUDA, "wide BVH quantisation overflow in the refit");
+    r->info.sah_cost = sah;
+    return B200RT_OK;
+}
+
+// b200rt_scene_update_triangles[_device]: new vertices for every replica of the scene. src is host memory, or (src_on_device) device
+// memory of the scene's first device that the caller's stream `caller_st` produces.
+int update_triangles(b200rt_scene* s, const void* src, bool src_on_device, int n_tri, cudaStream_t caller_st, b200rt_stats* stats)
+{
+    if (!s || !src) return fail(B200RT_ERR_ARG, "scene and triangle buffer must not be NULL");
+    if (n_tri != s->dev.n_tri) return fail(B200RT_ERR_ARG, "%d triangles, but the scene has %d (an update keeps the topology)", n_tri, s->dev.n_tri);
+    if (stats) std::memset(stats, 0, sizeof(*stats));
+    if (n_tri == 0) return B200RT_OK;
+    int rc = require_device("b200rt_scene_update_triangles");
+    if (rc) return rc;
+    const auto t0 = std::chrono::high_resolution_clock::now();
+    if (src_on_device)
+    {
+        cudaPointerAttributes pa;
+        if (cudaPointerGetAttributes(&pa, src) != cudaSuccess) { cudaGetLastError(); pa.type = cudaMemoryTypeUnregistered; }
+        if (!((pa.type == cudaMemoryTypeDevice && pa.device == s->device) || pa.type == cudaMemoryTypeManaged))
+            return fail(B200RT_ERR_ARG, "dev_tri_xyz9 must be device memory of the scene's first device (%d)", s->device);
+    }
+    std::vector<b200rt_scene*> ranks(1, s);
+    ranks.insert(ranks.end(), s->replicas.begin(), s->replicas.end());
+    const int n_dev = (int)ranks.size();
+    const size_t bytes = 9 * (size_t)n_tri * sizeof(float);
+    // 1. every replica's state and buffers: nothing resident is written yet
+    for (int d = 0; d < n_dev; d++)
+    {
+        b200rt_scene* r = ranks[(size_t)d];
+        if ((rc = ensure_refit(r))) return rc;
+        ON_DEVICE(r->device);
+        if ((rc = ensure_scratch(r, 0, 0, 0))) return rc;
+        if (d > 0 && (rc = ensure_rank_stream(r))) return rc;
+        if ((d > 0 || !src_on_device) && r->d_vertices.cap < 9 * (size_t)n_tri) CU(r->d_vertices.grow(9 * (size_t)n_tri));
+    }
+    // 2. the first device: the input there, then the extent pass; a non-finite coordinate refuses the update
+    ON_DEVICE(s->device);
+    const cudaStream_t st0 = src_on_device ? caller_st : 0;
+    const float* v0 = src_on_device ? static_cast<const float*>(src) : s->d_vertices.get();
+    if (!src_on_device && (rc = copy_to_device(s, s->d_vertices.get(), src, bytes, st0))) return rc;
+    LaunchResult extent;
+    extent.launches = 1;
+    unsigned int misc[2] = { 0, 0 };
+    rc = timed_launch(s, st0, false, &extent, [&] { CU(refit_extent(v0, n_tri, s->d_refit_misc, st0)); return B200RT_OK; },
+                      [&] { CU(cudaMemcpyAsync(misc, s->d_refit_misc, sizeof(misc), cudaMemcpyDeviceToHost, st0)); return B200RT_OK; });
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(st0));
+    if (misc[1]) return fail(B200RT_ERR_ARG, "a vertex coordinate is NaN or infinite: no refitted box can bound it");
+    float scene_abs;
+    std::memcpy(&scene_abs, &misc[0], sizeof(float));
+    const float abs_pad = 2e-6f * scene_abs + 1e-30f;          // as both builders derive it
+    // 3. every replica refits on its own device, from one host thread each; the others receive the vertices first
+    std::vector<LaunchResult> res((size_t)n_dev);
+    rc = run_ranks(n_dev, [&](int d) -> int {
+        if (d == 0) return refit_rank(s, v0, abs_pad, st0, &res[0]);
+        b200rt_scene* r = ranks[(size_t)d];
+        ON_DEVICE(r->device);
+        if (src_on_device) CU(cudaMemcpyPeerAsync(r->d_vertices.get(), r->device, src, s->device, bytes, r->mg_stream));
+        else
+        {
+            const int rc_c = copy_to_device(r, r->d_vertices.get(), src, bytes, r->mg_stream);
+            if (rc_c) return rc_c;
+        }
+        return refit_rank(r, r->d_vertices.get(), abs_pad, r->mg_stream, &res[(size_t)d]);
+    });
+    if (rc) return rc;
+    if (stats)
+    {
+        float ms = 0.0f;
+        stats->gpu_launches = extent.launches;
+        for (const LaunchResult& r : res) { ms = std::max(ms, r.ms); stats->gpu_launches += r.launches; }
+        stats->kernel_ms = extent.ms + ms;
+        stats->h2d_bytes = src_on_device ? 0 : bytes * (unsigned long long)n_dev;
+        stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::high_resolution_clock::now() - t0).count();
+    }
+    return B200RT_OK;
+}
+
 // One rank of a multi-GPU frame: render this device's interleaved tiles as mean radiance (B200RT_FLAG_LINEAR_TILES) and push them
 // into rank 0's gather buffer. Rank 0 renders straight into its slice of the gather buffer.
 int render_rank(b200rt_scene* r, b200rt_scene* root, const RenderParams& P, int integrator, size_t tiles_padded, LaunchResult* out)
@@ -1249,6 +1390,34 @@ int b200rt_render_region(b200rt_scene* s, const float* camera17, int w, int h, i
     launch_stats(r, stats);
     stats->samples = (unsigned long long)px * (unsigned long long)spp;
     stats->h2d_bytes = 17 * sizeof(float); stats->d2h_bytes = px * sizeof(float4);
+    return B200RT_OK;
+}
+
+} // extern "C"
+
+extern "C" {
+
+int b200rt_scene_update_triangles(b200rt_scene* s, const float* tri_xyz9, int n_tri, b200rt_stats* stats)
+{
+    return update_triangles(s, tri_xyz9, false, n_tri, 0, stats);
+}
+
+int b200rt_scene_update_triangles_device(b200rt_scene* s, const void* dev_tri_xyz9, int n_tri, void* cuda_stream, b200rt_stats* stats)
+{
+    return update_triangles(s, dev_tri_xyz9, true, n_tri, (cudaStream_t)cuda_stream, stats);
+}
+
+int b200rt_scene_get_bvh_arrays(b200rt_scene* s, int replica, void* wide80_out, float* axis16_out, float* diag16_out, float* tris12_out)
+{
+    if (!s) return fail(B200RT_ERR_ARG, "NULL scene");
+    if (replica < 0 || replica > (int)s->replicas.size()) return fail(B200RT_ERR_ARG, "replica %d of %d", replica, 1 + (int)s->replicas.size());
+    const b200rt_scene* r = replica == 0 ? s : s->replicas[(size_t)replica - 1];
+    ON_DEVICE(r->device);
+    const size_t n_wide = (size_t)r->info.n_wide_nodes, n_axis = (size_t)r->info.n_inner_nodes, n_tri = (size_t)r->dev.n_tri;
+    if (wide80_out && n_wide) CU(cudaMemcpy(wide80_out, r->dev.wide, n_wide * sizeof(WideNode), cudaMemcpyDeviceToHost));
+    if (axis16_out && n_axis) CU(cudaMemcpy(axis16_out, r->dev.axis, n_axis * sizeof(AxisNode), cudaMemcpyDeviceToHost));
+    if (diag16_out && n_axis && r->dev.has_diag) CU(cudaMemcpy(diag16_out, r->dev.diag, n_axis * sizeof(DiagNode), cudaMemcpyDeviceToHost));
+    if (tris12_out && n_tri) CU(cudaMemcpy(tris12_out, r->dev.tris, n_tri * sizeof(LeafTriangle), cudaMemcpyDeviceToHost));
     return B200RT_OK;
 }
 

@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/b200rt.h"
+#include "bvh_build.h"
 #include "device_types.h"
 
 namespace b200rt {
@@ -90,5 +91,28 @@ int persistent_grid();
 int persistent_slots(int grid);
 cudaError_t run_persistent(const SceneDev& S, const RenderParams& P, const WfBuffers& B, int grid, const float4* fb_in_rowmajor,
                            float4* out_tiles, cudaStream_t stream);
+
+// refit of a resident tree to new vertices of the same triangles (refit.cu; b200rt_scene_update_triangles)
+// misc[0] = max |coord| as float bits, misc[1] = 1 when a coordinate is NaN or +-Inf (misc: 2 words, zeroed here)
+cudaError_t refit_extent(const float* tri9, int n_tri, unsigned int* misc, cudaStream_t stream);
+// the nodes of each layout grouped by tree level, by a breadth-first walk from record 0: level k is idx[level[k] .. level[k + 1]).
+// Synchronises `stream`. cudaErrorInvalidValue: the records do not form one tree rooted at record 0.
+cudaError_t refit_levels(const WideNode* wide, int n_wide, const AxisNode* axis, int n_axis, int* wide_idx, int* axis_idx, int* counter,
+                         std::vector<int>& wide_level, std::vector<int>& axis_level, cudaStream_t stream);
+size_t refit_sah_scratch_doubles();
+struct RefitArgs
+{
+    const float* tri9;                     // new vertices, original triangle order, on this device
+    float4* tris; WideNode* wide; AxisNode* axis; DiagNode* diag;        // the resident arrays (diag: null = not refitted)
+    const int* wide_idx; const int* axis_idx;
+    const std::vector<int>* wide_level; const std::vector<int>* axis_level;
+    float4* wide_box; float4* axis_box;    // per-node exact boxes: 2 float4 per wide node, 4 per binary record
+    int n_tri, n_axis;
+    float abs_pad;
+    int* overflow;                         // set when a quantised box does not fit its node's grid
+    double* sah;                           // refit_sah_scratch_doubles(); the SAH cost lands in the last one
+};
+// triangle stream, then every level of both layouts deepest first, then the SAH cost; *launches = kernels launched
+cudaError_t refit_tree(const RefitArgs& args, cudaStream_t stream, int* launches);
 
 } // namespace b200rt
