@@ -280,7 +280,8 @@ void b200rt_accum_destroy(b200rt_accum* acc);
  *     primary maps, closest-hit ray batches, any-hit flags and ray counts (an any-hit t is whichever hit the traversal meets first,
  *     which depends on the tree's shape, for a fresh scene too). Only the speed differs: a tree refitted far from the shape it was
  *     built for has larger, more overlapping boxes. b200rt_scene_get_bvh_info then reports the refitted tree's sah_cost (sum over the binary records of child
- *     area / root area, leaves weighted by their triangle count, in double), so a caller can watch it grow and recreate the scene.
+ *     area / root area, leaves weighted by their triangle count, in double), so a caller can watch it grow and rebuild the tree
+ *     (b200rt_scene_rebuild_bvh below).
  *   Refusals change nothing: B200RT_ERR_ARG for a NULL pointer, a wrong n_tri, or any NaN or +-Inf coordinate (no box can bound it;
  *     the check is the first device pass and runs before anything resident is written).
  *   Blocking, like b200rt_scene_set_materials. Multi-device scenes: every replica is updated on its own device, from one host thread
@@ -294,6 +295,39 @@ void b200rt_accum_destroy(b200rt_accum* acc);
 int b200rt_scene_update_triangles(b200rt_scene* scene, const float* tri_xyz9, int n_tri, b200rt_stats* stats_or_null);
 int b200rt_scene_update_triangles_device(b200rt_scene* scene, const void* dev_tri_xyz9, int n_tri,
                                          void* cuda_stream, b200rt_stats* stats_or_null);
+/* Rebuilds the scene's BVH in place from new vertex positions, for geometry that has moved too far for a refit to serve it well (a
+ * refitted tree keeps its shape, and its boxes grow and overlap as the motion departs from the shape it was built for; sah_cost
+ * need not show it: a rigid rotation keeps it flat). Everything else stays resident: materials, the emissive list, spheres, the
+ * environment and its tables, the alias table, the wavefront and persistent slot state, and every accumulator. tri_xyz9 holds n_tri
+ * triangles in the creation layout; triangle i replaces triangle i, and n_tri must equal the scene's triangle count.
+ *   The tree is replaced, not refitted: afterwards the scene holds exactly what b200rt_bvh_build_device returns for the new vertices,
+ *     byte for byte (8-ary nodes, triangle stream, binary records, the bvh_info counts and depths), whichever builder serves it: the
+ *     clustering build, the Morton radix tree for inputs clustering gives up on, or the host SAH builder for at most 3 triangles and
+ *     for inputs both device builders decline. A device-built tree has no diagonal slabs, so a host-built scene that is rebuilt
+ *     reports has_diag_slabs = 0, and B200RT_FLAG_DIAG_SLABS then traverses the axis slabs, as on any device-built scene.
+ *   Exact, as an update: every entry point then returns bit for bit what a scene freshly created from the new vertices returns (an
+ *     any-hit t excepted). b200rt_scene_get_bvh_info reports the new tree; build_seconds is the rebuild's wall time and sah_cost the
+ *     refit's device reduction over the new binary records, so it compares with a refitted tree's.
+ *   On the device: the build reads the vertices on the scene's first device and writes the new arrays there. Only the builder's
+ *     top-level sweep (at most ~1 000 clusters) and the few outsized triangles of the top level (at most 45) cross PCIe, and the
+ *     extent pass's and the SAH's results; no tree-sized array does (the host builder's inputs excepted, which are small).
+ *   Refusals change nothing: B200RT_ERR_ARG for a NULL pointer, a wrong n_tri, a NaN or +-Inf coordinate (found by the extent pass
+ *     before anything is built) or more than 2^27 - 1 triangles. The new arrays are built beside the old ones and swapped in only
+ *     when every replica has its copy, so after a refusal, a failed allocation or a CUDA error the scene keeps its old tree, byte for
+ *     byte. Peak device memory holds both trees.
+ *   Blocking. Multi-device scenes: the tree is built once on the first device and copied device to device to every replica, which
+ *     stay byte-identical. The old arrays are freed with cudaFree, which waits for work already queued on the device: a render that
+ *     an earlier stream is still running when the rebuild returns finishes on the old tree.
+ *   Accumulators survive, as for an update. A refit (b200rt_scene_update_triangles) afterwards refits the new tree.
+ * stats (may be NULL): kernel_ms (CUDA events around the extent pass, the build and the SAH on the build's stream; it includes the
+ * builder's host round trips: the top-level sweep and its level-by-level size reads), total_ms, gpu_launches (a library sort or scan
+ * counts as one), h2d_bytes and d2h_bytes (the vertices when they come from the host, and every small copy of the build).
+ * _device: dev_tri_xyz9 is device memory of the scene's first device, read in place; the rebuild is ordered after the caller's prior
+ * work on cuda_stream (a cudaStream_t of that device; NULL = legacy default stream) and runs on it. The caller's current device is
+ * restored. */
+int b200rt_scene_rebuild_bvh(b200rt_scene* scene, const float* tri_xyz9, int n_tri, b200rt_stats* stats_or_null);
+int b200rt_scene_rebuild_bvh_device(b200rt_scene* scene, const void* dev_tri_xyz9, int n_tri,
+                                    void* cuda_stream, b200rt_stats* stats_or_null);
 /* Test / inspection hook: downloads replica `replica`'s resident arrays. Sizes from b200rt_scene_get_bvh_info: n_wide_nodes records
  * of 80 bytes (csrc/bvh_build.h WideNode), n_inner_nodes binary records of 16 floats each for axis and diag (diag is written only
  * when has_diag_slabs), n_triangles leaf records of 12 floats. Any output may be NULL. */

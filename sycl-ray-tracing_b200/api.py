@@ -480,6 +480,27 @@ class Scene:
         B.check(B.load_library().b200rt_scene_update_triangles_device(self._h, C.c_void_p(dev_ptr), n, C.c_void_p(stream_ptr), C.byref(st)))
         return st.as_dict()
 
+    def rebuild_bvh(self, triangles) -> dict:
+        """New vertex positions, as update_triangles, with the BVH rebuilt on the device instead of refitted
+        (b200rt_scene_rebuild_bvh): the scene then holds exactly the tree BVH(triangles, on_device=True) builds, and every result
+        equals a fresh Scene's from these vertices bit for bit. For motion that has left the refitted tree slow. Returns the stats
+        (kernel_ms, total_ms, gpu_launches, h2d_bytes, d2h_bytes)."""
+        tri = _f32(triangles)
+        if tri.shape != self.tri.shape:
+            raise ValueError(f"triangles have shape {tri.shape}; this scene takes {self.tri.shape} (a rebuild keeps the triangles)")
+        st = B.Stats()
+        B.check(B.load_library().b200rt_scene_rebuild_bvh(self._h, B.fptr(tri), len(tri), C.byref(st)))
+        self.tri = tri.copy() if tri is triangles else tri
+        return st.as_dict()
+
+    def rebuild_bvh_device(self, dev_ptr: int, n: int, stream_ptr: int = 0) -> dict:
+        """rebuild_bvh from device memory of the scene's first device (b200rt_scene_rebuild_bvh_device), e.g. tensor.data_ptr() of
+        an (n, 9) float32 CUDA tensor, read in place and ordered after the work already queued on stream_ptr. self.tri is not
+        updated. Returns the stats."""
+        st = B.Stats()
+        B.check(B.load_library().b200rt_scene_rebuild_bvh_device(self._h, C.c_void_p(dev_ptr), n, C.c_void_p(stream_ptr), C.byref(st)))
+        return st.as_dict()
+
     def bvh_arrays(self, replica: int = 0) -> dict:
         """The resident BVH of one replica, downloaded (b200rt_scene_get_bvh_arrays): wide (WIDE_NODE_DTYPE records), axis and diag
         ((n_inner_nodes, 16) float32; diag is empty without diagonal slabs) and tris ((n_triangles, 12) float32)."""

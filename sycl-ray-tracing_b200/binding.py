@@ -74,6 +74,7 @@ EXPORTS = [
     "b200rt_untile_device", "b200rt_trace_primary_device", "b200rt_trace_rays_device", "b200rt_quantise_rgba8", "b200rt_quantise_rgba8_device", "b200rt_last_error", "b200rt_version",
     "b200rt_render_aovs", "b200rt_render_aovs_device", "b200rt_denoise_guided",
     "b200rt_scene_update_triangles", "b200rt_scene_update_triangles_device", "b200rt_scene_get_bvh_arrays",
+    "b200rt_scene_rebuild_bvh", "b200rt_scene_rebuild_bvh_device",
 ]
 
 _lib = None
@@ -135,6 +136,8 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
     L.b200rt_scene_set_materials.argtypes = [VP, FP, I]
     L.b200rt_scene_update_triangles.argtypes = [VP, FP, I, C.POINTER(Stats)]
     L.b200rt_scene_update_triangles_device.argtypes = [VP, VP, I, VP, C.POINTER(Stats)]
+    L.b200rt_scene_rebuild_bvh.argtypes = [VP, FP, I, C.POINTER(Stats)]
+    L.b200rt_scene_rebuild_bvh_device.argtypes = [VP, VP, I, VP, C.POINTER(Stats)]
     L.b200rt_scene_get_bvh_arrays.argtypes = [VP, I, VP, FP, FP, FP]
     L.b200rt_scene_build_env_alias.argtypes = [VP]
     L.b200rt_env_alias_table.argtypes = [FP, I, I, FP, C.POINTER(C.c_int), C.POINTER(C.c_double)]

@@ -561,27 +561,26 @@ double sah_cost_of(const FlatBVH& bvh)
     return sah;
 }
 
-// Hangs triangles that were kept out of the tree (the device builder's outsized ones) in front of both layouts' roots: the old
-// root record moves to the end of its array, record 0 becomes a top-level node whose one inner child is the old root (or the
-// next top-level node) and whose other children are leaves holding the extra triangles (8-ary: 7 leaves x 3 triangles per
-// node; binary: one leaf of up to 15 per record). The extra triangles go to the end of the triangle stream.
-void append_top_level(FlatBVH& b, const float* tri9, const std::vector<int>& ids, float abs_pad)
+// The top level over triangles kept out of the tree (the device builder's outsized ones), in front of both layouts' roots: the old root
+// record moves behind the existing records, record 0 becomes a top-level node whose one inner child is the old root (or the next
+// top-level node) and whose other children are leaves holding the extra triangles (8-ary: 7 leaves x 3 triangles per node; binary: one
+// leaf of up to 15 per record). Works from record 0 of each layout and the extra triangles' vertices alone, so a tree that lives on the
+// device needs only those few records on the host.
+void make_top_level(const WideNode& w0, const AxisNode& a0, size_t n_wide, size_t n_axis, size_t first_slot, const float* extra9, int n_extra,
+                    float abs_pad, TopLevel& out, b200rt_bvh_info& info)
 {
-    if (ids.empty() || b.wide.empty() || b.axis.empty()) return;
-    const int n_extra = (int)ids.size();
-    const size_t first_slot = b.tris.size();
+    out.wide.clear(); out.axis.clear();
+    if (n_extra <= 0) return;
     std::vector<Box> tbox((size_t)n_extra);
     for (int i = 0; i < n_extra; i++)
     {
-        b.tris.push_back(make_leaf_triangle(tri9, ids[i]));
-        const float* p = tri9 + 9 * (size_t)ids[i];
+        const float* p = extra9 + 9 * (size_t)i;
         tbox[i].grow(p); tbox[i].grow(p + 3); tbox[i].grow(p + 6);
         for (int a = 0; a < 3; a++) { const float pad = box_pad(tbox[i].lo[a], tbox[i].hi[a], abs_pad); tbox[i].lo[a] -= pad; tbox[i].hi[a] += pad; }
     }
     // ---- 8-ary layout
     {
         Box root;                                                   // the old root's extent: union of its decoded child boxes
-        const WideNode w0 = b.wide[0];
         const uint8_t* ql[3] = { w0.lox, w0.loy, w0.loz };
         const uint8_t* qh[3] = { w0.hix, w0.hiy, w0.hiz };
         for (int s = 0; s < 8; s++)
@@ -598,10 +597,10 @@ void append_top_level(FlatBVH& b, const float* tri9, const std::vector<int>& ids
             root.grow(lo); root.grow(hi);
         }
         const int per_node = 7 * kWideMaxLeaf;
-        const int n_top = (n_extra + per_node - 1) / per_node;
-        const size_t moved = b.wide.size();
-        b.wide.push_back(w0);
-        b.wide.resize(moved + (size_t)n_top);                      // top node k lives at index 0 (k = 0) or moved + k
+        const int n_top = top_level_wide(n_extra);
+        const size_t moved = n_wide;
+        out.wide.resize((size_t)n_top + 1);                         // [0]: record 0; [1 + j]: record moved + j (the old root, then top node j)
+        out.wide[1] = w0;
         std::vector<Box> below((size_t)n_top + 1);                 // extent of everything under top node k's inner child
         below[(size_t)n_top] = root;
         for (int k = n_top - 1; k >= 0; k--)
@@ -631,24 +630,22 @@ void append_top_level(FlatBVH& b, const float* tri9, const std::vector<int>& ids
                 w.valid24 |= ((1u << cnt) - 1u) << (3 * s);
             }
             for (int a = 0; a < 3; a++) quantise_slots(w, a, klo[a], khi[a], used, overflow);
-            b.wide[k == 0 ? 0 : moved + (size_t)k] = w;
+            out.wide[k == 0 ? 0 : 1 + (size_t)k] = w;
         }
         if (overflow) throw std::runtime_error("wide BVH quantisation overflow (top level)");
-        b.info.n_wide_nodes = (int)b.wide.size();
-        b.info.wide_max_depth += n_top;
+        info.n_wide_nodes = (int)(n_wide + (size_t)n_top);
+        info.wide_max_depth += n_top;
     }
     // ---- binary layout
     {
-        const AxisNode a0 = b.axis[0];
         Box root;
         root.grow(a0.l_lo); root.grow(a0.l_hi);
         if (a0.r_lo[0] <= a0.r_hi[0]) { root.grow(a0.r_lo); root.grow(a0.r_hi); }
         const int per_rec = 15;
-        const int n_top = (n_extra + per_rec - 1) / per_rec;
-        const size_t moved = b.axis.size();
-        b.axis.push_back(a0);
-        b.axis.resize(moved + (size_t)n_top);
-        if (!b.diag.empty()) { b.diag.push_back(b.diag[0]); b.diag.resize(b.axis.size()); }
+        const int n_top = top_level_axis(n_extra);
+        const size_t moved = n_axis;
+        out.axis.resize((size_t)n_top + 1);
+        out.axis[1] = a0;
         std::vector<Box> below((size_t)n_top + 1);
         below[(size_t)n_top] = root;
         for (int k = n_top - 1; k >= 0; k--)
@@ -669,12 +666,12 @@ void append_top_level(FlatBVH& b, const float* tri9, const std::vector<int>& ids
             }
             an.l_ref = (int)(k + 1 < n_top ? moved + (size_t)k + 1 : moved); an.l_count = 0;
             an.r_ref = leaf_ref((int)(first_slot + (size_t)i0), cnt); an.r_count = cnt;
-            b.axis[k == 0 ? 0 : moved + (size_t)k] = an;
+            out.axis[k == 0 ? 0 : 1 + (size_t)k] = an;
         }
-        b.info.n_inner_nodes = (int)b.axis.size();
-        b.info.n_leaves += n_top;
-        b.info.max_depth += n_top;
-        b.info.max_leaf_size = std::max(b.info.max_leaf_size, std::min(per_rec, n_extra));
+        info.n_inner_nodes = (int)(n_axis + (size_t)n_top);
+        info.n_leaves += n_top;
+        info.max_depth += n_top;
+        info.max_leaf_size = std::max(info.max_leaf_size, std::min(per_rec, n_extra));
     }
 }
 

@@ -5,8 +5,11 @@
 // (include/bounding_volume.h:9-127, plane normals source/bvh.cpp:8-16).
 #pragma once
 #include <cstdint>
+#include <functional>
 #include <string>
 #include <vector>
+
+#include <cuda_runtime.h>
 
 #include "../../include/b200rt.h"
 
@@ -78,9 +81,30 @@ inline float diag_dist(int k, float x, float y, float z)
 void build_flat_bvh(const float* tri9, int n_tri, const b200rt_bvh_options& opts, FlatBVH& out);
 int check_flat_bvh(const FlatBVH& bvh, const float* tri9, int n_tri);
 double sah_cost_of(const FlatBVH& bvh);
-// triangles kept out of the tree become leaf children of extra top-level nodes in front of both layouts' roots (bvh_build.cpp)
-void append_top_level(FlatBVH& bvh, const float* tri9, const std::vector<int>& ids, float abs_pad);
-// device builder (bvh_build_gpu.cu): 0 = ok, 1 = CUDA error, 2 = input outside what it handles (err says why)
+// Triangles kept out of the tree (the device builder's outsized ones) become leaf children of extra top-level nodes in front of both
+// layouts' roots (bvh_build.cpp). From record 0 of each layout (w0, a0), the existing record counts, the extra triangles' vertices
+// (extra9: 9 floats each; their stream slots start at first_slot) and the tree's abs_pad: out.wide[0] / out.axis[0] replace record 0,
+// out.wide[1 + j] / out.axis[1 + j] become records n_wide + j / n_axis + j (the old root first). info's counts and depths follow.
+struct TopLevel { std::vector<WideNode> wide; std::vector<AxisNode> axis; };
+inline int top_level_wide(int n_extra) { return (n_extra + 7 * kWideMaxLeaf - 1) / (7 * kWideMaxLeaf); }
+inline int top_level_axis(int n_extra) { return (n_extra + 14) / 15; }
+void make_top_level(const WideNode& w0, const AxisNode& a0, size_t n_wide, size_t n_axis, size_t first_slot, const float* extra9, int n_extra,
+                    float abs_pad, TopLevel& out, b200rt_bvh_info& info);
+
+// ---- device builder (bvh_build_gpu.cu): 0 = ok, 1 = CUDA error, 2 = input outside what it handles (err says why) ----------------------
+// Where a device build writes its tree: arrays the caller owns and allocates when the build asks, once the sizes are known (again
+// for a second attempt, which replaces the first one's). wide_and_tris: n_wide WideNodes (5 float4 each), then the n_tri-record
+// triangle stream (3 float4 each) in the same allocation; axis: n_axis binary records.
+struct DeviceTree { float4* wide_and_tris = nullptr; AxisNode* axis = nullptr; };
+using DeviceTreeAlloc = std::function<cudaError_t(size_t n_wide, size_t n_axis, DeviceTree& out)>;
+struct DeviceBuildCounts { int launches = 0; unsigned long long h2d_bytes = 0, d2h_bytes = 0; };   // library sorts and scans count as one launch each
+// Builds over d_tri9 (device memory of the current device) on stream st, into the caller's arrays; info gets everything but
+// build_seconds and sah_cost. Clustering first; an input it gives up on gets the Morton radix tree. Synchronises st.
+int build_bvh_device(const float* d_tri9, int n_tri, cudaStream_t st, const DeviceTreeAlloc& alloc, b200rt_bvh_info& info,
+                     DeviceBuildCounts& counts, std::string& err);
+// the same build from host vertices into a host FlatBVH: upload, build_bvh_device, download
 int build_flat_bvh_device(const float* tri9_host, int n_tri, int device, FlatBVH& out, std::string& err);
+// slot_of_prim[prim of stream record j] = j for the n_tri records of a triangle stream
+cudaError_t launch_slot_of_prim(const float4* tris, int n_tri, int* slot_of_prim, cudaStream_t st);
 
 } // namespace b200rt

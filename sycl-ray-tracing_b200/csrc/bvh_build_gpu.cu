@@ -16,11 +16,13 @@
 //   6. emit: quantised 80-byte wide nodes + the leaf-ordered triangle stream (lw_emit), binary two-children records (lb_emit)
 // Outsized triangles (box diagonal > 1/4 of the scene's: a ground quad under a mesh) would drag every ancestor box of their
 // Morton leaf out to the whole scene; up to 45 of them are kept out of the tree and hung, as leaf children, under one to
-// three extra top-level nodes in front of the tree's root (append_top_level, on the host after the download).
+// three extra top-level nodes in front of the tree's root (make_top_level: the host works them out from record 0 of each layout and
+// the outsized triangles' vertices, and writes them back).
+// The build reads vertices already on the device and writes into arrays its caller owns (build_bvh_device): a resident scene rebuilds
+// its tree in place with it, and b200rt_bvh_build_device is upload, build, download (build_flat_bvh_device).
 // Output is the same FlatBVH the host builder produces (b200rt_bvh_check validates either), except that it carries no
 // diagonal slabs (has_diag_slabs = 0: the 7-plane ablation needs the host builder).
 #include <algorithm>
-#include <cfloat>
 #include <cfloat>
 #include <chrono>
 #include <cstdint>
@@ -491,6 +493,22 @@ __global__ void lw_emit(DevArrays A, WideArrays W, int n_wide, float abs_pad, Wi
     nodes[w] = node;
 }
 
+// the outsized triangles behind the tree's stream records (emit_triangle, as every other record), and their vertices for the host's
+// top-level arithmetic
+__global__ void lw_emit_extra(const float* tri9, const int* ids, int n, float4* tris, float* extra9)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    emit_triangle(tri9, ids[i], tris + 3 * (size_t)i);
+    for (int k = 0; k < 9; k++) extra9[9 * i + k] = tri9[9 * (size_t)ids[i] + k];
+}
+
+__global__ void k_slot_of_prim(const float4* tris, int n, int* slot_of_prim)
+{
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j < n) slot_of_prim[__float_as_int(tris[3 * (size_t)j].w)] = j;
+}
+
 // ---- binary records over the same tree and the same triangle stream ---------------------------------------------------------------------
 __global__ void lb_mark_live(DevArrays A, int* live)
 {
@@ -600,7 +618,8 @@ struct TopBuilder
 struct Pool       // frees everything it handed out
 {
     std::vector<void*> p;
-    ~Pool() { for (void* q : p) cudaFree(q); }
+    ~Pool() { release(); }
+    void release() { for (void* q : p) cudaFree(q); p.clear(); }
     template <typename T> cudaError_t get(T** out, size_t n)
     {
         void* d = nullptr;
@@ -619,11 +638,17 @@ struct Pool       // frees everything it handed out
     } while (0)
 
 // 0 = ok; 1 = CUDA error; 2 = the input is outside what this builder handles
-static int build_flat_bvh_device_impl(const float* tri9_host, int n_tri, int device, bool use_lbvh, FlatBVH& out, std::string& err)
+static int build_bvh_device_impl(const float* d_tri9, int n_tri, cudaStream_t st, bool use_lbvh, const DeviceTreeAlloc& alloc,
+                                 b200rt_bvh_info& info, DeviceBuildCounts& C, std::string& err)
 {
-    const auto t0 = std::chrono::high_resolution_clock::now();
     if (n_tri <= kWideMaxLeaf) { err = "fewer than 4 triangles"; return 2; }
-    GCU(cudaSetDevice(device));
+    // host <-> device: every copy is counted; a download returns once the host holds it
+    auto h2d = [&](void* dst, const void* src, size_t bytes) { C.h2d_bytes += bytes; return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st); };
+    auto d2h = [&](void* dst, const void* src, size_t bytes) {
+        C.d2h_bytes += bytes;
+        const cudaError_t e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st);
+        return e != cudaSuccess ? e : cudaStreamSynchronize(st);
+    };
     Pool pool;
     DevArrays A;
     memset(&A, 0, sizeof(A));
@@ -632,9 +657,6 @@ static int build_flat_bvh_device_impl(const float* tri9_host, int n_tri, int dev
     static const int ploc_radius = []() { const char* e = getenv("B200RT_PLOC_RADIUS"); const int v = e ? atoi(e) : 16; return v < 1 ? 1 : (v > kPlocRadius ? kPlocRadius : v); }();
     A.leaf_max = leaf_env;
     const size_t n = (size_t)n_tri;
-    float* d_tri9 = nullptr;
-    GCU(pool.get(&d_tri9, 9 * n));
-    GCU(cudaMemcpy(d_tri9, tri9_host, 9 * n * sizeof(float), cudaMemcpyHostToDevice));
     A.tri9 = d_tri9;
     GCU(pool.get(&A.plo, n)); GCU(pool.get(&A.phi, n));
     GCU(pool.get(&A.keys, n)); GCU(pool.get(&A.keys_alt, n)); GCU(pool.get(&A.vals, n)); GCU(pool.get(&A.vals_alt, n));
@@ -644,21 +666,21 @@ static int build_flat_bvh_device_impl(const float* tri9_host, int n_tri, int dev
     GCU(pool.get(&A.scene, 16));
     int* d_misc = nullptr;                   // [0] max depth, [1] overflow flag
     GCU(pool.get(&d_misc, 4));
-    GCU(cudaMemset(d_misc, 0, 4 * sizeof(int)));
-    GCU(cudaMemset(A.visits, 0, n * sizeof(unsigned int)));
+    GCU(cudaMemsetAsync(d_misc, 0, 4 * sizeof(int), st));
+    GCU(cudaMemsetAsync(A.visits, 0, n * sizeof(unsigned int), st));
     {
         const int init[16] = { INT32_MAX, INT32_MAX, INT32_MAX, INT32_MIN, INT32_MIN, INT32_MIN, INT32_MIN, 0,
                                INT32_MAX, INT32_MAX, INT32_MAX, INT32_MIN, INT32_MIN, INT32_MIN, 0, 0 };
-        GCU(cudaMemcpy(A.scene, init, sizeof(init), cudaMemcpyHostToDevice));
+        GCU(h2d(A.scene, init, sizeof(init)));
     }
     const int tb = 256;
     int grid_n = (n_tri + tb - 1) / tb;
-    lb_bounds<<<grid_n, tb>>>(A);
+    lb_bounds<<<grid_n, tb, 0, st>>>(A); C.launches++;
     size_t sort_bytes = 0;
     {
         cub::DoubleBuffer<unsigned long long> dk(A.keys, A.keys_alt);
         cub::DoubleBuffer<int> dv(A.vals, A.vals_alt);
-        GCU(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, dk, dv, n_tri, 0, 64));
+        GCU(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, dk, dv, n_tri, 0, 64, st));
     }
     char* sort_tmp = nullptr;
     GCU(pool.get(&sort_tmp, sort_bytes));
@@ -668,25 +690,26 @@ static int build_flat_bvh_device_impl(const float* tri9_host, int n_tri, int dev
         // first with the outsized triangles given the largest key (they sort to the end and stay out of the tree); if there are
         // too many of them for a few top-level nodes, or too few others for a tree, once more with everything in the tree
         A.segregate = attempt == 0 ? 1 : 0;
-        lb_morton<<<grid_n, tb>>>(A);
+        lb_morton<<<grid_n, tb, 0, st>>>(A); C.launches++;
         cub::DoubleBuffer<unsigned long long> dk(A.keys, A.keys_alt);
         cub::DoubleBuffer<int> dv(A.vals, A.vals_alt);
-        GCU(cub::DeviceRadixSort::SortPairs(sort_tmp, sort_bytes, dk, dv, n_tri, 0, 64));
+        GCU(cub::DeviceRadixSort::SortPairs(sort_tmp, sort_bytes, dk, dv, n_tri, 0, 64, st)); C.launches++;
         A.keys = dk.Current(); A.keys_alt = dk.Alternate(); A.vals = dv.Current(); A.vals_alt = dv.Alternate();
         n_large = 0;
-        if (attempt == 0) GCU(cudaMemcpy(&n_large, A.scene + 14, sizeof(int), cudaMemcpyDeviceToHost));
+        if (attempt == 0) GCU(d2h(&n_large, A.scene + 14, sizeof(int)));
         if (n_large <= 45 && n_tri - n_large > kWideMaxLeaf) break;
     }
     std::vector<int> large_ids((size_t)n_large);
-    if (n_large) GCU(cudaMemcpy(large_ids.data(), A.vals + (n_tri - n_large), (size_t)n_large * sizeof(int), cudaMemcpyDeviceToHost));
+    if (n_large) GCU(d2h(large_ids.data(), A.vals + (n_tri - n_large), (size_t)n_large * sizeof(int)));
     const int n_all = n_tri;
     n_tri -= n_large;                         // the tree is built over the first n_tri sorted triangles
     A.n = n_tri;
     grid_n = (n_tri + tb - 1) / tb;
     if (use_lbvh)
     {
-        lb_tree<<<grid_n, tb>>>(A);
-        lb_fit<<<grid_n, tb>>>(A, d_misc);
+        lb_tree<<<grid_n, tb, 0, st>>>(A);
+        lb_fit<<<grid_n, tb, 0, st>>>(A, d_misc);
+        C.launches += 2;
     }
     else
     {
@@ -695,26 +718,27 @@ static int build_flat_bvh_device_impl(const float* tri9_host, int n_tri, int dev
         for (int b = 0; b < 2; b++) { GCU(pool.get(&P.cid[b], n)); GCU(pool.get(&P.clo[b], n)); GCU(pool.get(&P.chi[b], n)); }
         GCU(pool.get(&P.nn, n)); GCU(pool.get(&P.valid, n)); GCU(pool.get(&P.pos, n)); GCU(pool.get(&P.size, n)); GCU(pool.get(&P.next_node, 1));
         size_t pscan_bytes = 0;
-        GCU(cub::DeviceScan::ExclusiveSum(nullptr, pscan_bytes, P.valid, P.pos, n_tri));
+        GCU(cub::DeviceScan::ExclusiveSum(nullptr, pscan_bytes, P.valid, P.pos, n_tri, st));
         char* pscan_tmp = nullptr;
         GCU(pool.get(&pscan_tmp, pscan_bytes));
         const int first_node = n_tri - 2;
-        GCU(cudaMemcpy(P.next_node, &first_node, sizeof(int), cudaMemcpyHostToDevice));
-        pl_init<<<grid_n, tb>>>(A, P);
+        GCU(h2d(P.next_node, &first_node, sizeof(int)));
+        pl_init<<<grid_n, tb, 0, st>>>(A, P); C.launches++;
         static const int top_clusters = []() { const char* e = getenv("B200RT_PLOC_TOP"); const int v = e ? atoi(e) : 1024; return v < 1 ? 1 : v; }();
         int nc = n_tri, cur = 0, rounds = 0;
         while (nc > top_clusters)
         {
             if (++rounds > 512) { err = "clustering needs more than 512 rounds (a size gradient along the Morton curve merges one pair per round)"; return 2; }
             const int g = (nc + kPlocBlock - 1) / kPlocBlock;
-            pl_nearest<<<g, kPlocBlock>>>(P.clo[cur], P.chi[cur], nc, ploc_radius, P.nn);
-            pl_merge<<<g, kPlocBlock>>>(A, P, cur, nc);
-            GCU(cub::DeviceScan::ExclusiveSum(pscan_tmp, pscan_bytes, P.valid, P.pos, nc));
-            pl_compact<<<g, kPlocBlock>>>(P, cur, nc);
-            int last_pos = 0, last_valid = 0;
-            GCU(cudaMemcpy(&last_pos, P.pos + nc - 1, sizeof(int), cudaMemcpyDeviceToHost));
-            GCU(cudaMemcpy(&last_valid, P.valid + nc - 1, sizeof(int), cudaMemcpyDeviceToHost));
-            const int next = last_pos + last_valid;
+            pl_nearest<<<g, kPlocBlock, 0, st>>>(P.clo[cur], P.chi[cur], nc, ploc_radius, P.nn);
+            pl_merge<<<g, kPlocBlock, 0, st>>>(A, P, cur, nc);
+            GCU(cub::DeviceScan::ExclusiveSum(pscan_tmp, pscan_bytes, P.valid, P.pos, nc, st));
+            pl_compact<<<g, kPlocBlock, 0, st>>>(P, cur, nc);
+            C.launches += 4;
+            int last[2] = { 0, 0 };
+            GCU(d2h(&last[0], P.pos + nc - 1, sizeof(int)));
+            GCU(d2h(&last[1], P.valid + nc - 1, sizeof(int)));
+            const int next = last[0] + last[1];
             if (next >= nc) { err = "clustering round merged nothing"; return 1; }
             nc = next; cur ^= 1;
         }
@@ -724,11 +748,11 @@ static int build_flat_bvh_device_impl(const float* tri9_host, int n_tri, int dev
             std::vector<int> h_cid((size_t)nc);
             std::vector<float4> h_lo((size_t)nc), h_hi((size_t)nc);
             std::vector<int> h_size((size_t)nc);
-            pl_cluster_sizes<<<(nc + 255) / 256, 256>>>(P.cid[cur], P.size, nc, P.nn);
-            GCU(cudaMemcpy(h_size.data(), P.nn, (size_t)nc * sizeof(int), cudaMemcpyDeviceToHost));
-            GCU(cudaMemcpy(h_cid.data(), P.cid[cur], (size_t)nc * sizeof(int), cudaMemcpyDeviceToHost));
-            GCU(cudaMemcpy(h_lo.data(), P.clo[cur], (size_t)nc * sizeof(float4), cudaMemcpyDeviceToHost));
-            GCU(cudaMemcpy(h_hi.data(), P.chi[cur], (size_t)nc * sizeof(float4), cudaMemcpyDeviceToHost));
+            pl_cluster_sizes<<<(nc + 255) / 256, 256, 0, st>>>(P.cid[cur], P.size, nc, P.nn); C.launches++;
+            GCU(d2h(h_size.data(), P.nn, (size_t)nc * sizeof(int)));
+            GCU(d2h(h_cid.data(), P.cid[cur], (size_t)nc * sizeof(int)));
+            GCU(d2h(h_lo.data(), P.clo[cur], (size_t)nc * sizeof(float4)));
+            GCU(d2h(h_hi.data(), P.chi[cur], (size_t)nc * sizeof(float4)));
             TopBuilder T;
             T.c.resize((size_t)nc);
             for (int i = 0; i < nc; i++)
@@ -743,17 +767,18 @@ static int build_flat_bvh_device_impl(const float* tri9_host, int n_tri, int dev
             T.left.resize(nt); T.right.resize(nt); T.size.resize(nt); T.nlo.resize(nt); T.nhi.resize(nt);
             const int root = T.build(0, nc);
             if (root != 0 || T.next != nc - 1) { err = "top-level build produced an inconsistent tree"; return 1; }
-            GCU(cudaMemcpy(A.left, T.left.data(), nt * sizeof(int), cudaMemcpyHostToDevice));
-            GCU(cudaMemcpy(A.right, T.right.data(), nt * sizeof(int), cudaMemcpyHostToDevice));
-            GCU(cudaMemcpy(P.size, T.size.data(), nt * sizeof(int), cudaMemcpyHostToDevice));
-            GCU(cudaMemcpy(A.nlo, T.nlo.data(), nt * sizeof(float4), cudaMemcpyHostToDevice));
-            GCU(cudaMemcpy(A.nhi, T.nhi.data(), nt * sizeof(float4), cudaMemcpyHostToDevice));
+            GCU(h2d(A.left, T.left.data(), nt * sizeof(int)));
+            GCU(h2d(A.right, T.right.data(), nt * sizeof(int)));
+            GCU(h2d(P.size, T.size.data(), nt * sizeof(int)));
+            GCU(h2d(A.nlo, T.nlo.data(), nt * sizeof(float4)));
+            GCU(h2d(A.nhi, T.nhi.data(), nt * sizeof(float4)));
+            GCU(cudaStreamSynchronize(st));          // T's vectors are the sources of the copies above
         }
         // the root is the node created last: index 0
         {
             const int none = -1, zero = 0;
-            GCU(cudaMemcpy(A.parent_node, &none, sizeof(int), cudaMemcpyHostToDevice));
-            GCU(cudaMemcpy(A.first, &zero, sizeof(int), cudaMemcpyHostToDevice));
+            GCU(h2d(A.parent_node, &none, sizeof(int)));
+            GCU(h2d(A.first, &zero, sizeof(int)));
         }
         // depth-first layout level by level (the clustering arrays are free again: frontiers, the leaf permutation, the relabelled nodes)
         int* front[2] = { P.cid[0], P.cid[1] };
@@ -762,31 +787,31 @@ static int build_flat_bvh_device_impl(const float* tri9_host, int n_tri, int dev
         int* pre = reinterpret_cast<int*>(A.visits);
         {
             const int zero = 0;
-            GCU(cudaMemcpy(front[0], &zero, sizeof(int), cudaMemcpyHostToDevice));
-            GCU(cudaMemcpy(pre, &zero, sizeof(int), cudaMemcpyHostToDevice));
+            GCU(h2d(front[0], &zero, sizeof(int)));
+            GCU(h2d(pre, &zero, sizeof(int)));
         }
         int n_front = 1, f = 0, depth = 1;
         while (n_front > 0)
         {
             depth++;
             if (depth > 4096) { err = "layout did not terminate"; return 1; }
-            GCU(cudaMemset(d_nnext, 0, sizeof(int)));
-            pl_layout<<<(n_front + 255) / 256, 256>>>(A, P, front[f], n_front, front[f ^ 1], d_nnext, newpos, pre);
-            GCU(cudaMemcpy(&n_front, d_nnext, sizeof(int), cudaMemcpyDeviceToHost));
+            GCU(cudaMemsetAsync(d_nnext, 0, sizeof(int), st));
+            pl_layout<<<(n_front + 255) / 256, 256, 0, st>>>(A, P, front[f], n_front, front[f ^ 1], d_nnext, newpos, pre); C.launches++;
+            GCU(d2h(&n_front, d_nnext, sizeof(int)));
             f ^= 1;
         }
-        GCU(cudaMemcpy(d_misc, &depth, sizeof(int), cudaMemcpyHostToDevice));
-        pl_permute_vals<<<grid_n, tb>>>(A.vals, newpos, n_tri, A.vals_alt);
+        GCU(h2d(d_misc, &depth, sizeof(int)));
+        pl_permute_vals<<<grid_n, tb, 0, st>>>(A.vals, newpos, n_tri, A.vals_alt); C.launches++;
         // the outsized triangles behind the tree keep their places in the order
-        if (n_large) GCU(cudaMemcpy(A.vals_alt + n_tri, A.vals + n_tri, (size_t)n_large * sizeof(int), cudaMemcpyDeviceToDevice));
-        pl_relabel_nodes<<<grid_n, tb>>>(A, pre, newpos, A.parent_node, A.parent_leaf, P.pos, P.valid, P.clo[0], P.chi[0]);
+        if (n_large) GCU(cudaMemcpyAsync(A.vals_alt + n_tri, A.vals + n_tri, (size_t)n_large * sizeof(int), cudaMemcpyDeviceToDevice, st));
+        pl_relabel_nodes<<<grid_n, tb, 0, st>>>(A, pre, newpos, A.parent_node, A.parent_leaf, P.pos, P.valid, P.clo[0], P.chi[0]); C.launches++;
         std::swap(A.vals, A.vals_alt);
         A.left = A.parent_node; A.right = A.parent_leaf; A.first = P.pos; A.last = P.valid; A.nlo = P.clo[0]; A.nhi = P.chi[0];
     }
     int scene_h[8];
     int misc_h[4];
-    GCU(cudaMemcpy(scene_h, A.scene, sizeof(scene_h), cudaMemcpyDeviceToHost));
-    GCU(cudaMemcpy(misc_h, d_misc, sizeof(misc_h), cudaMemcpyDeviceToHost));
+    GCU(d2h(scene_h, A.scene, sizeof(scene_h)));
+    GCU(d2h(misc_h, d_misc, sizeof(misc_h)));
     if (misc_h[0] > kMaxTraversalDepth) { err = "radix tree deeper than the traversal stack (" + std::to_string(misc_h[0]) + ")"; return 2; }
     float scene_abs = ord2f(scene_h[6]);
     if (!(scene_abs < FLT_MAX)) scene_abs = 1.0f;
@@ -799,89 +824,145 @@ static int build_flat_bvh_device_impl(const float* tri9_host, int n_tri, int dev
     GCU(pool.get(&W.root, n)); GCU(pool.get(&W.slots, 8 * n)); GCU(pool.get(&W.n_inner, n)); GCU(pool.get(&W.n_tris, n));
     GCU(pool.get(&W.child_base, n)); GCU(pool.get(&W.tri_base, n)); GCU(pool.get(&W.node_first, n)); GCU(pool.get(&W.leaf_first, n));
     size_t scan_bytes = 0;
-    GCU(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, W.n_inner, W.child_base, n_tri));
+    GCU(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, W.n_inner, W.child_base, n_tri, st));
     char* scan_tmp = nullptr;
     GCU(pool.get(&scan_tmp, scan_bytes));
     {
         const int zero = 0;
-        GCU(cudaMemcpy(W.root, &zero, sizeof(int), cudaMemcpyHostToDevice));
+        GCU(h2d(W.root, &zero, sizeof(int)));
     }
     int begin = 0, end = 1, wide_depth = 0;
     while (begin < end)
     {
         wide_depth++;
         const int cnt = end - begin, g = (cnt + 127) / 128;
-        lw_expand<<<g, 128>>>(A, W, begin, end);
-        GCU(cub::DeviceScan::ExclusiveSum(scan_tmp, scan_bytes, W.n_inner + begin, W.child_base + begin, cnt));
-        int last_base = 0, last_cnt = 0;
-        GCU(cudaMemcpy(&last_base, W.child_base + end - 1, sizeof(int), cudaMemcpyDeviceToHost));
-        GCU(cudaMemcpy(&last_cnt, W.n_inner + end - 1, sizeof(int), cudaMemcpyDeviceToHost));
-        const int next_cnt = last_base + last_cnt;
+        lw_expand<<<g, 128, 0, st>>>(A, W, begin, end);
+        GCU(cub::DeviceScan::ExclusiveSum(scan_tmp, scan_bytes, W.n_inner + begin, W.child_base + begin, cnt, st));
+        C.launches += 2;
+        int last[2] = { 0, 0 };
+        GCU(d2h(&last[0], W.child_base + end - 1, sizeof(int)));
+        GCU(d2h(&last[1], W.n_inner + end - 1, sizeof(int)));
+        const int next_cnt = last[0] + last[1];
         if (wide_depth > kMaxTraversalDepth) { err = "wide tree deeper than the traversal stack"; return 2; }
         if ((size_t)end + next_cnt > n) { err = "wide node count exceeds its bound"; return 1; }
-        lw_shift<<<g, 128>>>(W.child_base + begin, cnt, end);      // the scan is relative to the level's first child, which gets index `end`
-        lw_link<<<g, 128>>>(A, W, begin, end);
+        lw_shift<<<g, 128, 0, st>>>(W.child_base + begin, cnt, end);      // the scan is relative to the level's first child, which gets index `end`
+        lw_link<<<g, 128, 0, st>>>(A, W, begin, end);
+        C.launches += 2;
         begin = end; end += next_cnt;
     }
     const int n_wide = end;
-    GCU(cub::DeviceScan::ExclusiveSum(scan_tmp, scan_bytes, W.n_tris, W.tri_base, n_wide));
-    WideNode* d_wide = nullptr; float4* d_tris = nullptr;
-    GCU(pool.get(&d_wide, (size_t)n_wide)); GCU(pool.get(&d_tris, 3 * n));
-    lw_emit<<<(n_wide + 127) / 128, 128>>>(A, W, n_wide, abs_pad, d_wide, d_tris, d_misc + 1);
+    GCU(cub::DeviceScan::ExclusiveSum(scan_tmp, scan_bytes, W.n_tris, W.tri_base, n_wide, st));
 
-    // binary records
+    // binary records: which radix-tree nodes stay inner records, and their record indices
     int *d_live = nullptr, *d_axis_idx = nullptr;
     GCU(pool.get(&d_live, n)); GCU(pool.get(&d_axis_idx, n));
-    lb_mark_live<<<grid_n, tb>>>(A, d_live);
-    GCU(cub::DeviceScan::ExclusiveSum(scan_tmp, scan_bytes, d_live, d_axis_idx, n_tri - 1));
-    int n_axis = 0, last_live = 0;
-    GCU(cudaMemcpy(&n_axis, d_axis_idx + (n_tri - 2), sizeof(int), cudaMemcpyDeviceToHost));
-    GCU(cudaMemcpy(&last_live, d_live + (n_tri - 2), sizeof(int), cudaMemcpyDeviceToHost));
-    n_axis += last_live;
-    AxisNode* d_axis = nullptr;
-    GCU(pool.get(&d_axis, (size_t)std::max(n_axis, 1)));
-    lb_emit<<<grid_n, tb>>>(A, W, d_live, d_axis_idx, abs_pad, d_axis);
-    GCU(cudaMemcpy(misc_h, d_misc, sizeof(misc_h), cudaMemcpyDeviceToHost));
+    lb_mark_live<<<grid_n, tb, 0, st>>>(A, d_live);
+    GCU(cub::DeviceScan::ExclusiveSum(scan_tmp, scan_bytes, d_live, d_axis_idx, n_tri - 1, st));
+    C.launches += 3;
+    int last_axis[2] = { 0, 0 };
+    GCU(d2h(&last_axis[0], d_axis_idx + (n_tri - 2), sizeof(int)));
+    GCU(d2h(&last_axis[1], d_live + (n_tri - 2), sizeof(int)));
+    const int n_axis = last_axis[0] + last_axis[1];
+
+    // the caller's arrays, with room for the top level over the outsized triangles
+    const int n_top_wide = n_large ? top_level_wide(n_large) : 0, n_top_axis = n_large ? top_level_axis(n_large) : 0;
+    DeviceTree out;
+    GCU(alloc((size_t)n_wide + n_top_wide, (size_t)n_axis + n_top_axis, out));
+    WideNode* d_wide = reinterpret_cast<WideNode*>(out.wide_and_tris);
+    float4* d_tris = out.wide_and_tris + 5 * ((size_t)n_wide + n_top_wide);
+    lw_emit<<<(n_wide + 127) / 128, 128, 0, st>>>(A, W, n_wide, abs_pad, d_wide, d_tris, d_misc + 1);
+    lb_emit<<<grid_n, tb, 0, st>>>(A, W, d_live, d_axis_idx, abs_pad, out.axis);
+    C.launches += 2;
+    GCU(d2h(misc_h, d_misc, sizeof(misc_h)));
     GCU(cudaGetLastError());
     if (misc_h[1]) { err = "wide BVH quantisation overflow"; return 1; }
 
-    // room for the top level append_top_level may add: growing these vectors afterwards would copy gigabytes at 20 M triangles
-    out.wide.clear(); out.tris.clear(); out.axis.clear(); out.diag.clear();
-    out.wide.reserve((size_t)n_wide + 8); out.tris.reserve((size_t)n_all); out.axis.reserve((size_t)n_axis + 8);
-    out.wide.resize((size_t)n_wide); out.tris.resize((size_t)n_tri); out.axis.resize((size_t)n_axis);
-    GCU(cudaMemcpy(out.wide.data(), d_wide, (size_t)n_wide * sizeof(WideNode), cudaMemcpyDeviceToHost));
-    GCU(cudaMemcpy(out.tris.data(), d_tris, (size_t)n_tri * sizeof(LeafTriangle), cudaMemcpyDeviceToHost));
-    GCU(cudaMemcpy(out.axis.data(), d_axis, (size_t)n_axis * sizeof(AxisNode), cudaMemcpyDeviceToHost));
-    memset(&out.info, 0, sizeof(out.info));
-    out.info.n_triangles = n_all;
-    out.info.n_inner_nodes = n_axis;
-    out.info.n_leaves = n_axis + 1;
-    out.info.max_leaf_size = kWideMaxLeaf;
-    out.info.max_depth = misc_h[0];
-    out.info.has_diag_slabs = 0;
-    out.info.sah_cost = 0.0;
-    out.info.n_wide_nodes = n_wide;
-    out.info.wide_max_depth = wide_depth;
+    memset(&info, 0, sizeof(info));
+    info.n_triangles = n_all;
+    info.n_inner_nodes = n_axis;
+    info.n_leaves = n_axis + 1;
+    info.max_leaf_size = kWideMaxLeaf;
+    info.max_depth = misc_h[0];
+    info.has_diag_slabs = 0;
+    info.sah_cost = 0.0;
+    info.n_wide_nodes = n_wide;
+    info.wide_max_depth = wide_depth;
     if (n_large)
     {
+        // the outsized triangles' stream records on the device; record 0 of both layouts and their vertices to the host, which works
+        // out the few top-level records; those records back
         std::sort(large_ids.begin(), large_ids.end());
-        try { append_top_level(out, tri9_host, large_ids, abs_pad); }
+        int* d_ids = nullptr; float* d_extra9 = nullptr;
+        GCU(pool.get(&d_ids, (size_t)n_large)); GCU(pool.get(&d_extra9, 9 * (size_t)n_large));
+        GCU(h2d(d_ids, large_ids.data(), (size_t)n_large * sizeof(int)));
+        lw_emit_extra<<<1, 64, 0, st>>>(d_tri9, d_ids, n_large, d_tris + 3 * (size_t)n_tri, d_extra9); C.launches++;
+        std::vector<float> extra9(9 * (size_t)n_large);
+        WideNode w0; AxisNode a0;
+        GCU(d2h(extra9.data(), d_extra9, extra9.size() * sizeof(float)));
+        GCU(d2h(&w0, d_wide, sizeof(w0)));
+        GCU(d2h(&a0, out.axis, sizeof(a0)));
+        TopLevel top;
+        try { make_top_level(w0, a0, (size_t)n_wide, (size_t)n_axis, (size_t)n_tri, extra9.data(), n_large, abs_pad, top, info); }
         catch (const std::exception& e) { err = e.what(); return 1; }
-        if (out.info.max_depth > kMaxTraversalDepth || out.info.wide_max_depth > kMaxTraversalDepth) { err = "tree deeper than the traversal stack"; return 2; }
+        GCU(h2d(d_wide, top.wide.data(), sizeof(WideNode)));
+        GCU(h2d(d_wide + n_wide, top.wide.data() + 1, (top.wide.size() - 1) * sizeof(WideNode)));
+        GCU(h2d(out.axis, top.axis.data(), sizeof(AxisNode)));
+        GCU(h2d(out.axis + n_axis, top.axis.data() + 1, (top.axis.size() - 1) * sizeof(AxisNode)));
+        GCU(cudaStreamSynchronize(st));              // top's vectors are the sources of the copies above
+        if (info.max_depth > kMaxTraversalDepth || info.wide_max_depth > kMaxTraversalDepth) { err = "tree deeper than the traversal stack"; return 2; }
     }
+    GCU(cudaStreamSynchronize(st));
+    return 0;
+}
+
+int build_bvh_device(const float* d_tri9, int n_tri, cudaStream_t st, const DeviceTreeAlloc& alloc, b200rt_bvh_info& info,
+                     DeviceBuildCounts& counts, std::string& err)
+{
+    static const bool lbvh_only = []() { const char* e = getenv("B200RT_DEVICE_BUILDER"); return e && std::string(e) == "lbvh"; }();
+    int rc = 2;
+    if (!lbvh_only) rc = build_bvh_device_impl(d_tri9, n_tri, st, false, alloc, info, counts, err);
+    if (rc == 2) rc = build_bvh_device_impl(d_tri9, n_tri, st, true, alloc, info, counts, err);
+    return rc;
+}
+
+// 0 = ok; 1 = CUDA error; 2 = the input is outside what this builder handles (caller falls back to the host builder).
+int build_flat_bvh_device(const float* tri9_host, int n_tri, int device, FlatBVH& out, std::string& err)
+{
+    const auto t0 = std::chrono::high_resolution_clock::now();
+    if (n_tri <= kWideMaxLeaf) { err = "fewer than 4 triangles"; return 2; }
+    GCU(cudaSetDevice(device));
+    Pool in;
+    float* d_tri9 = nullptr;
+    GCU(in.get(&d_tri9, 9 * (size_t)n_tri));
+    GCU(cudaMemcpy(d_tri9, tri9_host, 9 * (size_t)n_tri * sizeof(float), cudaMemcpyHostToDevice));
+    Pool tree;
+    size_t n_wide = 0, n_axis = 0;
+    DeviceTree dt;
+    const DeviceTreeAlloc alloc = [&](size_t nw, size_t na, DeviceTree& o) {
+        tree.release();
+        n_wide = nw; n_axis = na;
+        cudaError_t e = tree.get(&o.wide_and_tris, 5 * nw + 3 * (size_t)n_tri);
+        if (e == cudaSuccess) e = tree.get(&o.axis, na);
+        dt = o;
+        return e;
+    };
+    DeviceBuildCounts counts;
+    b200rt_bvh_info info;
+    const int rc = build_bvh_device(d_tri9, n_tri, 0, alloc, info, counts, err);
+    if (rc) return rc;
+    out.wide.resize(n_wide); out.tris.resize((size_t)n_tri); out.axis.resize(n_axis); out.diag.clear();
+    GCU(cudaMemcpy(out.wide.data(), dt.wide_and_tris, n_wide * sizeof(WideNode), cudaMemcpyDeviceToHost));
+    GCU(cudaMemcpy(out.tris.data(), dt.wide_and_tris + 5 * n_wide, (size_t)n_tri * sizeof(LeafTriangle), cudaMemcpyDeviceToHost));
+    GCU(cudaMemcpy(out.axis.data(), dt.axis, n_axis * sizeof(AxisNode), cudaMemcpyDeviceToHost));
+    out.info = info;
     out.info.build_seconds = std::chrono::duration<double>(std::chrono::high_resolution_clock::now() - t0).count();
     return 0;
 }
 
-// 0 = ok; 1 = CUDA error; 2 = the input is outside what this builder handles (caller falls back to the host builder).
-// Clustering first; an input it gives up on (too many rounds, a tree deeper than the traversal stack) gets the Morton radix tree.
-int build_flat_bvh_device(const float* tri9_host, int n_tri, int device, FlatBVH& out, std::string& err)
+cudaError_t launch_slot_of_prim(const float4* tris, int n_tri, int* slot_of_prim, cudaStream_t st)
 {
-    static const bool lbvh_only = []() { const char* e = getenv("B200RT_DEVICE_BUILDER"); return e && std::string(e) == "lbvh"; }();
-    int rc = 2;
-    if (!lbvh_only) rc = build_flat_bvh_device_impl(tri9_host, n_tri, device, false, out, err);
-    if (rc == 2) rc = build_flat_bvh_device_impl(tri9_host, n_tri, device, true, out, err);
-    return rc;
+    if (n_tri > 0) k_slot_of_prim<<<(n_tri + 255) / 256, 256, 0, st>>>(tris, n_tri, slot_of_prim);
+    return cudaGetLastError();
 }
 
 } // namespace b200rt

@@ -58,12 +58,35 @@ struct DevArray
     }
 };
 
+// The BVH of one replica: the 8-ary nodes with the triangle stream right behind them (one allocation, DESIGN.md §2), the binary and
+// diagonal records, and slot_of_prim. A rebuild makes a new one beside the old one and swaps it in.
+struct SceneTree
+{
+    enum { kWideTris, kAxis, kDiag, kSlot, kArrays };
+    DevPtr mem[kArrays];
+    size_t bytes[kArrays] = {};
+    size_t n_wide4 = 0;                   // float4s of 8-ary nodes in front of the triangle stream
+    // array k of n elements of elem_bytes (at least one element, as every scene upload), on the current device
+    cudaError_t alloc(int k, size_t n, size_t elem_bytes)
+    {
+        mem[k].reset(); bytes[k] = 0;
+        void* p = nullptr;
+        const size_t b = std::max<size_t>(n, 1) * elem_bytes;
+        const cudaError_t e = cudaMalloc(&p, b);
+        if (e == cudaSuccess) { mem[k].reset(p); bytes[k] = b; }
+        return e;
+    }
+    template <typename T> T* get(int k) const { return static_cast<T*>(mem[k].get()); }
+    size_t total() const { size_t t = 0; for (size_t b : bytes) t += b; return t; }
+};
+
 struct b200rt_scene
 {
     int device = 0;
     SceneDev dev{};
     b200rt_bvh_info info{};
-    size_t bytes = 0;
+    size_t bytes = 0;                     // every device array below that the scene keeps, the tree included
+    SceneTree tree;
     std::vector<DevPtr> allocs;           // the scene's uploads and tables, counted in `bytes`
     DevArray<MaterialDev> d_mats;
     std::vector<char> mat_used;           // material slots some primitive references (slot 0 of parse_obj is emissive but normally unused)
@@ -95,11 +118,12 @@ struct b200rt_scene
     // pinned staging for copies from / to pageable caller memory: two chunks, ping-pong
     PinnedPtr h_stage[2]; cudaEvent_t stage_ev[2] = { nullptr, nullptr };
     // geometry updates (b200rt_scene_update_triangles): both layouts' level lists and per-node exact boxes, made on the first update,
-    // kept and counted in `bytes`; the new vertices when they have to be staged on this device
+    // kept and counted in `bytes`, sized for the tree they were made for (a rebuild releases them); the new vertices when they have to
+    // be staged on this device
     bool refit_ready = false;
     std::vector<int> wide_level, axis_level;
-    int *d_wide_idx = nullptr, *d_axis_idx = nullptr;
-    float4 *d_wide_box = nullptr, *d_axis_box = nullptr;
+    DevArray<int> d_wide_idx, d_axis_idx;
+    DevArray<float4> d_wide_box, d_axis_box;
     unsigned int* d_refit_misc = nullptr;     // [0] max |coord| bits, [1] non-finite flag, [2] quantisation overflow, [3] walk counter
     double* d_sah = nullptr;
     DevArray<float> d_vertices;
@@ -695,20 +719,12 @@ int validate_scene_args(const SceneArgs& a)
 // host-side products shared by every device replica of a scene (computed once)
 struct SceneHostData
 {
-    std::vector<float4> bvh_and_tris; size_t n_wide4 = 0;
     std::vector<unsigned char> oct_lut;
-    std::vector<int> slot_of_prim;
     std::vector<SphereDev> spheres;
 };
 
-void prepare_host_data(const SceneArgs& a, const FlatBVH& f, SceneHostData& h)
+void prepare_host_data(const SceneArgs& a, SceneHostData& h)
 {
-    // the 8-ary nodes and the triangle stream share one allocation (DESIGN.md §2): the triangles sit right behind the nodes
-    const size_t nw = f.wide.size() * 5, nt = f.tris.size() * 3;
-    h.bvh_and_tris.resize(std::max<size_t>(nw + nt, 1));
-    if (nw) std::memcpy(h.bvh_and_tris.data(), f.wide.data(), nw * sizeof(float4));
-    if (nt) std::memcpy(h.bvh_and_tris.data() + nw, f.tris.data(), nt * sizeof(float4));
-    h.n_wide4 = nw;
     h.oct_lut.resize(8 * 256);
     for (int o = 0; o < 8; o++)
         for (int m = 0; m < 256; m++)
@@ -717,10 +733,52 @@ void prepare_host_data(const SceneArgs& a, const FlatBVH& f, SceneHostData& h)
             for (int b = 0; b < 8; b++) if (m & (1 << b)) r |= 1u << (b ^ o);
             h.oct_lut[(size_t)o * 256 + m] = (unsigned char)r;
         }
-    h.slot_of_prim.assign((size_t)std::max(a.n_tri, 1), 0);
-    for (size_t i = 0; i < f.tris.size(); i++) h.slot_of_prim[f.tris[i].prim] = (int)i;
     h.spheres.resize((size_t)std::max(a.n_spheres, 1));
     for (int i = 0; i < a.n_spheres; i++) std::memcpy(&h.spheres[i], (const char*)a.spheres20 + 20 * (size_t)i, 20);
+}
+
+// the release of a replica's refit state: its per-node arrays are sized for the tree they were made for
+void release_refit(b200rt_scene* r)
+{
+    r->bytes -= (r->d_wide_idx.cap + r->d_axis_idx.cap) * sizeof(int) + (r->d_wide_box.cap + r->d_axis_box.cap) * sizeof(float4);
+    r->d_wide_idx = {}; r->d_axis_idx = {}; r->d_wide_box = {}; r->d_axis_box = {};
+    r->refit_ready = false;
+}
+
+// A host-built tree on the current device, as a replica's tree, copied on stream st (slot_of_prim computed there)
+int tree_from_host(const FlatBVH& f, int n_tri, cudaStream_t st, SceneTree& t)
+{
+    const size_t nw = f.wide.size() * 5, nt = f.tris.size() * 3;
+    CU(t.alloc(SceneTree::kWideTris, nw + nt, sizeof(float4)));
+    CU(t.alloc(SceneTree::kAxis, f.axis.size(), sizeof(AxisNode)));
+    CU(t.alloc(SceneTree::kDiag, f.diag.size() * 4, sizeof(float4)));
+    CU(t.alloc(SceneTree::kSlot, (size_t)n_tri, sizeof(int)));
+    t.n_wide4 = nw;
+    float4* wide = t.get<float4>(SceneTree::kWideTris);
+    if (nw) CU(cudaMemcpyAsync(wide, f.wide.data(), nw * sizeof(float4), cudaMemcpyHostToDevice, st));
+    if (nt) CU(cudaMemcpyAsync(wide + nw, f.tris.data(), nt * sizeof(float4), cudaMemcpyHostToDevice, st));
+    if (!f.axis.empty()) CU(cudaMemcpyAsync(t.get<void>(SceneTree::kAxis), f.axis.data(), f.axis.size() * sizeof(AxisNode), cudaMemcpyHostToDevice, st));
+    if (!f.diag.empty()) CU(cudaMemcpyAsync(t.get<void>(SceneTree::kDiag), f.diag.data(), f.diag.size() * sizeof(DiagNode), cudaMemcpyHostToDevice, st));
+    CU(launch_slot_of_prim(wide + nw, n_tri, t.get<int>(SceneTree::kSlot), st));
+    return B200RT_OK;
+}
+
+// Makes t replica r's tree, described by info, and releases the tree it replaces (r's device must be current)
+void install_tree(b200rt_scene* r, SceneTree&& t, const b200rt_bvh_info& info)
+{
+    SceneTree old = std::move(r->tree);
+    r->tree = std::move(t);
+    r->bytes = r->bytes - old.total() + r->tree.total();
+    const float4* wide = r->tree.get<float4>(SceneTree::kWideTris);
+    r->dev.wide = wide;
+    r->dev.tris = wide + r->tree.n_wide4;
+    r->dev.axis = r->tree.get<float4>(SceneTree::kAxis);
+    r->dev.diag = r->tree.get<float4>(SceneTree::kDiag);
+    r->dev.slot_of_prim = r->tree.get<int>(SceneTree::kSlot);
+    r->dev.has_wide = info.n_wide_nodes > 0 ? 1 : 0;
+    r->dev.has_diag = info.has_diag_slabs;
+    r->info = info;
+    release_refit(r);
 }
 
 // uploads one replica of the scene to `device`
@@ -731,19 +789,14 @@ int create_on_device(const SceneArgs& a, const FlatBVH& f, const SceneHostData& 
     std::unique_ptr<b200rt_scene> s(new (std::nothrow) b200rt_scene);     // frees a half-built replica on every early return
     if (!s) return fail(B200RT_ERR_ALLOC, "out of host memory");
     s->device = device;
-    s->info = f.info;
     s->mat_used.assign((size_t)a.n_materials, 0);
     for (int i = 0; i < a.n_material_indices; i++) { s->mat_used[a.tri_material[i]] = 1; s->max_mat_index = std::max(s->max_mat_index, a.tri_material[i]); }
-    const size_t nt = f.tris.size() * 3;
-    int rc = upload(s.get(), h.bvh_and_tris.data(), h.n_wide4 + nt, &s->dev.wide);
+    SceneTree tree;
+    int rc = tree_from_host(f, a.n_tri, 0, tree);
     if (rc) return rc;
-    s->dev.tris = s->dev.wide + h.n_wide4;
-    s->dev.has_wide = f.wide.empty() ? 0 : 1;
+    install_tree(s.get(), std::move(tree), f.info);
     s->dev.qmagic = 0x43000000u;
     if ((rc = upload(s.get(), h.oct_lut.data(), h.oct_lut.size(), &s->dev.oct_lut))) return rc;
-    if ((rc = upload(s.get(), reinterpret_cast<const float4*>(f.axis.data()), f.axis.size() * 4, &s->dev.axis))) return rc;
-    if ((rc = upload(s.get(), reinterpret_cast<const float4*>(f.diag.data()), f.diag.size() * 4, &s->dev.diag))) return rc;
-    if ((rc = upload(s.get(), h.slot_of_prim.data(), (size_t)a.n_tri, &s->dev.slot_of_prim))) return rc;
     if ((rc = upload(s.get(), a.tri_material, (size_t)a.n_material_indices, &s->dev.mat_idx))) return rc;
     if ((rc = upload(s.get(), a.emissive_tri, (size_t)a.n_emissive, &s->dev.emissive))) return rc;
     if ((rc = upload(s.get(), h.spheres.data(), (size_t)a.n_spheres, &s->dev.spheres))) return rc;
@@ -763,7 +816,6 @@ int create_on_device(const SceneArgs& a, const FlatBVH& f, const SceneHostData& 
     else if ((rc = upload(s.get(), reinterpret_cast<const float4*>(a.env_rgba), n_texels, &s->dev.env))) return rc;
     s->dev.n_tri = a.n_tri; s->dev.n_emissive = a.n_emissive; s->dev.n_spheres = a.n_spheres;
     s->dev.env_w = a.env_w; s->dev.env_h = a.env_h;
-    s->dev.has_diag = f.info.has_diag_slabs;
     // env tables (K5, env_tables.cu): per-texel luminance, the running-sum CDF in the reference's serial float order
     // (Utils::compute_env_map_cdf, utils.cpp:126-142) unless the caller brings its own, and the last-column copy the row search probes
     float* d_lum = nullptr; float* d_cdf = nullptr; float* d_row = nullptr;
@@ -825,7 +877,7 @@ int create_scene(const SceneArgs& a, const b200rt_bvh* bvh_or_null, const int* d
     if (bvh->flat.info.n_triangles != a.n_tri) { delete own; return fail(B200RT_ERR_ARG, "BVH was built for %d triangles, scene has %d", bvh->flat.info.n_triangles, a.n_tri); }
 
     SceneHostData h;
-    prepare_host_data(a, bvh->flat, h);
+    prepare_host_data(a, h);
     b200rt_scene* first = nullptr;
     rc = create_on_device(a, bvh->flat, h, devs[0], &first);
     for (int i = 1; i < n_devices && !rc; i++)
@@ -1126,20 +1178,39 @@ int run_ranks(int n_dev, F rank_body)
 
 // The refit state of one replica: level lists by a breadth-first walk of the resident records (which it only reads) and the per-node
 // exact-box arrays. Made once; a failure leaves the scene as it was, and the next update tries again.
+// the extent pass's words and the SAH scratch (the refit and the rebuild share them); r's device must be current
+int ensure_refit_scratch(b200rt_scene* r)
+{
+    int rc = B200RT_OK;
+    if (!r->d_refit_misc && (rc = device_alloc(r, &r->d_refit_misc, 4))) return rc;
+    if (!r->d_sah && (rc = device_alloc(r, &r->d_sah, refit_sah_scratch_doubles()))) return rc;
+    return B200RT_OK;
+}
+
+// a per-node refit array of at least n elements, counted in the scene's bytes
+template <typename T>
+int grow_counted(b200rt_scene* r, DevArray<T>& a, size_t n)
+{
+    n = std::max<size_t>(n, 1);
+    if (n <= a.cap) return B200RT_OK;
+    r->bytes -= a.cap * sizeof(T);
+    const cudaError_t e = a.grow(n);
+    r->bytes += a.cap * sizeof(T);
+    CU(e);
+    return B200RT_OK;
+}
+
 int ensure_refit(b200rt_scene* r)
 {
     if (r->refit_ready) return B200RT_OK;
     ON_DEVICE(r->device);
     const size_t n_wide = (size_t)r->info.n_wide_nodes, n_axis = (size_t)r->info.n_inner_nodes;
     int rc = B200RT_OK;
-    if (!r->d_refit_misc && (rc = device_alloc(r, &r->d_refit_misc, 4))) return rc;
-    if (!r->d_sah && (rc = device_alloc(r, &r->d_sah, refit_sah_scratch_doubles()))) return rc;
-    if (!r->d_wide_idx && (rc = device_alloc(r, &r->d_wide_idx, n_wide))) return rc;
-    if (!r->d_axis_idx && (rc = device_alloc(r, &r->d_axis_idx, n_axis))) return rc;
-    if (!r->d_wide_box && (rc = device_alloc(r, &r->d_wide_box, 2 * n_wide))) return rc;
-    if (!r->d_axis_box && (rc = device_alloc(r, &r->d_axis_box, 4 * n_axis))) return rc;
+    if ((rc = ensure_refit_scratch(r)) || (rc = grow_counted(r, r->d_wide_idx, n_wide)) || (rc = grow_counted(r, r->d_axis_idx, n_axis)) ||
+        (rc = grow_counted(r, r->d_wide_box, 2 * n_wide)) || (rc = grow_counted(r, r->d_axis_box, 4 * n_axis)))
+        return rc;
     const cudaError_t e = refit_levels(reinterpret_cast<const WideNode*>(r->dev.wide), (int)n_wide, reinterpret_cast<const AxisNode*>(r->dev.axis),
-                                       (int)n_axis, r->d_wide_idx, r->d_axis_idx, reinterpret_cast<int*>(r->d_refit_misc + 3),
+                                       (int)n_axis, r->d_wide_idx.get(), r->d_axis_idx.get(), reinterpret_cast<int*>(r->d_refit_misc + 3),
                                        r->wide_level, r->axis_level, 0);
     if (e == cudaErrorInvalidValue) return fail(B200RT_ERR_ARG, "the scene's BVH records do not form one tree rooted at record 0");
     if (e != cudaSuccess) return fail(B200RT_ERR_CUDA, "BVH level lists: %s", cudaGetErrorString(e));
@@ -1160,9 +1231,9 @@ int refit_rank(b200rt_scene* r, const float* v, float abs_pad, cudaStream_t st, 
     A.wide = reinterpret_cast<WideNode*>(const_cast<float4*>(r->dev.wide));
     A.axis = reinterpret_cast<AxisNode*>(const_cast<float4*>(r->dev.axis));
     A.diag = r->dev.has_diag ? reinterpret_cast<DiagNode*>(const_cast<float4*>(r->dev.diag)) : nullptr;
-    A.wide_idx = r->d_wide_idx; A.axis_idx = r->d_axis_idx;
+    A.wide_idx = r->d_wide_idx.get(); A.axis_idx = r->d_axis_idx.get();
     A.wide_level = &r->wide_level; A.axis_level = &r->axis_level;
-    A.wide_box = r->d_wide_box; A.axis_box = r->d_axis_box;
+    A.wide_box = r->d_wide_box.get(); A.axis_box = r->d_axis_box.get();
     A.n_tri = r->dev.n_tri; A.n_axis = r->info.n_inner_nodes;
     A.abs_pad = abs_pad;
     A.overflow = overflow;
@@ -1181,6 +1252,16 @@ int refit_rank(b200rt_scene* r, const float* v, float abs_pad, cudaStream_t st, 
     return B200RT_OK;
 }
 
+// vertices given to a _device entry point must be device (or managed) memory of the scene's first device
+int check_device_vertices(const b200rt_scene* s, const void* src)
+{
+    cudaPointerAttributes pa;
+    if (cudaPointerGetAttributes(&pa, src) != cudaSuccess) { cudaGetLastError(); pa.type = cudaMemoryTypeUnregistered; }
+    if (!((pa.type == cudaMemoryTypeDevice && pa.device == s->device) || pa.type == cudaMemoryTypeManaged))
+        return fail(B200RT_ERR_ARG, "dev_tri_xyz9 must be device memory of the scene's first device (%d)", s->device);
+    return B200RT_OK;
+}
+
 // b200rt_scene_update_triangles[_device]: new vertices for every replica of the scene. src is host memory, or (src_on_device) device
 // memory of the scene's first device that the caller's stream `caller_st` produces.
 int update_triangles(b200rt_scene* s, const void* src, bool src_on_device, int n_tri, cudaStream_t caller_st, b200rt_stats* stats)
@@ -1192,13 +1273,7 @@ int update_triangles(b200rt_scene* s, const void* src, bool src_on_device, int n
     int rc = require_device("b200rt_scene_update_triangles");
     if (rc) return rc;
     const auto t0 = std::chrono::high_resolution_clock::now();
-    if (src_on_device)
-    {
-        cudaPointerAttributes pa;
-        if (cudaPointerGetAttributes(&pa, src) != cudaSuccess) { cudaGetLastError(); pa.type = cudaMemoryTypeUnregistered; }
-        if (!((pa.type == cudaMemoryTypeDevice && pa.device == s->device) || pa.type == cudaMemoryTypeManaged))
-            return fail(B200RT_ERR_ARG, "dev_tri_xyz9 must be device memory of the scene's first device (%d)", s->device);
-    }
+    if (src_on_device && (rc = check_device_vertices(s, src))) return rc;
     std::vector<b200rt_scene*> ranks(1, s);
     ranks.insert(ranks.end(), s->replicas.begin(), s->replicas.end());
     const int n_dev = (int)ranks.size();
@@ -1251,6 +1326,136 @@ int update_triangles(b200rt_scene* s, const void* src, bool src_on_device, int n
         for (const LaunchResult& r : res) { ms = std::max(ms, r.ms); stats->gpu_launches += r.launches; }
         stats->kernel_ms = extent.ms + ms;
         stats->h2d_bytes = src_on_device ? 0 : bytes * (unsigned long long)n_dev;
+        stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::high_resolution_clock::now() - t0).count();
+    }
+    return B200RT_OK;
+}
+
+// b200rt_scene_rebuild_bvh[_device]: a new tree over new vertices for every replica. It is built on the scene's first device by the
+// device builder (or, for inputs it declines, by the host builder, as b200rt_bvh_build_device does) into arrays beside the old tree,
+// sent to the other replicas device to device, and swapped in only once every replica holds its copy: any refusal or failure before
+// that leaves every replica's old tree in place. src as for update_triangles.
+int rebuild_bvh(b200rt_scene* s, const void* src, bool src_on_device, int n_tri, cudaStream_t caller_st, b200rt_stats* stats)
+{
+    if (!s || !src) return fail(B200RT_ERR_ARG, "scene and triangle buffer must not be NULL");
+    if (n_tri != s->dev.n_tri) return fail(B200RT_ERR_ARG, "%d triangles, but the scene has %d (a rebuild keeps the triangles)", n_tri, s->dev.n_tri);
+    if (n_tri >= (1 << 27)) return fail(B200RT_ERR_ARG, "at most 2^27-1 triangles (leaf references pack first<<4|count)");
+    if (stats) std::memset(stats, 0, sizeof(*stats));
+    int rc = require_device("b200rt_scene_rebuild_bvh");
+    if (rc) return rc;
+    const auto t0 = std::chrono::high_resolution_clock::now();
+    if (src_on_device && (rc = check_device_vertices(s, src))) return rc;
+    const size_t bytes = 9 * (size_t)n_tri * sizeof(float);
+    for (b200rt_scene* r : s->replicas)
+        if ((rc = ensure_rank_stream(r))) return rc;
+    ON_DEVICE(s->device);
+    if ((rc = ensure_scratch(s, 0, 0, 0)) || (rc = ensure_refit_scratch(s))) return rc;
+    if (!src_on_device && s->d_vertices.cap < 9 * (size_t)n_tri) CU(s->d_vertices.grow(9 * (size_t)n_tri));
+    const cudaStream_t st = src_on_device ? caller_st : 0;
+    const float* v = src_on_device ? static_cast<const float*>(src) : s->d_vertices.get();
+    unsigned long long h2d = 0, d2h = 0;
+    int launches = 0;
+    if (!src_on_device)
+    {
+        if ((rc = copy_to_device(s, s->d_vertices.get(), src, bytes, st))) return rc;
+        h2d += bytes;
+    }
+    // 1. the extent pass: a non-finite coordinate refuses the rebuild before anything is built
+    CU(cudaEventRecord(s->ev0, st));
+    unsigned int misc[2] = { 0, 0 };
+    CU(refit_extent(v, n_tri, s->d_refit_misc, st));
+    CU(cudaMemcpyAsync(misc, s->d_refit_misc, sizeof(misc), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    launches += 1; d2h += sizeof(misc);
+    if (misc[1]) return fail(B200RT_ERR_ARG, "a vertex coordinate is NaN or infinite: no box can bound it");
+    // 2. the new tree on the first device, beside the old one
+    SceneTree tree;
+    b200rt_bvh_info info{};
+    int built = 2;
+    if (n_tri > kWideMaxLeaf)
+    {
+        const DeviceTreeAlloc alloc = [&](size_t n_wide, size_t n_axis, DeviceTree& out) {
+            tree = SceneTree{};                                      // a second attempt replaces the first one's arrays
+            tree.n_wide4 = 5 * n_wide;
+            cudaError_t e = tree.alloc(SceneTree::kWideTris, 5 * n_wide + 3 * (size_t)n_tri, sizeof(float4));
+            if (e == cudaSuccess) e = tree.alloc(SceneTree::kAxis, n_axis, sizeof(AxisNode));
+            if (e == cudaSuccess) e = tree.alloc(SceneTree::kDiag, 0, sizeof(float4));       // no diagonal slabs, as on a device-built scene
+            if (e == cudaSuccess) e = tree.alloc(SceneTree::kSlot, (size_t)n_tri, sizeof(int));
+            out.wide_and_tris = tree.get<float4>(SceneTree::kWideTris);
+            out.axis = tree.get<AxisNode>(SceneTree::kAxis);
+            return e;
+        };
+        DeviceBuildCounts counts;
+        std::string err;
+        try { built = build_bvh_device(v, n_tri, st, alloc, info, counts, err); }
+        catch (const std::exception& e) { err = e.what(); built = 1; }
+        if (built == 1) return fail(B200RT_ERR_CUDA, "device BVH build: %s", err.c_str());
+        launches += counts.launches; h2d += counts.h2d_bytes; d2h += counts.d2h_bytes;
+        if (built == 0) { CU(launch_slot_of_prim(tree.get<float4>(SceneTree::kWideTris) + tree.n_wide4, n_tri, tree.get<int>(SceneTree::kSlot), st)); launches += 1; }
+    }
+    if (built == 2)
+    {
+        // the host builder, for what the device builders decline (at most 3 triangles, a tree deeper than the traversal stack)
+        std::vector<float> host_v;
+        const float* hv = static_cast<const float*>(src);
+        if (src_on_device)
+        {
+            host_v.resize(9 * (size_t)n_tri);
+            if ((rc = copy_to_host(s, host_v.data(), v, bytes, st))) return rc;
+            d2h += bytes; hv = host_v.data();
+        }
+        b200rt_bvh* hb = nullptr;
+        if ((rc = b200rt_bvh_build(hv, n_tri, nullptr, &hb))) return rc;
+        const std::unique_ptr<b200rt_bvh, void (*)(b200rt_bvh*)> own(hb, b200rt_bvh_destroy);
+        tree = SceneTree{};
+        if ((rc = tree_from_host(hb->flat, n_tri, st, tree))) return rc;
+        CU(cudaStreamSynchronize(st));                               // the host tree is the copies' source
+        const FlatBVH& f = hb->flat;
+        info = f.info;
+        h2d += f.wide.size() * sizeof(WideNode) + f.tris.size() * sizeof(LeafTriangle) + f.axis.size() * sizeof(AxisNode) + f.diag.size() * sizeof(DiagNode);
+        launches += 1;
+    }
+    // 3. its SAH cost by the refit's reduction, so that it compares with a refitted tree's
+    double sah = 0.0;
+    CU(refit_sah(tree.get<AxisNode>(SceneTree::kAxis), info.n_inner_nodes, s->d_sah, st));
+    CU(cudaMemcpyAsync(&sah, s->d_sah + refit_sah_scratch_doubles() - 1, sizeof(double), cudaMemcpyDeviceToHost, st));
+    CU(cudaEventRecord(s->ev1, st));
+    CU(cudaStreamSynchronize(st));
+    launches += 2; d2h += sizeof(double);
+    info.sah_cost = sah;
+    // 4. the other replicas' copies, device to device, beside their old trees
+    std::vector<SceneTree> copies(s->replicas.size());
+    for (size_t i = 0; i < s->replicas.size(); i++)
+    {
+        b200rt_scene* r = s->replicas[i];
+        ON_DEVICE(r->device);
+        copies[i].n_wide4 = tree.n_wide4;
+        for (int k = 0; k < SceneTree::kArrays; k++)
+        {
+            CU(copies[i].alloc(k, tree.bytes[k], 1));
+            CU(cudaMemcpyPeerAsync(copies[i].mem[k].get(), r->device, tree.mem[k].get(), s->device, tree.bytes[k], r->mg_stream));
+        }
+    }
+    for (size_t i = 0; i < s->replicas.size(); i++)
+    {
+        ON_DEVICE(s->replicas[i]->device);
+        CU(cudaStreamSynchronize(s->replicas[i]->mg_stream));
+    }
+    // 5. every replica has its copy: swap them in (each old tree is freed on its own device)
+    info.build_seconds = std::chrono::duration<double>(std::chrono::high_resolution_clock::now() - t0).count();
+    for (size_t i = 0; i < s->replicas.size(); i++)
+    {
+        ON_DEVICE(s->replicas[i]->device);
+        install_tree(s->replicas[i], std::move(copies[i]), info);
+    }
+    install_tree(s, std::move(tree), info);
+    if (stats)
+    {
+        float ms = 0.0f;
+        CU(cudaEventElapsedTime(&ms, s->ev0, s->ev1));
+        stats->kernel_ms = ms;
+        stats->gpu_launches = launches;
+        stats->h2d_bytes = h2d; stats->d2h_bytes = d2h;
         stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::high_resolution_clock::now() - t0).count();
     }
     return B200RT_OK;
@@ -1405,6 +1610,16 @@ int b200rt_scene_update_triangles(b200rt_scene* s, const float* tri_xyz9, int n_
 int b200rt_scene_update_triangles_device(b200rt_scene* s, const void* dev_tri_xyz9, int n_tri, void* cuda_stream, b200rt_stats* stats)
 {
     return update_triangles(s, dev_tri_xyz9, true, n_tri, (cudaStream_t)cuda_stream, stats);
+}
+
+int b200rt_scene_rebuild_bvh(b200rt_scene* s, const float* tri_xyz9, int n_tri, b200rt_stats* stats)
+{
+    return rebuild_bvh(s, tri_xyz9, false, n_tri, 0, stats);
+}
+
+int b200rt_scene_rebuild_bvh_device(b200rt_scene* s, const void* dev_tri_xyz9, int n_tri, void* cuda_stream, b200rt_stats* stats)
+{
+    return rebuild_bvh(s, dev_tri_xyz9, true, n_tri, (cudaStream_t)cuda_stream, stats);
 }
 
 int b200rt_scene_get_bvh_arrays(b200rt_scene* s, int replica, void* wide80_out, float* axis16_out, float* diag16_out, float* tris12_out)

@@ -114,5 +114,7 @@ struct RefitArgs
 };
 // triangle stream, then every level of both layouts deepest first, then the SAH cost; *launches = kernels launched
 cudaError_t refit_tree(const RefitArgs& args, cudaStream_t stream, int* launches);
+// the SAH cost of n_axis > 0 binary records (sah_cost_of's formula, fixed summation order) into sah[refit_sah_scratch_doubles() - 1]; 2 launches
+cudaError_t refit_sah(const AxisNode* axis, int n_axis, double* sah, cudaStream_t stream);
 
 } // namespace b200rt

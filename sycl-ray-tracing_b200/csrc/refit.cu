@@ -5,7 +5,7 @@
 //   3. one launch per tree level, deepest first, for each layout: a node's exact (unpadded) box goes to a per-node scratch array,
 //      and the node pads its children's exact boxes once, exactly as the builders do                  (rf_wide_level, rf_axis_level)
 //   4. the SAH cost of the refitted binary records, sah_cost_of's formula, in double                   (rf_sah_partial, rf_sah_final)
-// Level lists come from a breadth-first walk from record 0 (rf_bfs_*): record order is not a topological order (append_top_level
+// Level lists come from a breadth-first walk from record 0 (rf_bfs_*): record order is not a topological order (make_top_level
 // moves the old root to the end of both arrays).
 #include <algorithm>
 #include <cfloat>
@@ -350,10 +350,17 @@ cudaError_t refit_tree(const RefitArgs& R, cudaStream_t st, int* launches)
     }
     if (R.n_axis > 0)
     {
-        rf_sah_partial<<<kSahBlocks, kSahThreads, 0, st>>>(R.axis, R.n_axis, R.sah);
-        rf_sah_final<<<1, kSahThreads, 0, st>>>(R.sah);
+        cudaError_t e = refit_sah(R.axis, R.n_axis, R.sah, st);
+        if (e != cudaSuccess) return e;
         *launches += 2;
     }
+    return cudaGetLastError();
+}
+
+cudaError_t refit_sah(const AxisNode* axis, int n_axis, double* sah, cudaStream_t st)
+{
+    rf_sah_partial<<<kSahBlocks, kSahThreads, 0, st>>>(axis, n_axis, sah);
+    rf_sah_final<<<1, kSahThreads, 0, st>>>(sah);
     return cudaGetLastError();
 }
 
