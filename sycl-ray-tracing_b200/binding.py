@@ -11,7 +11,7 @@ import os
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("B200RT_LIB") or os.path.join(HERE, "libb200rt.so")     # B200RT_LIB: development builds with other tunables
+LIB_PATH = os.environ.get("B200RT_LIB") or os.path.join(HERE, "libb200rt.so")     # B200RT_LIB: another build of the library (A/B comparisons)
 
 INTEGRATOR_MEGAKERNEL = 0
 INTEGRATOR_WAVEFRONT = 1

@@ -13,7 +13,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
-LIB = os.path.join(HERE, os.environ.get("B200RT_BUILD_LIB", "libb200rt.so"))
+LIB = os.path.join(HERE, os.environ.get("B200RT_BUILD_LIB", "libb200rt.so"))     # B200RT_BUILD_LIB: a second library beside the default, for A/B comparisons
 SOURCES = ["capi.cu", "kernels.cu", "wavefront.cu", "persist.cu", "env_tables.cu", "denoise.cu", "bvh_build_gpu.cu", "refit.cu", "bvh_build.cpp", "obj_ingest.cpp", "hdr_ingest.cpp"]
 HEADERS = ["bvh_build.h", "bvh_emit.cuh", "device_types.h", "kernels.h", "pt_device.cuh", "wf_device.cuh", "obj_ingest.h", os.path.join("..", "..", "include", "b200rt.h")]
 
@@ -21,7 +21,6 @@ NVCC_FLAGS = [
     "-O3", "-std=c++17", "-lineinfo",
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-fmad=false",
-] + (["-DB200RT_PREFETCH"] if os.environ.get("B200RT_BUILD_PREFETCH") else []) + os.environ.get("B200RT_BUILD_DEFS", "").split() + [
     "-Xcompiler", "-fPIC,-fopenmp,-O3",
     "-ccbin", "/usr/bin/g++",
 ]

@@ -5,8 +5,6 @@
 #include <atomic>
 #include <chrono>
 #include <cmath>
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <limits>
 #include <stdexcept>
@@ -477,7 +475,6 @@ void build_flat_bvh(const float* tri9, int n_tri, const b200rt_bvh_options& opts
     }
     else builder.make_leaf(root, 0, 0);
 
-    if (getenv("B200RT_BUILD_TIMING")) fprintf(stderr, "bvh build: sah %.3f s\n", std::chrono::duration<double>(std::chrono::high_resolution_clock::now() - t0).count());
     const float abs_pad = 2e-6f * scene_abs + 1e-30f;
     out.axis.reserve((size_t)std::max(1, n_tri / 2));
     out.tris.reserve((size_t)n_tri);
@@ -493,7 +490,6 @@ void build_flat_bvh(const float* tri9, int n_tri, const b200rt_bvh_options& opts
         if (wb.overflow) throw std::runtime_error("wide BVH quantisation overflow");
         wide_depth = wb.max_depth;
     }
-    if (getenv("B200RT_BUILD_TIMING")) fprintf(stderr, "bvh build: +wide %.3f s\n", std::chrono::duration<double>(std::chrono::high_resolution_clock::now() - t0).count());
     Flattener fl{ builder, tri9, out, abs_pad };
     if (!leaf_first.empty()) fl.leaf_first = &leaf_first;
     Slabs s; int cnt = 0;
@@ -514,7 +510,6 @@ void build_flat_bvh(const float* tri9, int n_tri, const b200rt_bvh_options& opts
     }
     else fl.flatten(root, 0, s, cnt);
 
-    if (getenv("B200RT_BUILD_TIMING")) fprintf(stderr, "bvh build: +flatten %.3f s\n", std::chrono::duration<double>(std::chrono::high_resolution_clock::now() - t0).count());
     // SAH cost of the final tree (diagnostic): sum over inner nodes of child areas / root area
     double root_area = std::max(1e-30f, builder.nodes[root].box.half_area());
     double sah = 0.0;

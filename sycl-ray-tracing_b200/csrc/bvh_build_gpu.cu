@@ -8,8 +8,9 @@
 //      clustering for bounding volume hierarchy construction", TVCG 2018): every cluster looks 16 places left and right along the
 //      Morton curve for the neighbour whose merged box has the smallest surface area; mutual nearest neighbours merge; repeat
 //      (~30 rounds). A surface-area-driven agglomerative build: round 1 built the radix tree of the Morton codes instead (Karras 2012,
-//      still available as B200RT_DEVICE_BUILDER=lbvh: lb_tree + lb_fit), whose splits ignore surface area — path tracing was 8-13 %
-//      and coherent camera rays 57 % slower on its trees than on the host builder's binned-SAH ones
+//      lb_tree + lb_fit), whose splits ignore surface area — path tracing was 8-13 % and coherent camera rays 57 % slower on its
+//      trees than on the host builder's binned-SAH ones. The radix tree remains the fallback for inputs that clustering refuses
+//      (more than 512 rounds, or a tree deeper than the traversal stack)
 //   4. the clustered tree is laid out depth-first (pl_layout): every subtree covers a contiguous range of the triangle order
 //   5. subtrees of <= 3 triangles become leaves; level-by-level collapse into the 8-ary layout: every wide node opens its
 //      largest children until it has 8, assigns them to octant slots     (lw_expand, lw_link; prefix sums give child_base / tri_base)
@@ -26,7 +27,6 @@
 #include <cfloat>
 #include <chrono>
 #include <cstdint>
-#include <cstdlib>
 #include <cstring>
 #include <string>
 #include <vector>
@@ -216,6 +216,7 @@ __global__ void lb_fit(DevArrays A, int* max_depth)
 
 // ---- parallel locally-ordered clustering -----------------------------------------------------------------------------------------
 constexpr int kPlocRadius = 32;          // largest search radius (shared-memory halo); the radius in use is a launch argument
+constexpr int kPlocSearchRadius = 16;    // the radius in use
 constexpr int kPlocBlock = 256;
 
 struct PlocArrays
@@ -547,9 +548,10 @@ __global__ void lb_emit(DevArrays A, WideArrays W, const int* live, const int* a
 
 // ---- top of the clustered tree: surface-area-heuristic sweep on the host -----------------------------------------------------------
 // Agglomerative clustering builds excellent lower levels and mediocre upper ones (few, large clusters seen through a fixed window
-// along the Morton curve), and every ray walks the upper levels. When at most 1024 clusters (B200RT_PLOC_TOP) are left the clustering stops and
+// along the Morton curve), and every ray walks the upper levels. When at most kPlocTop clusters are left the clustering stops and
 // the tree above them is built top-down by a full SAH sweep (sort by centroid on every axis, cost = area x triangles below): a few
 // thousand boxes, well under a millisecond on the host.
+constexpr int kPlocTop = 1024;
 struct TopCluster { float lo[3], hi[3]; int ref, size; };
 
 struct TopBuilder
@@ -653,9 +655,7 @@ static int build_bvh_device_impl(const float* d_tri9, int n_tri, cudaStream_t st
     DevArrays A;
     memset(&A, 0, sizeof(A));
     A.n = n_tri;
-    static const int leaf_env = []() { const char* e = getenv("B200RT_DEVICE_LEAF"); const int v = e ? atoi(e) : kWideMaxLeaf; return v < 1 ? 1 : (v > kWideMaxLeaf ? kWideMaxLeaf : v); }();
-    static const int ploc_radius = []() { const char* e = getenv("B200RT_PLOC_RADIUS"); const int v = e ? atoi(e) : 16; return v < 1 ? 1 : (v > kPlocRadius ? kPlocRadius : v); }();
-    A.leaf_max = leaf_env;
+    A.leaf_max = kWideMaxLeaf;
     const size_t n = (size_t)n_tri;
     A.tri9 = d_tri9;
     GCU(pool.get(&A.plo, n)); GCU(pool.get(&A.phi, n));
@@ -724,13 +724,12 @@ static int build_bvh_device_impl(const float* d_tri9, int n_tri, cudaStream_t st
         const int first_node = n_tri - 2;
         GCU(h2d(P.next_node, &first_node, sizeof(int)));
         pl_init<<<grid_n, tb, 0, st>>>(A, P); C.launches++;
-        static const int top_clusters = []() { const char* e = getenv("B200RT_PLOC_TOP"); const int v = e ? atoi(e) : 1024; return v < 1 ? 1 : v; }();
         int nc = n_tri, cur = 0, rounds = 0;
-        while (nc > top_clusters)
+        while (nc > kPlocTop)
         {
             if (++rounds > 512) { err = "clustering needs more than 512 rounds (a size gradient along the Morton curve merges one pair per round)"; return 2; }
             const int g = (nc + kPlocBlock - 1) / kPlocBlock;
-            pl_nearest<<<g, kPlocBlock, 0, st>>>(P.clo[cur], P.chi[cur], nc, ploc_radius, P.nn);
+            pl_nearest<<<g, kPlocBlock, 0, st>>>(P.clo[cur], P.chi[cur], nc, kPlocSearchRadius, P.nn);
             pl_merge<<<g, kPlocBlock, 0, st>>>(A, P, cur, nc);
             GCU(cub::DeviceScan::ExclusiveSum(pscan_tmp, pscan_bytes, P.valid, P.pos, nc, st));
             pl_compact<<<g, kPlocBlock, 0, st>>>(P, cur, nc);
@@ -918,9 +917,7 @@ static int build_bvh_device_impl(const float* d_tri9, int n_tri, cudaStream_t st
 int build_bvh_device(const float* d_tri9, int n_tri, cudaStream_t st, const DeviceTreeAlloc& alloc, b200rt_bvh_info& info,
                      DeviceBuildCounts& counts, std::string& err)
 {
-    static const bool lbvh_only = []() { const char* e = getenv("B200RT_DEVICE_BUILDER"); return e && std::string(e) == "lbvh"; }();
-    int rc = 2;
-    if (!lbvh_only) rc = build_bvh_device_impl(d_tri9, n_tri, st, false, alloc, info, counts, err);
+    int rc = build_bvh_device_impl(d_tri9, n_tri, st, false, alloc, info, counts, err);
     if (rc == 2) rc = build_bvh_device_impl(d_tri9, n_tri, st, true, alloc, info, counts, err);
     return rc;
 }

@@ -449,9 +449,6 @@ int alloc_wf_buffers(std::vector<DevPtr>& mem, WfBuffers& w, size_t n)
 // (multi-GPU) is latency-bound per pass and gains a little from a fourth chain (one rank of 8 emulated: 115.9 -> 112.2 ms)
 int wavefront_group_count(const RenderParams& P)
 {
-    const char* e = getenv("B200RT_WF_GROUPS");          // read per frame (tools sweep it inside one process)
-    const int env_n = e ? std::min(atoi(e), kMaxWfGroups) : 0;
-    if (env_n >= 1) return env_n;
     return (long long)P.n_rank_tiles * kTilePixels < 700000 ? 4 : 3;
 }
 
@@ -830,9 +827,9 @@ int create_on_device(const SceneArgs& a, const FlatBVH& f, const SceneHostData& 
     if (ce == cudaSuccess) ce = cudaMemcpy(&s->dev.cdf_total, d_cdf + n_texels - 1, sizeof(float), cudaMemcpyDeviceToHost);
     if (ce != cudaSuccess) return fail(B200RT_ERR_CUDA, "env tables: %s", cudaGetErrorString(ce));
     s->dev.cdf = d_cdf; s->dev.row_cdf = d_row; s->d_env_lum = d_lum;
-    // guide table of the CDF search (bit-identical texel choice, ~2 probes instead of log2(W) + log2(H)); B200RT_CDF_GUIDE=0 turns it off
-    static const int guide_buckets = []() { const char* e = getenv("B200RT_CDF_GUIDE"); int v = e ? atoi(e) : 65536; return v < 0 ? 0 : v; }();
-    if (guide_buckets > 0 && n_texels >= 64)
+    // guide table of the CDF search (bit-identical texel choice, ~2 probes instead of log2(W) + log2(H))
+    constexpr int guide_buckets = 65536;
+    if (n_texels >= 64)
     {
         unsigned int* d_guide = nullptr;
         if ((rc = device_alloc(s.get(), &d_guide, (size_t)guide_buckets + 2))) return rc;
@@ -869,8 +866,7 @@ int create_scene(const SceneArgs& a, const b200rt_bvh* bvh_or_null, const int* d
     if (!bvh)
     {
         // above ~5 M triangles the host SAH build dominates the whole job (12.5 s at 20 M, DESIGN.md): build on the GPU instead
-        static const int device_build_threshold = []() { const char* e = getenv("B200RT_DEVICE_BUILD_MIN_TRIS"); return e ? atoi(e) : 5000000; }();
-        rc = a.n_tri >= device_build_threshold ? b200rt_bvh_build_device(a.tri_xyz9, a.n_tri, devs[0], &own) : b200rt_bvh_build(a.tri_xyz9, a.n_tri, nullptr, &own);
+        rc = a.n_tri >= 5000000 ? b200rt_bvh_build_device(a.tri_xyz9, a.n_tri, devs[0], &own) : b200rt_bvh_build(a.tri_xyz9, a.n_tri, nullptr, &own);
         if (rc) return rc;
         bvh = own;
     }
@@ -1882,7 +1878,7 @@ int b200rt_env_cdf_search(b200rt_scene* s, const float* values, int n, int use_g
     ON_DEVICE(s->device);
     SceneDev dev = s->dev;
     if (!use_guide) dev.cdf_guide = nullptr;
-    else if (!dev.cdf_guide) return fail(B200RT_ERR_ARG, "this scene has no CDF guide table (the running sum is not monotone, or B200RT_CDF_GUIDE=0)");
+    else if (!dev.cdf_guide) return fail(B200RT_ERR_ARG, "this scene has no CDF guide table (the running sum is not monotone, or the map has fewer than 64 texels)");
     DevArray<float> d_v; DevArray<int> d_xy;
     cudaError_t e = d_v.grow((size_t)n);
     if (e == cudaSuccess) e = d_xy.grow(2 * (size_t)n);

@@ -10,21 +10,19 @@
 // costs what ITS warp's rays cost. Same device functions on the same per-pixel RNG streams: the frame is bit-identical to
 // the other integrators' and the ray count is the same.
 #include <algorithm>
-#include <cstdlib>
 
 #include "wf_device.cuh"
 
 namespace b200rt {
 
-#ifndef PERSIST_MIN_BLOCKS
-#define PERSIST_MIN_BLOCKS 5
-#endif
+constexpr int kPersistMinBlocks = 5;
+constexpr int kPersistSlotsPerLane = 2;       // K: state slots per lane of pt_persist
 
-template <int K>
-__global__ void __launch_bounds__(32 * kCoopMaxWarps, PERSIST_MIN_BLOCKS)
+__global__ void __launch_bounds__(32 * kCoopMaxWarps, kPersistMinBlocks)
 pt_persist(SceneDev S, RenderParams P, WfBuffers B, unsigned int* next_pixel, int n_frame_slots, const float4* __restrict__ fb_in_rowmajor,
            float4* __restrict__ out_tiles)
 {
+    constexpr int K = kPersistSlotsPerLane;
     __shared__ CoopWarp s_warps[kCoopMaxWarps];
     __shared__ uint2 s_stack[kSharedStackDepth * 32 * kCoopMaxWarps];
     CoopWarp& W = s_warps[threadIdx.x >> 5];
@@ -135,7 +133,7 @@ __global__ void __launch_bounds__(256) wf_compact_active(WfBuffers B, unsigned i
     wf_enqueue(list, n_active, alive, (unsigned int)slot);
 }
 
-__global__ void __launch_bounds__(32 * kCoopMaxWarps, PERSIST_MIN_BLOCKS)
+__global__ void __launch_bounds__(32 * kCoopMaxWarps, kPersistMinBlocks)
 wf_tail(SceneDev S, RenderParams P, WfBuffers B, const unsigned int* list, const unsigned int* n_active_ptr, unsigned int* claim_counter,
         unsigned int* queue_mem, const float4* __restrict__ fb_in_rowmajor, float4* __restrict__ out_tiles)
 {
@@ -253,31 +251,16 @@ int wavefront_tail_max_ctas()
     return current_sm_count() * per_sm;
 }
 
-typedef void (*PersistKernel)(SceneDev, RenderParams, WfBuffers, unsigned int*, int, const float4*, float4*);
-
-static PersistKernel persist_kernel(int k)
-{
-    return k == 1 ? pt_persist<1> : (k == 4 ? pt_persist<4> : pt_persist<2>);
-}
-
-int persistent_slots_per_lane()
-{
-    static const int k = []() { const char* e = getenv("B200RT_PERSIST_K"); const int v = e ? atoi(e) : 2; return (v == 1 || v == 4) ? v : 2; }();
-    return k;
-}
-
 // CTAs of the persistent grid on the current device (a whole number per SM: every CTA is resident for the whole frame)
 int persistent_grid()
 {
     int per_sm = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, persist_kernel(persistent_slots_per_lane()), 32 * kCoopMaxWarps, 0);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pt_persist, 32 * kCoopMaxWarps, 0);
     if (per_sm <= 0) per_sm = 1;
-    static const int cap = []() { const char* e = getenv("B200RT_PERSIST_CTAS"); return e ? atoi(e) : 0; }();
-    if (cap > 0 && cap < per_sm) per_sm = cap;
     return current_sm_count() * per_sm;
 }
 
-int persistent_slots(int grid) { return grid * kCoopMaxWarps * persistent_slots_per_lane() * 32; }
+int persistent_slots(int grid) { return grid * kCoopMaxWarps * kPersistSlotsPerLane * 32; }
 
 // B: state for persistent_slots(grid) slots (n_slots set accordingly), queue of 5 * n_slots entries, counters >= 1 word (the next-pixel
 // counter), rays_total. The frame's pixels are this rank's tile-major slots [0, n_rank_tiles * 256); out_tiles is indexed by them.
@@ -292,7 +275,7 @@ cudaError_t run_persistent(const SceneDev& S, const RenderParams& P, const WfBuf
     // no more warps than there are 32-pixel patches to start with
     const int warps_needed = (n_frame_slots + 31) / 32;
     const int ctas = std::min(grid, (warps_needed + kCoopMaxWarps - 1) / kCoopMaxWarps);
-    persist_kernel(persistent_slots_per_lane())<<<ctas, 32 * kCoopMaxWarps, 0, stream>>>(S, P, B, B.counters, n_frame_slots, fb_in_rowmajor, out_tiles);
+    pt_persist<<<ctas, 32 * kCoopMaxWarps, 0, stream>>>(S, P, B, B.counters, n_frame_slots, fb_in_rowmajor, out_tiles);
     return cudaGetLastError();
 }
 

@@ -189,15 +189,6 @@ __device__ __forceinline__ void trav_init(Trav& T, v3 o, v3 d, float tmax, const
     T.sp = 0; T.cur = 0; T.done = false;
 }
 
-// hint: bring the record a reference points at (inner node or first leaf triangle) towards L1 ahead of its use
-__device__ __forceinline__ void prefetch_ref(const SceneDev& S, int ref)
-{
-#ifdef B200RT_PREFETCH
-    const void* p = ref >= 0 ? (const void*)(S.axis + 4 * (size_t)ref) : (const void*)(S.tris + 3 * (size_t)((~ref) >> 4));
-    asm volatile("prefetch.global.L1 [%0];" ::"l"(p));
-#endif
-}
-
 // pop the next subtree, skipping those that start beyond the current best; T.done when the stack is empty
 __device__ __forceinline__ void trav_pop(Trav& T, TravStack& K)
 {
@@ -271,7 +262,6 @@ __device__ __forceinline__ void trav_inner(const SceneDev& S, Trav& T, TravStack
             K.t[T.sp] = r_first ? tnL : tnR;
             T.sp++;
             T.cur = r_first ? refR : refL;
-            prefetch_ref(S, r_first ? refL : refR);
             return;
         }
         if (hitL) { T.cur = refL; return; }
@@ -376,10 +366,7 @@ struct TravStack8
     __device__ __forceinline__ void push(int sp, uint2 v) { e[sp] = v; }
     __device__ __forceinline__ uint2 pop(int sp) const { return e[sp]; }
 };
-#ifndef B200RT_SHARED_STACK_DEPTH
-#define B200RT_SHARED_STACK_DEPTH 10
-#endif
-constexpr int kSharedStackDepth = B200RT_SHARED_STACK_DEPTH;     // (a build with 2 runs the whole GPU test suite through the local-memory overflow)
+constexpr int kSharedStackDepth = 10;
 struct TravStack8Shared
 {
     uint2* sh;          // this thread's column: entry i at sh[i * blockDim.x]
@@ -488,16 +475,6 @@ __device__ __forceinline__ void trav8_node(const SceneDev& S, Trav8& T, Stack& K
     T.tg.x = __float_as_uint(n1.y);
     T.tg.y = (x * 7u) & T.tvalid;
     if (T.tg.y == 0u && !inner) trav8_pop(T, K);
-#ifdef B200RT_WIDE_PREFETCH
-    // the node this lane fetches next is already known: start bringing its lines towards L1 while the warp does its housekeeping
-    if (!T.done && (T.ng.y & 0xff000000u))
-    {
-        const unsigned int nslot = (unsigned int)(31 - __clz((int)T.ng.y) - 24) ^ T.oct;
-        const char* nx = (const char*)(S.wide + 5 * (size_t)(T.ng.x + __popc(T.ng.y & 0xffu & ~(0xffffffffu << nslot))));
-        asm volatile("prefetch.global.L1 [%0];" ::"l"(nx));
-        asm volatile("prefetch.global.L1 [%0];" ::"l"(nx + 64));
-    }
-#endif
 }
 
 // pre: !trav8_has_node(T). Exact triangle tests of the pending triangle group, then the next node group.
@@ -643,21 +620,9 @@ __device__ __forceinline__ float ggx_d(float alpha, float NoH)
 __device__ __forceinline__ float g1_schlick(float k, float dp) { return dp / (dp * (1.0f - k) + k); }
 __device__ __forceinline__ float power_heuristic(float a, float b) { float a2 = a * a; return a2 / (a2 + b * b); }
 
-// B200RT_CT_NOINLINE: the BRDF evaluation / sampling bodies become real functions (5 + 3 call sites per surface interaction):
-// the shade kernel shrinks and stalls less on instruction fetch
-#ifdef B200RT_CT_NOINLINE
-#define B200RT_CT_INLINE static __noinline__
-#else
-#define B200RT_CT_INLINE __forceinline__
-#endif
-#if defined(B200RT_CT_NOINLINE) && B200RT_CT_NOINLINE >= 2
-#define B200RT_CT_INLINE2 static __noinline__
-#else
-#define B200RT_CT_INLINE2 __forceinline__
-#endif
 // D = ggx_d(roughness^2, NoH), computed by the caller (the light- and env-sample paths need it for the pdf whether or not the BRDF
 // itself is evaluated: one double-precision division per pair instead of two)
-__device__ B200RT_CT_INLINE2 col ct_terms(const MaterialDev& m, float NoV, float NoL, float NoH, float VoH, float D, float* pdf_out)   // :272-298 / :424-448
+__device__ __forceinline__ col ct_terms(const MaterialDev& m, float NoV, float NoL, float NoH, float VoH, float D, float* pdf_out)   // :272-298 / :424-448
 {
     const float metalness = m.metalness;
     const float alpha = m.roughness * m.roughness;
@@ -696,7 +661,7 @@ __device__ __forceinline__ col ct_brdf_and_pdf(const MaterialDev& m, v3 to_light
 }
 
 // cook_torrance_brdf_importance_sample :392-451 — consumes exactly two draws
-__device__ B200RT_CT_INLINE col ct_sample(const MaterialDev& m, v3 view, v3 n, v3& out_dir, float& pdf, uint32_t& rng)
+__device__ __forceinline__ col ct_sample(const MaterialDev& m, v3 view, v3 n, v3& out_dir, float& pdf, uint32_t& rng)
 {
     pdf = 0.0f;
     const float alpha = m.roughness * m.roughness;

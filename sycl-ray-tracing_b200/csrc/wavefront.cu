@@ -15,8 +15,6 @@
 // No RNG draw depends on a trace result (SURVEY a5), which is what allows a whole surface interaction — all four side
 // rays and the continuation ray — to be generated in one shade pass and traced in one trace pass.
 #include <algorithm>
-#include <cstdio>
-#include <cstdlib>
 #include <utility>
 #include <vector>
 
@@ -24,12 +22,8 @@
 
 namespace b200rt {
 
-#ifndef WF_SHADE_BLOCK
-#define WF_SHADE_BLOCK 256              // threads per wf_shade CTA
-#endif
-#ifndef WF_SHADE_MIN_BLOCKS
-#define WF_SHADE_MIN_BLOCKS (1024 / WF_SHADE_BLOCK)      // 64 registers
-#endif
+constexpr int kShadeBlock = 256;                        // threads per wf_shade CTA
+constexpr int kShadeMinBlocks = 1024 / kShadeBlock;     // 64 registers
 
 __global__ void __launch_bounds__(256) wf_init(SceneDev S, RenderParams P, WfBuffers B, const float4* __restrict__ fb_in_rowmajor,
                                                float4* __restrict__ out_tiles)
@@ -58,7 +52,7 @@ __global__ void __launch_bounds__(256) wf_init(SceneDev S, RenderParams P, WfBuf
     wf_enqueue(B.queue, &B.counters[3], q_path, ((unsigned int)slot << 3) | 4u);
 }
 
-__global__ void __launch_bounds__(WF_SHADE_BLOCK, WF_SHADE_MIN_BLOCKS) wf_shade(SceneDev S, RenderParams P, WfBuffers B, const float4* __restrict__ fb_in_rowmajor,
+__global__ void __launch_bounds__(kShadeBlock, kShadeMinBlocks) wf_shade(SceneDev S, RenderParams P, WfBuffers B, const float4* __restrict__ fb_in_rowmajor,
                                                 float4* __restrict__ out_tiles, int parity)
 {
     const int slot = blockIdx.x * blockDim.x + threadIdx.x;
@@ -110,43 +104,12 @@ __global__ void wf_trace_simple(SceneDev S, WfBuffers B, int parity)
 // phase-vote persistent kernel (the default on the binary layout): every lane owns one traversal state; whenever at least
 // kRefillThreshold lanes of a warp are idle they are refilled with new rays from the warp's private block of the queue (blocks
 // of kWarpBlock rays are claimed with one atomic), so no lane waits for the slowest ray of its warp (Aila & Laine's persistent
-// threads, per lane).
-#ifndef WF_LEAF_MIN
-#define WF_LEAF_MIN 4
-#endif
-#ifdef WF_TRACE_MIN_BLOCKS
-#define WF_TRACE_BOUNDS __launch_bounds__(128, WF_TRACE_MIN_BLOCKS)
-#else
-#define WF_TRACE_BOUNDS
-#endif
-constexpr int kLeafThreshold = WF_LEAF_MIN;
-
-// one interface over the binary and the 8-ary traversal state machines, so the persistent kernel below serves every layout
-template <int TL>
-struct TravOps
-{
-    typedef Trav State;
-    typedef TravStack Stack;
-    static __device__ __forceinline__ void init(State& T, v3 o, v3 d, float tmax, int mode) { trav_init<TL == TL_DIAG>(T, o, d, tmax, mode); }
-    static __device__ __forceinline__ bool at_node(const State& T) { return T.cur >= 0; }
-    static __device__ __forceinline__ void node(const SceneDev& S, State& T, Stack& K) { trav_inner<TL == TL_DIAG>(S, T, K); }
-    static __device__ __forceinline__ void leaf(const SceneDev& S, State& T, Stack& K) { trav_leaf(S, T, K); }
-};
-template <>
-struct TravOps<TL_WIDE>
-{
-    typedef Trav8 State;
-    typedef TravStack8 Stack;
-    static __device__ __forceinline__ void init(State& T, v3 o, v3 d, float tmax, int mode) { trav8_init(T, o, d, tmax, mode); }
-    static __device__ __forceinline__ bool at_node(const State& T) { return trav8_has_node(T); }
-    static __device__ __forceinline__ void node(const SceneDev& S, State& T, Stack& K) { trav8_node(S, T, K); }
-    static __device__ __forceinline__ void leaf(const SceneDev& S, State& T, Stack& K) { trav8_tris(S, T, K); }
-};
+// threads, per lane). TL is TL_AXIS or TL_DIAG.
+constexpr int kLeafThreshold = 4;
 
 template <int TL>
-__global__ void WF_TRACE_BOUNDS wf_trace(SceneDev S, WfBuffers B, int parity)
+__global__ void wf_trace(SceneDev S, WfBuffers B, int parity)
 {
-    typedef TravOps<TL> Ops;
     const unsigned int FULL = 0xffffffffu;
     const int lane = threadIdx.x & 31;
     const unsigned int n_rays = B.counters[3 + parity];
@@ -159,8 +122,8 @@ __global__ void WF_TRACE_BOUNDS wf_trace(SceneDev S, WfBuffers B, int parity)
     const unsigned int total_warps = gridDim.x * (blockDim.x >> 5);
     const unsigned int warp_block = min((unsigned int)kWarpBlock, max(32u, (n_rays / total_warps) & ~31u));
 
-    typename Ops::State T;
-    typename Ops::Stack K;
+    Trav T;
+    TravStack K;
     T.done = true;
     bool active = false;
     size_t r = 0;
@@ -194,7 +157,7 @@ __global__ void WF_TRACE_BOUNDS wf_trace(SceneDev S, WfBuffers B, int parity)
                         const float4 ro4 = B.ray_o[r], rd4 = B.ray_d[r];
                         const int kind = __float_as_int(rd4.w);
                         mode = kind == SIDE_SHADOW ? TRACE_SHADOW : (kind == SIDE_CLOSEST_LIGHT ? TRACE_CLOSEST : TRACE_ANY);
-                        Ops::init(T, V(ro4.x, ro4.y, ro4.z), V(rd4.x, rd4.y, rd4.z), ro4.w, spheres ? TRACE_CLOSEST : mode);
+                        trav_init<TL == TL_DIAG>(T, V(ro4.x, ro4.y, ro4.z), V(rd4.x, rd4.y, rd4.z), ro4.w, spheres ? TRACE_CLOSEST : mode);
                         active = true;
                     }
                     blk_next = min(blk_next + (unsigned int)__popc(idle), blk_end);
@@ -204,15 +167,15 @@ __global__ void WF_TRACE_BOUNDS wf_trace(SceneDev S, WfBuffers B, int parity)
         }
         // warp-level phase vote: all lanes that hold an inner node step together, or all lanes that hold a leaf run the
         // exact triangle tests together, whichever is the majority — the two kinds of work never interleave inside a warp
-        const bool has_inner = active && Ops::at_node(T), has_leaf = active && !Ops::at_node(T);
+        const bool has_inner = active && T.cur >= 0, has_leaf = active && T.cur < 0;
         const unsigned int m_inner = __ballot_sync(FULL, has_inner), m_leaf = __ballot_sync(FULL, has_leaf);
         if (!(m_inner | m_leaf))
         {
             if (exhausted) break;
             continue;
         }
-        if (m_inner && __popc(m_leaf) < max(__popc(m_inner), kLeafThreshold)) { if (has_inner) Ops::node(S, T, K); }
-        else if (has_leaf) Ops::leaf(S, T, K);
+        if (m_inner && __popc(m_leaf) < max(__popc(m_inner), kLeafThreshold)) { if (has_inner) trav_inner<TL == TL_DIAG>(S, T, K); }
+        else if (has_leaf) trav_leaf(S, T, K);
         if (active && T.done)
         {
             bool found = T.hit.t > 0.0f;
@@ -224,10 +187,8 @@ __global__ void WF_TRACE_BOUNDS wf_trace(SceneDev S, WfBuffers B, int parity)
 }
 
 // ---- default trace kernel for the 8-ary layout: persistent lanes + warp-cooperative triangle tests (wf_device.cuh) ------------------
-#ifndef WF_COOP_MIN_BLOCKS
-#define WF_COOP_MIN_BLOCKS 7            // <= 72 registers: 28 warps per SM; 32 (64 registers) measured the same, 16 (117 registers) 20 % slower
-#endif
-__global__ void __launch_bounds__(32 * kCoopMaxWarps, WF_COOP_MIN_BLOCKS) wf_trace_coop(SceneDev S, WfBuffers B, int parity)
+constexpr int kCoopMinBlocks = 7;      // <= 72 registers: 28 warps per SM; 32 (64 registers) measured the same, 16 (117 registers) 20 % slower
+__global__ void __launch_bounds__(32 * kCoopMaxWarps, kCoopMinBlocks) wf_trace_coop(SceneDev S, WfBuffers B, int parity)
 {
     __shared__ CoopWarp s_warps[kCoopMaxWarps];
     CoopWarp& W = s_warps[threadIdx.x >> 5];
@@ -240,13 +201,9 @@ __global__ void __launch_bounds__(32 * kCoopMaxWarps, WF_COOP_MIN_BLOCKS) wf_tra
     src.head = &B.counters[5 + parity];
     src.n_rays = n_rays;
     src.warp_block = min((unsigned int)kWarpBlock, max(32u, (n_rays / total_warps) & ~31u));
-#ifdef WF_COOP_LOCAL_STACK
-    TravStack8 K;
-#else
     __shared__ uint2 s_stack[kSharedStackDepth * 32 * kCoopMaxWarps];
     TravStack8Shared K;
     K.sh = s_stack + threadIdx.x; K.stride = 32 * kCoopMaxWarps;
-#endif
     coop_trace_queue(S, B, B.queue, src, W, K);
 }
 
@@ -263,26 +220,21 @@ cudaError_t run_wavefront(const SceneDev& S, const RenderParams& P, const WfGrou
     int launches = 0;
     const int tl = traversal_layout(S, P.flags);
     const bool simple = (P.flags & B200RT_FLAG_SIMPLE_TRACE) != 0;
-    static const int tb_env = []() { const char* e = getenv("B200RT_TRACE_BLOCK"); int v = e ? atoi(e) : 128; return (v == 64 || v == 128 || v == 256) ? v : 128; }();
-    int per_sm = 0;
     typedef void (*TraceKernel)(SceneDev, WfBuffers, int);
-    static const TraceKernel kernels[2][3] = { { wf_trace<TL_AXIS>, wf_trace<TL_DIAG>, wf_trace<TL_WIDE> },
+    static const TraceKernel kernels[2][3] = { { wf_trace<TL_AXIS>, wf_trace<TL_DIAG>, wf_trace_coop },
                                                { wf_trace_simple<TL_AXIS>, wf_trace_simple<TL_DIAG>, wf_trace_simple<TL_WIDE> } };
-    static const bool vote_wide = []() { const char* e = getenv("B200RT_WIDE_TRACE"); return e && e[0] == 'v'; }();   // ablation: phase-vote kernel on the 8-ary layout
-    const bool coop = tl == TL_WIDE && !simple && !vote_wide;
-    const TraceKernel trace_kernel = coop ? wf_trace_coop : kernels[simple ? 1 : 0][tl];
-    const int tb = coop ? 32 * kCoopMaxWarps : tb_env;
+    const TraceKernel trace_kernel = kernels[simple ? 1 : 0][tl];
+    const bool coop = tl == TL_WIDE && !simple;
+    const int tb = 32 * kCoopMaxWarps;         // every trace kernel runs 128-thread CTAs (wf_trace_coop's shared state is sized for them)
+    int per_sm = 0;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, trace_kernel, tb, 0);
     if (per_sm <= 0) per_sm = 1;
-    // With several tile groups in flight a persistent trace kernel takes only ~4/7 of the CTAs that fit (B200RT_TRACE_GRID_PCT,
-    // default 58): the rest of every SM stays free for the other groups' trace / shade kernels, which then overlap with the
-    // whole pass instead of only with its tail (C3, 32 spp: 2 179 vs 2 108 Mrays/s; 72 %: 2 157, 43 %: 2 112).
-    static const int grid_pct_env = []() { const char* e = getenv("B200RT_TRACE_GRID_PCT"); int v = e ? atoi(e) : 0; return v > 100 ? 100 : v; }();
-    const bool timing_mode = getenv("B200RT_WF_TIMING") != nullptr || (P.flags & B200RT_FLAG_TIME_KERNELS);      // kernels run one at a time: full grid
-    const int grid_pct = grid_pct_env >= 10 ? grid_pct_env : ((n_groups > 1 && !timing_mode) ? 58 : 100);
+    const bool timing = (P.flags & B200RT_FLAG_TIME_KERNELS) != 0;     // kernels run one at a time: full grid
+    // With several tile groups in flight a persistent trace kernel takes only ~4/7 of the CTAs that fit: the rest of every SM
+    // stays free for the other groups' trace / shade kernels, which then overlap with the whole pass instead of only with its
+    // tail (C3, 32 spp: 2 179 vs 2 108 Mrays/s; 72 %: 2 157, 43 %: 2 112).
+    const int grid_pct = (n_groups > 1 && !timing) ? 58 : 100;
     const int trace_grid = n_sm * std::max(1, (per_sm * grid_pct + 50) / 100);
-    static const bool timing_env = getenv("B200RT_WF_TIMING") != nullptr;  // diagnostics: per-kernel times on stderr (serialises the groups)
-    const bool timing = timing_env || (P.flags & B200RT_FLAG_TIME_KERNELS);
     WfTimeline* const tln = (!timing && (P.flags & B200RT_FLAG_TIME_INLINE)) ? timeline : nullptr;
     if (tln)
     {
@@ -299,17 +251,15 @@ cudaError_t run_wavefront(const SceneDev& S, const RenderParams& P, const WfGrou
     cudaError_t err = cudaSuccess;
 #define WF_TRY(expr) do { if (err == cudaSuccess) { const cudaError_t e__ = (expr); if (e__ != cudaSuccess) err = e__; } } while (0)
     struct GroupRun { RenderParams P; int parity; bool finished, forked; int slot_grid; long long it, poll_it; bool poll_pending; unsigned int tail_below; };
-    // barrier-free tail (persist.cu): when a group has at most B200RT_WF_TAIL_PCT % of its pixels (and at most B200RT_WF_TAIL_CAP) left,
-    // or is smaller than B200RT_WF_TAIL_MIN pixels to begin with. 8-ary layout, default trace kernel only; not in the per-kernel timing modes.
+    // barrier-free tail (persist.cu): when a group has at most kTailPct % of its pixels (and at most kTailCap) left, or is smaller
+    // than kTailMin pixels to begin with. 8-ary layout, default trace kernel only; not under B200RT_FLAG_TIME_KERNELS.
     // Measured on C3 at 64 spp (profiles/r2_tail.jsonl): whole frame 433.3 ms without, 428.9 with a 30 k cap (445 with 100 k: the tail
     // kernel's throughput is below the pass kernels', it only pays once passes are latency-bound); one rank of 8: 108.1 -> 101.7 ms at 20 %.
-    // (the knobs are read per frame: tools/tail_bench.py sweeps them inside one process)
-    auto env_ll = [](const char* name, long long dflt) { const char* e = getenv(name); return e ? atoll(e) : dflt; };
-    const int tail_pct = (int)std::min(100ll, std::max(0ll, env_ll("B200RT_WF_TAIL_PCT", 20)));
-    const long long tail_cap = env_ll("B200RT_WF_TAIL_CAP", 30000);
-    const int tail_min = (int)env_ll("B200RT_WF_TAIL_MIN", 16384);
+    constexpr int kTailPct = 20;
+    constexpr long long kTailCap = 30000;
+    constexpr int kTailMin = 16384;
     const bool passes_only = (P.flags & B200RT_FLAG_WF_PASSES_ONLY) != 0;
-    const bool tail_ok = coop && tail_pct > 0 && !timing && !passes_only;
+    const bool tail_ok = coop && !timing && !passes_only;
     const int tail_ctas = tail_ok ? std::max(1, wavefront_tail_max_ctas() / n_groups) : 0;
     // launches the tail that finishes group g behind whatever is queued on its stream
     auto finish_group = [&](int g, const RenderParams& GP) -> cudaError_t
@@ -344,8 +294,8 @@ cudaError_t run_wavefront(const SceneDev& S, const RenderParams& P, const WfGrou
         if (R.finished) continue;
         wf_init<<<R.slot_grid, 256, 0, G.stream>>>(S, R.P, G.buf, fb_in_rowmajor, out_tiles);
         launches++;
-        R.tail_below = (unsigned int)std::min<long long>(tail_cap, (long long)G.buf.n_slots * tail_pct / 100);
-        if (tail_ok && G.buf.n_slots <= tail_min)
+        R.tail_below = (unsigned int)std::min<long long>(kTailCap, (long long)G.buf.n_slots * kTailPct / 100);
+        if (tail_ok && G.buf.n_slots <= kTailMin)
         {
             // a group this small is latency-bound from its first pass on: barrier-free from the start
             WF_TRY(finish_group(g, R.P));
@@ -400,7 +350,7 @@ cudaError_t run_wavefront(const SceneDev& S, const RenderParams& P, const WfGrou
             if (timing) cudaEventRecord(tev[1], G.stream);
             if (tln) { tll.e1 = tln->used; cudaEventRecord(tln->take(), G.stream); }
             R.parity ^= 1;
-            wf_shade<<<(G.buf.n_slots + WF_SHADE_BLOCK - 1) / WF_SHADE_BLOCK, WF_SHADE_BLOCK, 0, G.stream>>>(S, R.P, G.buf, fb_in_rowmajor, out_tiles, R.parity);
+            wf_shade<<<(G.buf.n_slots + kShadeBlock - 1) / kShadeBlock, kShadeBlock, 0, G.stream>>>(S, R.P, G.buf, fb_in_rowmajor, out_tiles, R.parity);
             if (tln) { tll.e2 = tln->used; cudaEventRecord(tln->take(), G.stream); tln->launches.push_back(tll); }
             launches += 2;
             WF_TRY(cudaGetLastError());
@@ -410,10 +360,7 @@ cudaError_t run_wavefront(const SceneDev& S, const RenderParams& P, const WfGrou
                 WF_TRY(cudaEventSynchronize(tev[2]));
                 float a = 0, b = 0;
                 cudaEventElapsedTime(&a, tev[0], tev[1]); cudaEventElapsedTime(&b, tev[1], tev[2]);
-                unsigned int nq[8] = {};
-                WF_TRY(cudaMemcpy(nq, G.buf.counters, sizeof(nq), cudaMemcpyDeviceToHost));
                 t_trace += a; t_shade += b; n_trace++; n_shade++;
-                if (timing_env) fprintf(stderr, "wf g%d it %lld: trace %.3f ms  shade %.3f ms  active px %u  next queue %u\n", g, R.it, a, b, nq[2], nq[3 + R.parity]);
             }
             R.it++;
             if (!R.poll_pending && ((R.it & 3) == 0 || R.it >= max_iters))
@@ -436,7 +383,6 @@ cudaError_t run_wavefront(const SceneDev& S, const RenderParams& P, const WfGrou
 #undef WF_TRY
     if (timing)
     {
-        if (timing_env) fprintf(stderr, "wf total: trace %.3f ms  shade %.3f ms  launches %d\n", t_trace, t_shade, launches);
         if (kernel_times4) { kernel_times4[0] = t_trace; kernel_times4[1] = t_shade; kernel_times4[2] = n_trace; kernel_times4[3] = n_shade; }
         for (int i = 0; i < 3; i++) cudaEventDestroy(tev[i]);
     }

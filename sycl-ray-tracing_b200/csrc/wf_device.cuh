@@ -299,22 +299,10 @@ __device__ __forceinline__ void wf_store_result(const WfBuffers& B, size_t r, in
 // drain; a ray is finished when it has no node work and no descriptor left in the ring.
 // (Round 1 appended every (owner, triangle) pair separately in a per-lane loop: 13.5 % of the kernel's instructions at 4.4
 // active lanes, profiles/r1b_blocks_wf_trace_coop_c3.txt.)
-#ifndef WF_WARP_BLOCK
-#define WF_WARP_BLOCK 64
-#endif
-#ifndef WF_REFILL
-#define WF_REFILL 8
-#endif
-#ifndef WF_COOP_DRAIN_TRIS
-#define WF_COOP_DRAIN_TRIS 64
-#endif
-#ifndef WF_COOP_RING
-#define WF_COOP_RING 64
-#endif
-constexpr int kWarpBlock = WF_WARP_BLOCK;
-constexpr int kRefillThreshold = WF_REFILL;
-constexpr int kCoopDrainTris = WF_COOP_DRAIN_TRIS;      // 32 or 64: pairs tested per drain
-constexpr int kCoopRing = WF_COOP_RING;                 // descriptors per warp (power of two, >= 64: a node step appends up to 32 and
+constexpr int kWarpBlock = 64;
+constexpr int kRefillThreshold = 8;
+constexpr int kCoopDrainTris = 64;                      // 32 or 64: pairs tested per drain
+constexpr int kCoopRing = 64;                           // descriptors per warp (power of two, >= 64: a node step appends up to 32 and
                                                         // a drain leaves at most 32 behind)
 constexpr int kCoopWork = 96;                           // expanded pairs per drain when flushing (>= kCoopDrainTris, multiple of 32)
 constexpr int kCoopMaxWarps = 4;                        // the kernels are launched with 128-thread CTAs
@@ -478,7 +466,6 @@ __device__ __forceinline__ void coop_trace_queue(const SceneDev& S, const WfBuff
                         const unsigned int qi = blk_base + 32u * j + (unsigned int)lane;
                         qe[j] = qi < blk_end ? queue[qi] : 0u;
                     }
-#ifndef B200RT_NO_RAY_PREFETCH
                     // ... and the ray records those entries name start moving towards L1 now (a pass kernel reads each of them
                     // exactly once, through L1: see the load below)
 #pragma unroll
@@ -489,7 +476,6 @@ __device__ __forceinline__ void coop_trace_queue(const SceneDev& S, const WfBuff
                             asm volatile("prefetch.global.L1 [%0];" ::"l"(B.ray_o + pr));
                             asm volatile("prefetch.global.L1 [%0];" ::"l"(B.ray_d + pr));
                         }
-#endif
                 }
             }
             if (blk_next < blk_end)
